@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N --steps K --warmup W]            our CUDA path
   python bench.py --impl reference [...]                     the CPU arm (oracle port, all host threads)
+  python bench.py --dump-outputs DIR [...]                   also write the timed path's outputs (see dump_outputs)
 
 Workload (configs 3+4 of BASELINE.json): 65,536 independent 64 KiB blocks of mixed entropy
 (DESIGN.md "generator"), AdaptiveTreeModel, Parameters(8,14,16) by default.  One STEP = encode the whole
@@ -35,19 +36,30 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from
 
 SEED = 0x5EED202610180000
 METRIC = "encode+decode round-trip throughput of raw input (bit-exact)"
 UNIT = "MB/s"
 NCU_TRAFFIC = ("r02_ncu_traffic.json", "r01_ncu_traffic.json")
 ISSUE_PEAK = "r01_issue_peak.json"
+DUMP_LIMIT = 64 * 10 ** 6           # bytes of .npy files --dump-outputs writes at most
+
+
+def int_at_least(minimum):
+    def parse(s):
+        v = int(s)
+        if v < minimum:
+            raise argparse.ArgumentTypeError("must be >= %d" % minimum)
+        return v
+    return parse
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int_at_least(1), default=5, help="timed steps of the headline measurement")
+    ap.add_argument("--warmup", type=int_at_least(0), default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--blocks", type=int, default=65536)
     ap.add_argument("--block-len", type=int, default=65536)
@@ -60,6 +72,8 @@ def parse_args():
     ap.add_argument("--no-ctx", action="store_true")
     ap.add_argument("--no-host-memory-kinds", action="store_true", help="skip the pageable / registered e2e legs")
     ap.add_argument("--cpu-sample-blocks", type=int, default=0, help="0 = 32 blocks per host thread")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed "
+                                                          "(rank 0's batch) as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -368,6 +382,43 @@ class DeviceBatch:
         return t_enc / steps, t_dec / steps
 
 
+def dump_sample_size(rb, n, L, params):
+    """How many blocks dump_outputs samples: as many as fit DUMP_LIMIT next to the per-block arrays, at the worst-case
+    stream length, so that the count (and with it the sample) depends on the arguments only."""
+    per_block = 8 * (4 * n + 1) + 4096                                  # float64 arrays over all blocks, npy headers
+    per_sample = 4 * (L + rb.compress_bound(L, params[2], params[0])) + 16
+    k = min(n, (DUMP_LIMIT - per_block) // per_sample)
+    if k < 1:
+        raise SystemExit("bench.py: --dump-outputs cannot fit %d blocks of %d B into %d bytes" % (n, L, DUMP_LIMIT))
+    return k
+
+
+def dump_outputs(out_dir, B, torch, k):
+    """What the timed path's last step returned to its caller, as .npy files under out_dir (at most DUMP_LIMIT bytes):
+      compressed_offsets, status, raw_lens, consumed   every block, float64 (exact below 2**53); status is the decoder's
+      sample_blocks                                     k block indices drawn with SEED (same arguments, same sample)
+      sample_compressed, sample_compressed_offsets      those blocks' streams (float32 per byte) and where each starts
+      sample_decoded                                    those blocks' decoded bytes, float32 [k, block_len]
+    Two builds run with the same arguments compute the same inputs, so their files compare value for value."""
+    import numpy as np
+    torch.cuda.synchronize()
+    off = B.comp_off.cpu().numpy()
+    idx = np.sort(np.random.default_rng(SEED).choice(B.n, size=k, replace=False))
+    streams = [B.comp[int(off[i]):int(off[i + 1])] for i in idx]
+    s_off = np.zeros(k + 1, dtype=np.float64)
+    np.cumsum([s.numel() for s in streams], out=s_off[1:])
+    decoded = B.back.view(B.n, B.L)[torch.as_tensor(idx, device=B.back.device)]
+    arrays = {
+        "compressed_offsets": off, "status": B.status.cpu().numpy(), "raw_lens": B.raw_lens.cpu().numpy(),
+        "consumed": B.consumed.cpu().numpy(), "sample_blocks": idx, "sample_compressed_offsets": s_off,
+        "sample_compressed": torch.cat(streams).cpu().numpy().astype(np.float32),
+        "sample_decoded": decoded.cpu().numpy().astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def copy_ceiling(torch, h_a, h_b, d_a, d_b, comp_bytes, barrier, steps=3):
     """The end-to-end step's byte counts moved by bare pinned copies, H2D and D2H concurrently on two streams:
     [raw up | streams down] then [streams up | raw down].  Every rank does it at once (barrier), so at N GPUs
@@ -437,14 +488,31 @@ def run_ours(a):
     ctx.set_text_corpus(text_corpus())
     first_block = sharding.weak_first_block(n, rank)      # weak scaling: distinct blocks per rank
 
+    dump_k = dump_sample_size(rb, n, L, params) if a.dump_outputs else 0
+
     # ---- synthetic batch, resident in HBM
     B = DeviceBatch(rb, ctx, torch, local, n, L, first_block, params, a.model)
     for _ in range(a.warmup):
         B.enc()
         B.dec()
+
+    # ---- timed region: K steps, device resident
+    sampler = ClockSampler(local)
+    ctx.timing_enable(True)
+    ctx.timing_collect()
+    launches0 = ctx.kernel_launches
+    sampler.start()
+    wall0 = time.perf_counter()
+    t_e, t_d = B.timed(torch, a.steps, barrier)
+    wall = time.perf_counter() - wall0
+    clocks = sampler.stop()
+    launches = ctx.kernel_launches - launches0
+    ktimes = ctx.timing_collect()
+    ctx.timing_enable(False)
+
     comp_bytes = B.check(torch)
 
-    # ---- parity of the batch being timed: the first blocks' streams against the oracle's bytes (every rank, untimed).
+    # ---- parity of the timed steps' output: the first blocks' streams against the oracle's bytes (every rank, untimed).
     # With the CPU baseline on (rank 0, N = 1) the same oracle run is the baseline's sample.
     import oracle_lib as o
     threads = host_threads()
@@ -462,19 +530,8 @@ def run_ours(a):
                      "%d of %d blocks (%d B each), one stream per thread" % (ns, n, L), oracle_build) if want_cpu else None
     del want, got
 
-    # ---- timed region: K steps, device resident
-    sampler = ClockSampler(local)
-    ctx.timing_enable(True)
-    ctx.timing_collect()
-    launches0 = ctx.kernel_launches
-    sampler.start()
-    wall0 = time.perf_counter()
-    t_e, t_d = B.timed(torch, a.steps, barrier)
-    wall = time.perf_counter() - wall0
-    clocks = sampler.stop()
-    launches = ctx.kernel_launches - launches0
-    ktimes = ctx.timing_collect()
-    ctx.timing_enable(False)
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, B, torch, dump_k)
 
     t_step, t_e, t_d = rank_max([t_e + t_d, t_e, t_d])
     raw_bytes = n * L

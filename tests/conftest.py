@@ -9,8 +9,6 @@ for p in (HERE, ROOT):
     if p not in sys.path:
         sys.path.insert(0, p)
 
-REFERENCE_RESOURCES = "/root/reference/resources"  # CPU container only; absent on the GPU box
-
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a real B200 (run with -m gpu on the GPU box)")
@@ -19,7 +17,3 @@ def pytest_configure(config):
 @pytest.fixture(scope="session")
 def golden_dir():
     return os.path.join(HERE, "golden")
-
-
-def has_reference_resources():
-    return os.path.isdir(REFERENCE_RESOURCES)

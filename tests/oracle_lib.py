@@ -3,16 +3,19 @@
 TEST INFRASTRUCTURE ONLY: imported by tests/, __graft_entry__.smoke() and bench.py's
 cpu_baseline / --impl reference legs.  The product package (redux_b200/) never imports it.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 ORACLE_DIR = os.path.join(os.path.dirname(_HERE), "oracle")
-_SO = os.path.join(ORACLE_DIR, "libredux_oracle.so")
-_SO_NATIVE = os.path.join(ORACLE_DIR, "libredux_oracle_native.so")
+_SO_PORTABLE = os.path.join(ORACLE_DIR, "libredux_oracle.so")
+_SO = _SO_PORTABLE
 
 OK, EOF, INVALID_INPUT, IO_ERROR = 0, 1, 2, 3
 LINEAR, TREE = 0, 1
@@ -26,10 +29,10 @@ class Params(C.Structure):
 
 def build(force=False):
     srcs = [os.path.join(ORACLE_DIR, f) for f in ("redux_oracle.c", "synth_blocks.c", "redux_oracle.h")]
-    if force or not os.path.exists(_SO) or any(
-            os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(_SO) for src in srcs):
+    if force or not os.path.exists(_SO_PORTABLE) or any(
+            os.path.exists(src) and os.path.getmtime(src) > os.path.getmtime(_SO_PORTABLE) for src in srcs):
         subprocess.run(["make", "-C", ORACLE_DIR, "-s"], check=True)
-    return _SO
+    return _SO_PORTABLE
 
 
 _lib = None
@@ -38,15 +41,20 @@ _flavour = "portable (-O3)"
 
 def use_native_build():
     """bench.py's CPU arm: rebuild the oracle with -O3 -march=native ON THIS HOST and load that build (must be
-    called before the first lib()).  Falls back to the portable build when there is no compiler.  Returns a
-    description for the JSON line."""
+    called before the first lib()).  The build goes to a temporary directory (removed at exit), so that the
+    benchmark runs from a read-only tree.  Falls back to the portable build when there is no compiler.  Returns
+    a description for the JSON line."""
     global _SO, _flavour
     if _lib is not None:
         return _flavour
     try:
-        r = subprocess.run(["make", "-C", ORACLE_DIR, "-s", "-B", "native"], capture_output=True, text=True, timeout=120)
-        if r.returncode == 0 and os.path.exists(_SO_NATIVE):
-            _SO = _SO_NATIVE
+        tmp = tempfile.mkdtemp(prefix="redux_oracle_")
+        atexit.register(shutil.rmtree, tmp, True)
+        native = os.path.join(tmp, "libredux_oracle_native.so")
+        r = subprocess.run(["make", "-C", ORACLE_DIR, "-s", "NATIVE=" + native, "native"],
+                           capture_output=True, text=True, timeout=120)
+        if r.returncode == 0 and os.path.exists(native):
+            _SO = native
             _flavour = "-O3 -march=native, built on this host"
     except Exception:
         pass
@@ -57,7 +65,7 @@ def lib():
     global _lib
     if _lib is not None:
         return _lib
-    if _SO != _SO_NATIVE:
+    if _SO == _SO_PORTABLE:
         build()
     L = C.CDLL(_SO)
     L.oracle_generate_blocks.argtypes = [C.c_void_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64]

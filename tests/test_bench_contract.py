@@ -1,7 +1,10 @@
 """bench.py's JSON line against the driver's contract, checked on the committed record of the last GPU run
-(profiles/r02_bench_default.json, profiles/r02_bench_reference_arm.json).  No GPU needed."""
+(profiles/r02_bench_default.json, profiles/r02_bench_reference_arm.json).  No GPU needed, except for the `-m gpu`
+test of --dump-outputs."""
 import json
 import os
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASELINE = json.load(open(os.path.join(ROOT, "BASELINE.json")))
@@ -79,3 +82,40 @@ def test_reference_arm_runs_without_mapping_the_product_library():
     line = out["line"]
     assert line["impl"] == "reference" and line["value"] > 0 and line["cpu_baseline"]["kind"] == "port"
     assert line["cpu_baseline"]["per_thread_MBps"] > 0 and line["cpu_baseline"]["MiBps"] > 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_what_the_timed_steps_computed(tmp_path):
+    """--dump-outputs: float .npy files within the size limit, the same for the same workload whatever --steps and
+    --warmup (0 included), every block decoded whole, and the sampled streams / decoded blocks equal to the oracle's
+    streams / the generated input."""
+    import subprocess
+    import sys
+
+    import numpy as np
+
+    import bench
+    import oracle_lib as o
+    n, L = 256, 65536
+    dumps = []
+    for steps, warmup in ((1, 0), (2, 1)):
+        d = tmp_path / ("s%d_w%d" % (steps, warmup))
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", str(warmup),
+                            "--blocks", str(n), "--block-len", str(L), "--no-e2e", "--no-classes", "--no-cpu-baseline",
+                            "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 0, r.stderr[-2000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        assert sum(f.stat().st_size for f in d.iterdir()) <= bench.DUMP_LIMIT
+        dumps.append({f.stem: np.load(f) for f in d.iterdir()})
+    a, b = dumps
+    assert sorted(a) == sorted(b) and all(np.array_equal(a[k], b[k]) for k in a)
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert (a["status"] == 0).all() and (a["raw_lens"] == L).all()
+    assert (a["consumed"] == np.diff(a["compressed_offsets"])).all()
+    idx, s_off = a["sample_blocks"].astype(np.int64), a["sample_compressed_offsets"].astype(np.int64)
+    assert 0 < idx.size < n and a["sample_decoded"].shape == (idx.size, L)
+    raw = o.generate_blocks(0, n, L, bench.SEED, corpus=bench.text_corpus())
+    for j, i in enumerate(idx):
+        block = raw[i * L:(i + 1) * L]
+        assert a["sample_compressed"][s_off[j]:s_off[j + 1]].astype(np.uint8).tobytes() == o.compress(block, o.TREE, (8, 14, 16))[1]
+        assert (a["sample_decoded"][j].astype(np.uint8) == block).all()

@@ -246,16 +246,29 @@ def test_generator_host_is_deterministic_and_mixed():
     assert ent[0] > 7.8 and 4.0 < ent[1] < 5.2 and 1.6 < ent[2] < 2.3 and ent[3] < 0.5, ent
 
 
+def _run_without_a_device(body):
+    """Run `body` in a fresh interpreter that sees no CUDA device (CUDA_VISIBLE_DEVICES=""), so that what the library
+    does without a device is checked on every machine, one with GPUs included."""
+    import subprocess
+    import sys
+    import textwrap
+    code = "import sys\nsys.path.insert(0, %r)\n" % ROOT + textwrap.dedent(body)
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, timeout=120)
+    assert r.returncode == 0, r.stderr[-2000:]
+
+
 def test_no_gpu_means_cuda_error_not_fallback():
     """The product path must fail loudly without a device (no CPU fallback)."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    with pytest.raises(rb.CudaError):
-        rb.Context()
-    import io
-    with pytest.raises(rb.CudaError):
-        rb.compress(io.BytesIO(b"redux"), io.BytesIO(), rb.AdaptiveTreeModel(rb.Parameters(8, 14, 16)))
+    _run_without_a_device("""
+        import io
+        import pytest
+        import redux_b200 as rb
+        with pytest.raises(rb.CudaError):
+            rb.Context()
+        with pytest.raises(rb.CudaError):
+            rb.compress(io.BytesIO(b"redux"), io.BytesIO(), rb.AdaptiveTreeModel(rb.Parameters(8, 14, 16)))
+    """)
 
 
 def test_product_package_does_not_touch_oracle():
@@ -324,12 +337,14 @@ def test_process_init_is_explicit_and_respects_the_applications_setting():
 
 
 def test_pinned_memory_entry_points_fail_loudly_without_a_device():
-    """No GPU here: page-locking needs CUDA, and the entry points say so instead of handing out pageable memory."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("a CUDA device is present")
-    p = C.c_void_p()
-    assert rb.lib().redux_host_alloc(4096, C.byref(p)) == rb.CUDA_ERROR and not p.value
-    buf = np.zeros(4096, dtype=np.uint8)
-    assert rb.lib().redux_host_register(buf.ctypes.data, buf.nbytes) == rb.CUDA_ERROR
-    assert rb.lib().redux_host_alloc(0, C.byref(p)) == rb.OK          # nothing to allocate
+    """No device: page-locking needs CUDA, and the entry points say so instead of handing out pageable memory."""
+    _run_without_a_device("""
+        import ctypes as C
+        import numpy as np
+        import redux_b200 as rb
+        p = C.c_void_p()
+        assert rb.lib().redux_host_alloc(4096, C.byref(p)) == rb.CUDA_ERROR and not p.value
+        buf = np.zeros(4096, dtype=np.uint8)
+        assert rb.lib().redux_host_register(buf.ctypes.data, buf.nbytes) == rb.CUDA_ERROR
+        assert rb.lib().redux_host_alloc(0, C.byref(p)) == rb.OK          # nothing to allocate
+    """)

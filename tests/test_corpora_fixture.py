@@ -1,7 +1,6 @@
-"""The corpora fixture that travels to the GPU box is the reference's own data: every member matches the
-manifest, the manifest matches /root/reference/resources where that exists (this container), and the oracle's
-compressed size + SHA-256 prefix of every file equals SURVEY.md's B.2 table (tests/golden/corpus_table.json) --
-the same check as tests/test_oracle_corpora.py, but from the fixture, so it also runs without the reference."""
+"""The corpora fixture is the reference's own data: every member matches the manifest (size and SHA-256 of every
+file of the reference's resources/), and the oracle's compressed size + SHA-256 prefix of every file equals
+SURVEY.md's B.2 table (tests/golden/corpus_table.json) -- for all 36 files as one batch."""
 import hashlib
 import os
 
@@ -10,7 +9,6 @@ import pytest
 
 import corpora_fixture as cf
 import oracle_lib as o
-from conftest import REFERENCE_RESOURCES, has_reference_resources
 
 
 def test_fixture_matches_manifest_and_table():
@@ -23,13 +21,6 @@ def test_fixture_matches_manifest_and_table():
     assert sorted(table) == sorted(files)
     assert all(table[f]["raw"] == len(files[f]) for f in files)
     assert sum(len(v) for k, v in files.items() if k.startswith(("calgary/", "canterbury/"))) == 6040451   # config 2
-
-
-@pytest.mark.skipif(not has_reference_resources(), reason="reference fixtures not present")
-def test_fixture_equals_reference_tree():
-    files = cf.corpora()
-    for name, data in files.items():
-        assert open(os.path.join(REFERENCE_RESOURCES, name), "rb").read() == data, name
 
 
 @pytest.mark.parametrize("triple", ["8,14,16", "8,22,24", "8,30,32"])

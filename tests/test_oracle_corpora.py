@@ -1,16 +1,16 @@
 """tests/corpora.rs restated for the oracle: round trip + exact byte accounting on the reference's
-fixtures, plus the SURVEY.md Appendix B.2 size/SHA cross-check.  Needs /root/reference/resources, so it
-runs in the CPU container only (skipped on the GPU box, where the reference tree does not exist)."""
+fixtures, plus the SURVEY.md Appendix B.2 size/SHA cross-check.  The fixtures come from
+tests/golden/corpora/corpora.tar.xz, byte-identical to the reference's resources/ (its MANIFEST.json holds
+their SHA-256, checked by tests/test_corpora_fixture.py)."""
 import hashlib
 import json
 import os
 
 import pytest
 
+import corpora_fixture as cf
 import oracle_lib as o
-from conftest import REFERENCE_RESOURCES, has_reference_resources
 
-pytestmark = pytest.mark.skipif(not has_reference_resources(), reason="reference fixtures not present")
 TABLE = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "corpus_table.json")))
 SMALL = [r for r in TABLE if r["raw"] <= 150000]
 
@@ -21,7 +21,7 @@ def test_corpus_table_tree(triple):
     decoder consumes exactly the compressed length (tests/corpora.rs:40-41,59,61)."""
     p = tuple(int(x) for x in triple.split(","))
     for row in SMALL:
-        data = open(os.path.join(REFERENCE_RESOURCES, row["file"]), "rb").read()
+        data = cf.corpora()[row["file"]]
         assert len(data) == row["raw"]
         rc, comp, ic, oc = o.compress(data, o.TREE, p)
         assert rc == o.OK and ic == len(data) and oc == len(comp)
@@ -34,7 +34,7 @@ def test_corpus_table_tree(triple):
 def test_corpus_linear_equals_tree_small():
     """AdaptiveLinearModel and AdaptiveTreeModel give identical bytes (config 2's claim)."""
     for row in [r for r in TABLE if r["raw"] <= 60000]:
-        data = open(os.path.join(REFERENCE_RESOURCES, row["file"]), "rb").read()
+        data = cf.corpora()[row["file"]]
         for p in ((8, 14, 16), (8, 30, 32)):
             a = o.compress(data, o.LINEAR, p)
             b = o.compress(data, o.TREE, p)
@@ -46,7 +46,7 @@ def test_corpus_linear_equals_tree_small():
 def test_book1_cli_parameters():
     """Config 1: calgary/book1, Tree, (8,30,32) (src/main.rs:108)."""
     row = [r for r in TABLE if r["file"] == "calgary/book1"][0]
-    data = open(os.path.join(REFERENCE_RESOURCES, "calgary/book1"), "rb").read()
+    data = cf.corpora()["calgary/book1"]
     rc, comp, ic, oc = o.compress(data, o.TREE, (8, 30, 32))
     assert (rc, ic, oc) == (o.OK, 768771, 435400)
     assert hashlib.sha256(comp).hexdigest()[:16] == row["8,30,32"][1]
