@@ -155,7 +155,8 @@ int redux_encode_batch(redux_ctx_t *ctx, int model_kind, const redux_params_t *p
  *   raw[raw_offsets[i] ..) with capacity raw_offsets[i+1]-raw_offsets[i]; raw_lens[i] = bytes written
  *   (second tuple element of decompress()), consumed[i] = compressed bytes read (first element).
  *   A truncated stream gives status REDUX_EOF with the bytes decoded so far left in place; bytes beyond
- *   raw_lens[i] inside slot i are unspecified. */
+ *   raw_lens[i] inside slot i are unspecified.  A full slot gives REDUX_OUT_CAPACITY (unless the stream ends or is
+ *   cut first); consumed[i] then includes the bits of the symbol that found no room, as the reference's reader. */
 int redux_decode_batch(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
                        const uint8_t *comp, const uint64_t *comp_offsets, uint64_t n_blocks,
                        uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
@@ -254,6 +255,14 @@ void redux_debug_renorm(uint64_t low, uint64_t high, uint32_t code_bits,
 
 /* Resident CTAs per SM of the tuned encoder / decoder with 16-bit tables (must be 2; needs a device). */
 int redux_debug_lane_occupancy(int *enc_ctas_per_sm, int *dec_ctas_per_sm);
+
+/* Which coder kernels the context has launched: bit k of *mask is set when the kernel instantiation with ID k ran
+ * since the last reset (reset != 0 clears the mask after reading it).  Lets tests check which of the ~45 kernels a
+ * parameter set, block length, capacity, model and schedule actually selects.  Costs one host-side atomic OR per
+ * coder launch. */
+int redux_debug_launched_kernels(redux_ctx_t *ctx, uint64_t *mask, int reset);
+/* Name of kernel ID id, e.g. "decode_lane_al<u32,WideD,full,c32>"; NULL past the last ID.  Needs no device. */
+const char *redux_debug_kernel_name(int id);
 
 /* The host front end's partition rule: device g of n_devices codes blocks [first, first+count). */
 void redux_debug_shard(uint64_t n_blocks, uint32_t n_devices, uint32_t g, uint64_t *first, uint64_t *count);

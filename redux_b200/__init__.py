@@ -19,7 +19,7 @@ import numpy as np
 __all__ = [
     "Parameters", "AdaptiveLinearModel", "AdaptiveTreeModel", "Model", "compress", "decompress",
     "Context", "ReduxError", "Eof", "InvalidInput", "IoError", "CudaError", "Unsupported", "OutCapacity",
-    "compress_bound", "build", "lib", "process_init", "HostBuffer", "host_register", "host_unregister",
+    "compress_bound", "kernel_names", "build", "lib", "process_init", "HostBuffer", "host_register", "host_unregister",
 ]
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -142,6 +142,9 @@ def lib():
     L.redux_debug_shard.argtypes = [u64, u32, u32, C.POINTER(u64), C.POINTER(u64)]
     L.redux_debug_shard.restype = None
     L.redux_debug_lane_occupancy.argtypes = [C.POINTER(C.c_int), C.POINTER(C.c_int)]
+    L.redux_debug_launched_kernels.argtypes = [vp, C.POINTER(u64), i32]
+    L.redux_debug_kernel_name.argtypes = [i32]
+    L.redux_debug_kernel_name.restype = C.c_char_p
     L.redux_process_init.argtypes = []
     L.redux_host_alloc.argtypes = [C.c_size_t, C.POINTER(vp)]
     L.redux_host_free.argtypes = [vp]
@@ -199,6 +202,16 @@ def host_register(array):
 
 def host_unregister(array):
     _raise(lib().redux_host_unregister(array.ctypes.data))
+
+
+def kernel_names():
+    """Names of every coder kernel instantiation the library can launch, in ID order (needs no device)."""
+    names = []
+    while True:
+        n = lib().redux_debug_kernel_name(len(names))
+        if n is None:
+            return names
+        names.append(n.decode())
 
 
 def compress_bound(in_len, code_bits, symbol_bits=8):
@@ -349,6 +362,12 @@ class Context:
     @property
     def kernel_launches(self):
         return int(lib().redux_ctx_kernel_launches(self._h))
+
+    def launched_kernels(self, reset=True):
+        """Names of the coder kernels launched since the last reset (see kernel_names())."""
+        mask = C.c_uint64()
+        _raise(lib().redux_debug_launched_kernels(self._h, C.byref(mask), 1 if reset else 0), self)
+        return {n for i, n in enumerate(kernel_names()) if mask.value >> i & 1}
 
     def set_schedule(self, sched):
         _raise(lib().redux_ctx_set_schedule(self._h, sched), self)

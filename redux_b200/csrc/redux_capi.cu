@@ -46,6 +46,60 @@ extern "C" int redux_process_init(void)
 
 namespace {
 
+// One ID per kernel instantiation a launch_* function below can start (redux_debug_launched_kernels).  Lane
+// kernels: <table entry type, class, full tree values, code_bits == 32[, staged window refill]>; generic kernels:
+// Fenwick columns in shared memory (symbol_bits <= kGenericSmemSymbolBits) or in global memory.
+#define RDX_KERNEL_IDS(X) \
+    X(kEncNarrow,          "encode_lane_al<u16,Narrow,full,!c32>")       \
+    X(kEncWideU32,         "encode_lane_al<u32,Wide,full,!c32>")         \
+    X(kEncWideU16Full,     "encode_lane_al<u16,Wide,full,!c32>")         \
+    X(kEncWideU16,         "encode_lane_al<u16,Wide,!full,!c32>")        \
+    X(kEncWideU32C32,      "encode_lane_al<u32,Wide,full,c32>")          \
+    X(kEncWideU16FullC32,  "encode_lane_al<u16,Wide,full,c32>")          \
+    X(kEncWideU16C32,      "encode_lane_al<u16,Wide,!full,c32>")         \
+    X(kEncWideDU32,        "encode_lane_al<u32,WideD,full,!c32>")        \
+    X(kEncWideDU16Full,    "encode_lane_al<u16,WideD,full,!c32>")        \
+    X(kEncWideDU16,        "encode_lane_al<u16,WideD,!full,!c32>")       \
+    X(kEncWideDU32C32,     "encode_lane_al<u32,WideD,full,c32>")         \
+    X(kEncWideDU16FullC32, "encode_lane_al<u16,WideD,full,c32>")         \
+    X(kEncWideDU16C32,     "encode_lane_al<u16,WideD,!full,c32>")        \
+    X(kDecNarrowStg,       "decode_lane_al<u16,Narrow,full,!c32,stg>")   \
+    X(kDecNarrow,          "decode_lane_al<u16,Narrow,full,!c32>")       \
+    X(kDecWideU32,         "decode_lane_al<u32,Wide,full,!c32>")         \
+    X(kDecWideU16Full,     "decode_lane_al<u16,Wide,full,!c32>")         \
+    X(kDecWideU16,         "decode_lane_al<u16,Wide,!full,!c32>")        \
+    X(kDecWideU32C32,      "decode_lane_al<u32,Wide,full,c32>")          \
+    X(kDecWideU16FullC32,  "decode_lane_al<u16,Wide,full,c32>")          \
+    X(kDecWideU16C32,      "decode_lane_al<u16,Wide,!full,c32>")         \
+    X(kDecWideDU32,        "decode_lane_al<u32,WideD,full,!c32>")        \
+    X(kDecWideDU16Full,    "decode_lane_al<u16,WideD,full,!c32>")        \
+    X(kDecWideDU16,        "decode_lane_al<u16,WideD,!full,!c32>")       \
+    X(kDecWideDU32C32,     "decode_lane_al<u32,WideD,full,c32>")         \
+    X(kDecWideDU16FullC32, "decode_lane_al<u16,WideD,full,c32>")         \
+    X(kDecWideDU16C32,     "decode_lane_al<u16,WideD,!full,c32>")        \
+    X(kEncHugeU16,         "encode_lane<u16,Huge>")                      \
+    X(kEncHugeU32,         "encode_lane<u32,Huge>")                      \
+    X(kDecHugeU16,         "decode_lane<u16,Huge>")                      \
+    X(kDecHugeU32,         "decode_lane<u32,Huge>")                      \
+    X(kEncWarpNarrow,      "encode_warp<Narrow>")                        \
+    X(kEncWarpWide,        "encode_warp<Wide>")                          \
+    X(kEncWarpHuge,        "encode_warp<Huge>")                          \
+    X(kDecWarpNarrow,      "decode_warp_al<Narrow,!c32>")                \
+    X(kDecWarpWide,        "decode_warp_al<Wide,!c32>")                  \
+    X(kDecWarpWideC32,     "decode_warp_al<Wide,c32>")                   \
+    X(kDecWarpHuge,        "decode_warp<Huge>")                          \
+    X(kSplitNarrow,        "split_coder<Narrow,!c32>")                   \
+    X(kSplitWide,          "split_coder<Wide,!c32>")                     \
+    X(kSplitWideC32,       "split_coder<Wide,c32>")                      \
+    X(kEncGenericSmem,     "encode_generic<smem>")                       \
+    X(kEncGenericGlobal,   "encode_generic<global>")                     \
+    X(kDecGenericSmem,     "decode_generic<smem>")                       \
+    X(kDecGenericGlobal,   "decode_generic<global>")
+#define RDX_KERNEL_ENUM(id, name) id,
+enum KernelId : int { RDX_KERNEL_IDS(RDX_KERNEL_ENUM) kKernelIdCount };
+#undef RDX_KERNEL_ENUM
+static_assert(kKernelIdCount <= 64, "the launched-kernel mask is 64 bits wide");
+
 struct MagicEntry { int cls; uint32_t nbits; uint32_t len; void *ptr; };
 
 // Grow-only device buffer.
@@ -207,6 +261,10 @@ struct redux_ctx {
     std::vector<TimedSpan> spans;
     StagingConfig staging;
     CopyPool *pool = nullptr;              // created by the first call that meets pageable memory
+    // bit k: kernel KernelId k was launched since the last reset (redux_debug_launched_kernels).  Atomic: the
+    // per-device workers of a multi-device call OR their bits in from their own threads.
+    std::atomic<uint64_t> kernels_launched{0};
+    void note_kernel(int id) { kernels_launched.fetch_or((uint64_t)1 << id, std::memory_order_relaxed); }
 };
 
 namespace {
@@ -466,83 +524,84 @@ GenericJob generic_job(const Plan &pl)
     return g;
 }
 
+// Every launch_* function returns the KernelId of the kernel it started.
 // code_bits > 32: the generic kernels
 template <typename TW>
-void launch_encode(const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_encode(const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
     encode_lane_kernel<TW, kHuge><<<grid, kLaneThreads, smem, s>>>(job);
+    return sizeof(TW) == 4 ? kEncHugeU32 : kEncHugeU16;
 }
 template <typename TW>
-void launch_decode(const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_decode(const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
     decode_lane_kernel<TW, kHuge><<<grid, kLaneThreads, smem, s>>>(job);
+    return sizeof(TW) == 4 ? kDecHugeU32 : kDecHugeU16;
 }
 
 // code_bits <= 32: the tuned kernels
 template <bool C32>
-void launch_encode_wide(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_encode_wide(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.wide_table)       encode_lane_al_kernel<uint32_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);
-    else if (pl.full_table)  encode_lane_al_kernel<uint16_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);
-    else                     encode_lane_al_kernel<uint16_t, kWide, false, C32><<<grid, kLaneThreads, smem, s>>>(job);
+    if (pl.wide_table)      { encode_lane_al_kernel<uint32_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideU32C32 : kEncWideU32; }
+    else if (pl.full_table) { encode_lane_al_kernel<uint16_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideU16FullC32 : kEncWideU16Full; }
+    else                    { encode_lane_al_kernel<uint16_t, kWide, false, C32><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kEncWideU16C32 : kEncWideU16; }
 }
 template <bool C32>
-void launch_decode_wide(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_decode_wide(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.wide_table)       decode_lane_al_kernel<uint32_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
-    else if (pl.full_table)  decode_lane_al_kernel<uint16_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
-    else                     decode_lane_al_kernel<uint16_t, kWide, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
+    if (pl.wide_table)      { decode_lane_al_kernel<uint32_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideU32C32 : kDecWideU32; }
+    else if (pl.full_table) { decode_lane_al_kernel<uint16_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideU16FullC32 : kDecWideU16Full; }
+    else                    { decode_lane_al_kernel<uint16_t, kWide, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kDecWideU16C32 : kDecWideU16; }
 }
 template <bool C32>
-void launch_encode_wided(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_encode_wided(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.wide_table)      encode_lane_al_kernel<uint32_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);
-    else if (pl.full_table) encode_lane_al_kernel<uint16_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);
-    else                    encode_lane_al_kernel<uint16_t, kWideD, false, C32><<<grid, kLaneThreads, smem, s>>>(job);
+    if (pl.wide_table)      { encode_lane_al_kernel<uint32_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideDU32C32 : kEncWideDU32; }
+    else if (pl.full_table) { encode_lane_al_kernel<uint16_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideDU16FullC32 : kEncWideDU16Full; }
+    else                    { encode_lane_al_kernel<uint16_t, kWideD, false, C32><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kEncWideDU16C32 : kEncWideDU16; }
 }
 template <bool C32>
-void launch_decode_wided(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_decode_wided(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.wide_table)      decode_lane_al_kernel<uint32_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
-    else if (pl.full_table) decode_lane_al_kernel<uint16_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
-    else                    decode_lane_al_kernel<uint16_t, kWideD, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job);
+    if (pl.wide_table)      { decode_lane_al_kernel<uint32_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideDU32C32 : kDecWideDU32; }
+    else if (pl.full_table) { decode_lane_al_kernel<uint16_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideDU16FullC32 : kDecWideDU16Full; }
+    else                    { decode_lane_al_kernel<uint16_t, kWideD, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kDecWideDU16C32 : kDecWideDU16; }
 }
-void launch_encode_al(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_encode_al(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.lane_cls == kWideD) { if (pl.c == 32) launch_encode_wided<true>(pl, job, grid, smem, s); else launch_encode_wided<false>(pl, job, grid, smem, s); return; }
-    if (pl.cls == kNarrow) encode_lane_al_kernel<uint16_t, kNarrow, true, false><<<grid, kLaneThreads, smem, s>>>(job);
-    else if (pl.c == 32)   launch_encode_wide<true>(pl, job, grid, smem, s);
-    else                   launch_encode_wide<false>(pl, job, grid, smem, s);
+    if (pl.lane_cls == kWideD) return pl.c == 32 ? launch_encode_wided<true>(pl, job, grid, smem, s) : launch_encode_wided<false>(pl, job, grid, smem, s);
+    if (pl.cls == kNarrow) { encode_lane_al_kernel<uint16_t, kNarrow, true, false><<<grid, kLaneThreads, smem, s>>>(job); return kEncNarrow; }
+    return pl.c == 32 ? launch_encode_wide<true>(pl, job, grid, smem, s) : launch_encode_wide<false>(pl, job, grid, smem, s);
 }
-void launch_decode_al(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+int launch_decode_al(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
 {
-    if (pl.lane_cls == kWideD) { if (pl.c == 32) launch_decode_wided<true>(pl, job, grid, smem, s); else launch_decode_wided<false>(pl, job, grid, smem, s); return; }
+    if (pl.lane_cls == kWideD) return pl.c == 32 ? launch_decode_wided<true>(pl, job, grid, smem, s) : launch_decode_wided<false>(pl, job, grid, smem, s);
     if (pl.cls == kNarrow) {
-        if (pl.c <= 16) decode_lane_al_kernel<uint16_t, kNarrow, true, false, true><<<grid, kLaneThreads, smem, s>>>(job);
-        else            decode_lane_al_kernel<uint16_t, kNarrow, true, false, false><<<grid, kLaneThreads, smem, s>>>(job);
+        if (pl.c <= 16) { decode_lane_al_kernel<uint16_t, kNarrow, true, false, true><<<grid, kLaneThreads, smem, s>>>(job);  return kDecNarrowStg; }
+        else            { decode_lane_al_kernel<uint16_t, kNarrow, true, false, false><<<grid, kLaneThreads, smem, s>>>(job); return kDecNarrow; }
     }
-    else if (pl.c == 32)   launch_decode_wide<true>(pl, job, grid, smem, s);
-    else                   launch_decode_wide<false>(pl, job, grid, smem, s);
+    return pl.c == 32 ? launch_decode_wide<true>(pl, job, grid, smem, s) : launch_decode_wide<false>(pl, job, grid, smem, s);
 }
 
-void launch_encode_warp(int cls, const LaneEncJob &job, cudaStream_t s)
+int launch_encode_warp(int cls, const LaneEncJob &job, cudaStream_t s)
 {
     const uint32_t grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
-    if (cls == kNarrow)    encode_warp_kernel<kNarrow><<<grid, kWarpCtaThreads, 0, s>>>(job);
-    else if (cls == kWide) encode_warp_kernel<kWide><<<grid, kWarpCtaThreads, 0, s>>>(job);
-    else                   encode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);
+    if (cls == kNarrow)    { encode_warp_kernel<kNarrow><<<grid, kWarpCtaThreads, 0, s>>>(job); return kEncWarpNarrow; }
+    else if (cls == kWide) { encode_warp_kernel<kWide><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kEncWarpWide; }
+    else                   { encode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kEncWarpHuge; }
 }
-void launch_decode_warp(int cls, const LaneDecJob &job, cudaStream_t s)
+int launch_decode_warp(int cls, const LaneDecJob &job, cudaStream_t s)
 {
     const uint32_t grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
-    if (cls == kNarrow)     decode_warp_al_kernel<kNarrow, false><<<grid, kWarpCtaThreads, 0, s>>>(job);
-    else if (cls == kHuge)  decode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);
-    else if (job.c == 32)   decode_warp_al_kernel<kWide, true><<<grid, kWarpCtaThreads, 0, s>>>(job);
-    else                    decode_warp_al_kernel<kWide, false><<<grid, kWarpCtaThreads, 0, s>>>(job);
+    if (cls == kNarrow)     { decode_warp_al_kernel<kNarrow, false><<<grid, kWarpCtaThreads, 0, s>>>(job); return kDecWarpNarrow; }
+    else if (cls == kHuge)  { decode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);            return kDecWarpHuge; }
+    else if (job.c == 32)   { decode_warp_al_kernel<kWide, true><<<grid, kWarpCtaThreads, 0, s>>>(job);    return kDecWarpWideC32; }
+    else                    { decode_warp_al_kernel<kWide, false><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kDecWarpWide; }
 }
 
-// Split encoder: model phase over all chunks of all streams, then one coder warp per stream.
-int launch_encode_split(redux_ctx *ctx, DeviceState *d, const Plan &pl, const LaneEncJob &job, cudaStream_t s)
+// Split encoder: model phase over all chunks of all streams, then one coder warp per stream (its KernelId in *kid).
+int launch_encode_split(redux_ctx *ctx, DeviceState *d, const Plan &pl, const LaneEncJob &job, cudaStream_t s, int *kid)
 {
     if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
     SplitJob sj;
@@ -558,9 +617,9 @@ int launch_encode_split(redux_ctx *ctx, DeviceState *d, const Plan &pl, const La
     split_scan_kernel<<<(uint32_t)job.n_blocks, 256, 0, s>>>(sj);
     split_model_kernel<<<(uint32_t)((chunks + kSplitModelWarps - 1) / kSplitModelWarps), kSplitModelWarps * 32, 0, s>>>(sj);
     const uint32_t grid = (uint32_t)job.n_blocks;
-    if (pl.cls == kNarrow)   split_coder_kernel<kNarrow, false><<<grid, 32, 0, s>>>(job, sj);
-    else if (pl.c == 32)     split_coder_kernel<kWide, true><<<grid, 32, 0, s>>>(job, sj);
-    else                     split_coder_kernel<kWide, false><<<grid, 32, 0, s>>>(job, sj);
+    if (pl.cls == kNarrow)   { split_coder_kernel<kNarrow, false><<<grid, 32, 0, s>>>(job, sj); *kid = kSplitNarrow; }
+    else if (pl.c == 32)     { split_coder_kernel<kWide, true><<<grid, 32, 0, s>>>(job, sj);    *kid = kSplitWideC32; }
+    else                     { split_coder_kernel<kWide, false><<<grid, 32, 0, s>>>(job, sj);   *kid = kSplitWide; }
     ctx->launches += 3;      // + the one counted by the caller
     return REDUX_OK;
 }
@@ -709,6 +768,21 @@ extern "C" int redux_debug_lane_occupancy(int *enc_ctas_per_sm, int *dec_ctas_pe
         (void)cudaGetLastError();
         return REDUX_CUDA_ERROR;
     }
+    return REDUX_OK;
+}
+
+extern "C" const char *redux_debug_kernel_name(int id)
+{
+#define RDX_KERNEL_NAME(id, name) name,
+    static const char *const names[] = { RDX_KERNEL_IDS(RDX_KERNEL_NAME) };
+#undef RDX_KERNEL_NAME
+    return id >= 0 && id < kKernelIdCount ? names[id] : nullptr;
+}
+
+extern "C" int redux_debug_launched_kernels(redux_ctx_t *ctx, uint64_t *mask, int reset)
+{
+    if (!ctx || !mask) return REDUX_INVALID_INPUT;
+    *mask = reset ? ctx->kernels_launched.exchange(0) : ctx->kernels_launched.load();
     return REDUX_OK;
 }
 
@@ -930,21 +1004,24 @@ int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     const size_t smem = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * (pl.wide_table ? 4 : 2) + kTabPadBytes;
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_ENCODE);
+        int kid;
         if (pl.generic) {
             GenericJob g = generic_job(pl);
             g.in = d_in; g.in_off = d_in_off; g.n_blocks = n_blocks;
             g.slots = slots; g.slot_stride = pl.slot_stride; g.sizes = sizes; g.status = d_status;
             encode_generic_kernel<<<pl.gen_threads / kGenericThreads, kGenericThreads, generic_smem_bytes(pl.s), s>>>(g);
+            kid = pl.s <= kGenericSmemSymbolBits ? kEncGenericSmem : kEncGenericGlobal;
         }
         else if (pl.split) {
             DeviceState *d = find_dev(ctx, device);
-            int rc = launch_encode_split(ctx, d, pl, job, s);
+            int rc = launch_encode_split(ctx, d, pl, job, s, &kid);
             if (rc) return rc;
         }
-        else if (pl.warp)       launch_encode_warp(pl.cls, job, s);
-        else if (pl.aligned)    launch_encode_al(pl, job, grid, smem, s);
-        else if (pl.wide_table) launch_encode<uint32_t>(job, grid, smem, s);
-        else                    launch_encode<uint16_t>(job, grid, smem, s);
+        else if (pl.warp)       kid = launch_encode_warp(pl.cls, job, s);
+        else if (pl.aligned)    kid = launch_encode_al(pl, job, grid, smem, s);
+        else if (pl.wide_table) kid = launch_encode<uint32_t>(job, grid, smem, s);
+        else                    kid = launch_encode<uint16_t>(job, grid, smem, s);
+        ctx->note_kernel(kid);
     }
     ctx->launches++;
     CU_TRY(ctx, cudaGetLastError());
@@ -981,16 +1058,19 @@ int decode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     const size_t smem = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * (pl.wide_table ? 4 : 2) + kTabPadBytes;
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_DECODE);
+        int kid;
         if (pl.generic) {
             GenericJob g = generic_job(pl);
             g.in = d_comp; g.in_off = d_comp_off; g.n_blocks = n_blocks;
             g.raw = d_raw; g.raw_off = d_raw_off; g.raw_len = d_raw_lens; g.consumed = d_consumed; g.status = d_status;
             decode_generic_kernel<<<pl.gen_threads / kGenericThreads, kGenericThreads, generic_smem_bytes(pl.s), s>>>(g);
+            kid = pl.s <= kGenericSmemSymbolBits ? kDecGenericSmem : kDecGenericGlobal;
         }
-        else if (pl.warp)       launch_decode_warp(pl.cls, job, s);
-        else if (pl.aligned)    launch_decode_al(pl, job, grid, smem, s);
-        else if (pl.wide_table) launch_decode<uint32_t>(job, grid, smem, s);
-        else                    launch_decode<uint16_t>(job, grid, smem, s);
+        else if (pl.warp)       kid = launch_decode_warp(pl.cls, job, s);
+        else if (pl.aligned)    kid = launch_decode_al(pl, job, grid, smem, s);
+        else if (pl.wide_table) kid = launch_decode<uint32_t>(job, grid, smem, s);
+        else                    kid = launch_decode<uint16_t>(job, grid, smem, s);
+        ctx->note_kernel(kid);
     }
     ctx->launches++;
     CU_TRY(ctx, cudaGetLastError());
@@ -1191,6 +1271,7 @@ void for_each_device(redux_ctx *ctx, size_t nd, std::vector<int> &rcs, F fn)
         view.staging = ctx->staging; view.pool = ctx->pool;
         view.devs.push_back(ctx->devs[g]);
         rcs[g] = fn(&view, &view.devs[0], g);
+        ctx->kernels_launched.fetch_or(view.kernels_launched.load(std::memory_order_relaxed), std::memory_order_relaxed);
         ctx->devs[g] = view.devs[0];          // workspaces may have grown
         view.devs.clear(); view.pool = nullptr;
         errs[g] = view.last_error; launches[g] = view.launches; spans[g] = view.spans;

@@ -985,7 +985,7 @@ struct LaneDecoderAl {
         if ((int)PEEK | (int)is_eof | (int)(n > left)) {            // bitwise: one condition, one branch
             if (is_eof) st = -1;
             else if (n > left) { st = 1; left = 0; }
-            else st = 6;
+            else { st = 6; left -= n; }       // the reference read this symbol's bits before its write failed
             return false;
         }
         left -= n;

@@ -620,7 +620,7 @@ struct LaneDecoder {
             const Renorm<S> r = renorm<S>(low, high, c);
             const uint32_t n = r.n1 + r.k;
             if (!src.has(n)) { st = 1; src.left = 0; return; }    // Err(Eof) inside get_bit
-            if (t >= cap) { st = 6; return; }                     // sink full
+            if (t >= cap) { src.left -= n; st = 6; return; }      // sink full (the symbol's bits were read)
             const S chunk = (S)src.take64(n);
             S v1 = (r.n1 >= sizeof(S) * 8) ? (S)0 : (S)((value << r.n1) & maxv);
             v1 |= (S)(chunk >> r.k);

@@ -264,7 +264,7 @@ struct WarpDecoder {
             const Renorm<S> r = renorm<S>(low, high, c);                // src/codec.rs:140-158
             const uint32_t n = r.n1 + r.k;
             if (!src.has(n)) { st = 1; src.left = 0; return; }
-            if (t >= cap) { st = 6; return; }
+            if (t >= cap) { src.left -= n; st = 6; return; }           // sink full (the symbol's bits were read)
             const S chunk = (S)src.take64(n);
             S v1 = (r.n1 >= sizeof(S) * 8) ? (S)0 : (S)((value << r.n1) & maxv);
             v1 |= (S)(chunk >> r.k);
@@ -412,7 +412,7 @@ decode_warp_al_kernel(const LaneDecJob job)
         renorm_counts<C32>(l2, nh2, n1, n);
         const uint32_t k = n - n1;
         if (n > left) { st = 1; left = 0; break; }                 // Err(Eof) inside get_bit (:49-52)
-        if (t >= cap) { st = 6; break; }                           // sink full
+        if (t >= cap) { st = 6; left -= n; break; }                // sink full (the symbol's bits were read)
         left -= n;
         const uint32_t win = bw.win();
         const uint32_t A = __funnelshift_lc(win, V, n1);

@@ -85,6 +85,13 @@ extern "C" uint64_t emu_slot_stride(uint32_t f, uint32_t c, uint64_t max_block_l
     return lane_plan(f, c, max_block_len).slot_stride;
 }
 
+// The front end's lane_plan (the same header): out = {cls, wide_table, full_table, aligned, tcap}.
+extern "C" void emu_lane_plan(uint32_t f, uint32_t c, uint64_t max_block_len, uint32_t count0, int pretrained, uint32_t *out)
+{
+    const LanePlan pl = lane_plan(f, c, max_block_len, count0, pretrained != 0);
+    out[0] = (uint32_t)pl.cls; out[1] = pl.wide_table; out[2] = pl.full_table; out[3] = pl.aligned; out[4] = pl.tcap;
+}
+
 // force_wide_table: -1 = as the front end would choose, 0 = u16 entries, 1 = u32 entries; +2 = force the
 // generic kernels (redux_lane_codec.cuh) where the tuned ones (redux_lane_al.cuh) would be chosen
 namespace {

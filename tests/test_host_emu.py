@@ -34,11 +34,17 @@ def _build():
 
 @pytest.fixture(scope="module")
 def emu():
+    return load_emu()
+
+
+def load_emu():
     _build()
     L = C.CDLL(EMU_SO)
     u32, u64, vp, i32 = C.c_uint32, C.c_uint64, C.c_void_p, C.c_int
     L.emu_slot_stride.argtypes = [u32, u32, u64]
     L.emu_slot_stride.restype = u64
+    L.emu_lane_plan.argtypes = [u32, u32, u64, u32, i32, vp]
+    L.emu_lane_plan.restype = None
     L.emu_encode_lane.argtypes = [u32, u32, u64, i32, vp, vp, u64, vp, vp, vp]
     L.emu_decode_lane.argtypes = [u32, u32, u64, i32, vp, vp, u64, vp, vp, vp, vp, vp]
     L.emu_encode_lane_ex.argtypes = [u32, u32, u64, i32, vp, vp, vp, u64, vp, vp, vp]
