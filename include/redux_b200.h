@@ -257,7 +257,7 @@ void redux_debug_renorm(uint64_t low, uint64_t high, uint32_t code_bits,
 int redux_debug_lane_occupancy(int *enc_ctas_per_sm, int *dec_ctas_per_sm);
 
 /* Which coder kernels the context has launched: bit k of *mask is set when the kernel instantiation with ID k ran
- * since the last reset (reset != 0 clears the mask after reading it).  Lets tests check which of the ~45 kernels a
+ * since the last reset (reset != 0 clears the mask after reading it).  Lets tests check which of the 37 kernels a
  * parameter set, block length, capacity, model and schedule actually selects.  Costs one host-side atomic OR per
  * coder launch. */
 int redux_debug_launched_kernels(redux_ctx_t *ctx, uint64_t *mask, int reset);

@@ -46,48 +46,50 @@ extern "C" int redux_process_init(void)
 
 namespace {
 
-// One ID per kernel instantiation a launch_* function below can start (redux_debug_launched_kernels).  Lane
-// kernels: <table entry type, class, full tree values, code_bits == 32[, staged window refill]>; generic kernels:
-// Fenwick columns in shared memory (symbol_bits <= kGenericSmemSymbolBits) or in global memory.
-#define RDX_KERNEL_IDS(X) \
-    X(kEncNarrow,          "encode_lane_al<u16,Narrow,full,!c32>")       \
-    X(kEncWideU32,         "encode_lane_al<u32,Wide,full,!c32>")         \
-    X(kEncWideU16Full,     "encode_lane_al<u16,Wide,full,!c32>")         \
-    X(kEncWideU16,         "encode_lane_al<u16,Wide,!full,!c32>")        \
-    X(kEncWideU32C32,      "encode_lane_al<u32,Wide,full,c32>")          \
-    X(kEncWideU16FullC32,  "encode_lane_al<u16,Wide,full,c32>")          \
-    X(kEncWideU16C32,      "encode_lane_al<u16,Wide,!full,c32>")         \
-    X(kEncWideDU32,        "encode_lane_al<u32,WideD,full,!c32>")        \
-    X(kEncWideDU16Full,    "encode_lane_al<u16,WideD,full,!c32>")        \
-    X(kEncWideDU16,        "encode_lane_al<u16,WideD,!full,!c32>")       \
-    X(kEncWideDU32C32,     "encode_lane_al<u32,WideD,full,c32>")         \
-    X(kEncWideDU16FullC32, "encode_lane_al<u16,WideD,full,c32>")         \
-    X(kEncWideDU16C32,     "encode_lane_al<u16,WideD,!full,c32>")        \
-    X(kDecNarrowStg,       "decode_lane_al<u16,Narrow,full,!c32,stg>")   \
-    X(kDecNarrow,          "decode_lane_al<u16,Narrow,full,!c32>")       \
-    X(kDecWideU32,         "decode_lane_al<u32,Wide,full,!c32>")         \
-    X(kDecWideU16Full,     "decode_lane_al<u16,Wide,full,!c32>")         \
-    X(kDecWideU16,         "decode_lane_al<u16,Wide,!full,!c32>")        \
-    X(kDecWideU32C32,      "decode_lane_al<u32,Wide,full,c32>")          \
-    X(kDecWideU16FullC32,  "decode_lane_al<u16,Wide,full,c32>")          \
-    X(kDecWideU16C32,      "decode_lane_al<u16,Wide,!full,c32>")         \
-    X(kDecWideDU32,        "decode_lane_al<u32,WideD,full,!c32>")        \
-    X(kDecWideDU16Full,    "decode_lane_al<u16,WideD,full,!c32>")        \
-    X(kDecWideDU16,        "decode_lane_al<u16,WideD,!full,!c32>")       \
-    X(kDecWideDU32C32,     "decode_lane_al<u32,WideD,full,c32>")         \
-    X(kDecWideDU16FullC32, "decode_lane_al<u16,WideD,full,c32>")         \
-    X(kDecWideDU16C32,     "decode_lane_al<u16,WideD,!full,c32>")        \
-    X(kEncHugeU16,         "encode_lane<u16,Huge>")                      \
-    X(kEncHugeU32,         "encode_lane<u32,Huge>")                      \
-    X(kDecHugeU16,         "decode_lane<u16,Huge>")                      \
-    X(kDecHugeU32,         "decode_lane<u32,Huge>")                      \
-    X(kEncWarpNarrow,      "encode_warp<Narrow>")                        \
-    X(kEncWarpWide,        "encode_warp<Wide>")                          \
-    X(kEncWarpHuge,        "encode_warp<Huge>")                          \
-    X(kDecWarpNarrow,      "decode_warp_al<Narrow,!c32>")                \
-    X(kDecWarpWide,        "decode_warp_al<Wide,!c32>")                  \
-    X(kDecWarpWideC32,     "decode_warp_al<Wide,c32>")                   \
-    X(kDecWarpHuge,        "decode_warp<Huge>")                          \
+// Every coder kernel the dispatcher can launch, each listed once: its KernelId (redux_debug_launched_kernels), its
+// name, and for the lane and warp kernels the instantiation and (lane kernels) the table entry type that sizes its
+// dynamic shared memory.  Enum, names, shared-memory limits and the launch switches below are generated from these
+// lists.  Lane kernels: <table entry type, class, full tree values, code_bits == 32[, staged window refill]>; NARROW
+// (c + f <= 30) implies at most 16,126 updates, so u16 entries with full values; plain WIDE (totals reach 349,525)
+// always takes u32 entries (lane_plan).
+#define RDX_LANE_ENCODERS(X) \
+    X(kEncNarrow,          "encode_lane_al<u16,Narrow,full,!c32>",     (encode_lane_al_kernel<uint16_t, kNarrow, true, false>), uint16_t)        \
+    X(kEncWideU32,         "encode_lane_al<u32,Wide,full,!c32>",       (encode_lane_al_kernel<uint32_t, kWide, true, false>), uint32_t)          \
+    X(kEncWideU32C32,      "encode_lane_al<u32,Wide,full,c32>",        (encode_lane_al_kernel<uint32_t, kWide, true, true>), uint32_t)           \
+    X(kEncWideDU32,        "encode_lane_al<u32,WideD,full,!c32>",      (encode_lane_al_kernel<uint32_t, kWideD, true, false>), uint32_t)         \
+    X(kEncWideDU16Full,    "encode_lane_al<u16,WideD,full,!c32>",      (encode_lane_al_kernel<uint16_t, kWideD, true, false>), uint16_t)         \
+    X(kEncWideDU16,        "encode_lane_al<u16,WideD,!full,!c32>",     (encode_lane_al_kernel<uint16_t, kWideD, false, false>), uint16_t)        \
+    X(kEncWideDU32C32,     "encode_lane_al<u32,WideD,full,c32>",       (encode_lane_al_kernel<uint32_t, kWideD, true, true>), uint32_t)          \
+    X(kEncWideDU16FullC32, "encode_lane_al<u16,WideD,full,c32>",       (encode_lane_al_kernel<uint16_t, kWideD, true, true>), uint16_t)          \
+    X(kEncWideDU16C32,     "encode_lane_al<u16,WideD,!full,c32>",      (encode_lane_al_kernel<uint16_t, kWideD, false, true>), uint16_t)         \
+    X(kEncHugeU16,         "encode_lane<u16,Huge>",                    (encode_lane_kernel<uint16_t, kHuge>), uint16_t)                                  \
+    X(kEncHugeU32,         "encode_lane<u32,Huge>",                    (encode_lane_kernel<uint32_t, kHuge>), uint32_t)
+// The narrow decoder comes twice: code_bits <= 16 runs the STAGED window refill (redux_lane_al.cuh, BitWindow).
+#define RDX_LANE_DECODERS(X) \
+    X(kDecNarrowStg,       "decode_lane_al<u16,Narrow,full,!c32,stg>", (decode_lane_al_kernel<uint16_t, kNarrow, true, false, true>), uint16_t)   \
+    X(kDecNarrow,          "decode_lane_al<u16,Narrow,full,!c32>",     (decode_lane_al_kernel<uint16_t, kNarrow, true, false, false>), uint16_t)  \
+    X(kDecWideU32,         "decode_lane_al<u32,Wide,full,!c32>",       (decode_lane_al_kernel<uint32_t, kWide, true, false, false>), uint32_t)    \
+    X(kDecWideU32C32,      "decode_lane_al<u32,Wide,full,c32>",        (decode_lane_al_kernel<uint32_t, kWide, true, true, false>), uint32_t)     \
+    X(kDecWideDU32,        "decode_lane_al<u32,WideD,full,!c32>",      (decode_lane_al_kernel<uint32_t, kWideD, true, false, false>), uint32_t)   \
+    X(kDecWideDU16Full,    "decode_lane_al<u16,WideD,full,!c32>",      (decode_lane_al_kernel<uint16_t, kWideD, true, false, false>), uint16_t)   \
+    X(kDecWideDU16,        "decode_lane_al<u16,WideD,!full,!c32>",     (decode_lane_al_kernel<uint16_t, kWideD, false, false, false>), uint16_t)  \
+    X(kDecWideDU32C32,     "decode_lane_al<u32,WideD,full,c32>",       (decode_lane_al_kernel<uint32_t, kWideD, true, true, false>), uint32_t)    \
+    X(kDecWideDU16FullC32, "decode_lane_al<u16,WideD,full,c32>",       (decode_lane_al_kernel<uint16_t, kWideD, true, true, false>), uint16_t)    \
+    X(kDecWideDU16C32,     "decode_lane_al<u16,WideD,!full,c32>",      (decode_lane_al_kernel<uint16_t, kWideD, false, true, false>), uint16_t)   \
+    X(kDecHugeU16,         "decode_lane<u16,Huge>",                    (decode_lane_kernel<uint16_t, kHuge>), uint16_t)                                  \
+    X(kDecHugeU32,         "decode_lane<u32,Huge>",                    (decode_lane_kernel<uint32_t, kHuge>), uint32_t)
+#define RDX_WARP_ENCODERS(X) \
+    X(kEncWarpNarrow,      "encode_warp<Narrow>",                      encode_warp_kernel<kNarrow>)                  \
+    X(kEncWarpWide,        "encode_warp<Wide>",                        encode_warp_kernel<kWide>)                    \
+    X(kEncWarpHuge,        "encode_warp<Huge>",                        encode_warp_kernel<kHuge>)
+#define RDX_WARP_DECODERS(X) \
+    X(kDecWarpNarrow,      "decode_warp_al<Narrow,!c32>",              (decode_warp_al_kernel<kNarrow, false>))      \
+    X(kDecWarpWide,        "decode_warp_al<Wide,!c32>",                (decode_warp_al_kernel<kWide, false>))        \
+    X(kDecWarpWideC32,     "decode_warp_al<Wide,c32>",                 (decode_warp_al_kernel<kWide, true>))         \
+    X(kDecWarpHuge,        "decode_warp<Huge>",                        decode_warp_kernel<kHuge>)
+// Launched by hand (their launch shapes differ): the split coder and the generic kernels, whose Fenwick columns are in
+// shared memory (symbol_bits <= kGenericSmemSymbolBits) or in global memory.
+#define RDX_OTHER_KERNELS(X) \
     X(kSplitNarrow,        "split_coder<Narrow,!c32>")                   \
     X(kSplitWide,          "split_coder<Wide,!c32>")                     \
     X(kSplitWideC32,       "split_coder<Wide,c32>")                      \
@@ -95,8 +97,10 @@ namespace {
     X(kEncGenericGlobal,   "encode_generic<global>")                     \
     X(kDecGenericSmem,     "decode_generic<smem>")                       \
     X(kDecGenericGlobal,   "decode_generic<global>")
-#define RDX_KERNEL_ENUM(id, name) id,
-enum KernelId : int { RDX_KERNEL_IDS(RDX_KERNEL_ENUM) kKernelIdCount };
+#define RDX_ALL_KERNELS(X) \
+    RDX_LANE_ENCODERS(X) RDX_LANE_DECODERS(X) RDX_WARP_ENCODERS(X) RDX_WARP_DECODERS(X) RDX_OTHER_KERNELS(X)
+#define RDX_KERNEL_ENUM(id, ...) id,
+enum KernelId : int { RDX_ALL_KERNELS(RDX_KERNEL_ENUM) kKernelIdCount };
 #undef RDX_KERNEL_ENUM
 static_assert(kKernelIdCount <= 64, "the launched-kernel mask is 64 bits wide");
 
@@ -297,39 +301,19 @@ cudaError_t allow_smem(K kernel, size_t bytes)
     return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
+// Dynamic shared memory of a lane kernel: one table of TW entries per warp + the pad (redux_lane_codec.cuh)
+template <typename TW>
+constexpr size_t lane_smem() { return (size_t)kLaneWarpsPerCta * kTabNodes * 32 * sizeof(TW) + kTabPadBytes; }
+
 cudaError_t configure_kernels()
 {
-    const size_t s16 = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * 2 + kTabPadBytes;
-    const size_t s32 = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * 4 + kTabPadBytes;
     cudaError_t e;
-#define RDX_CFG(K, BYTES) if ((e = allow_smem(K, BYTES)) != cudaSuccess) return e;
-    // generic kernels (redux_lane_codec.cuh): code_bits > 32 only
-    RDX_CFG((encode_lane_kernel<uint16_t, kHuge>), s16)   RDX_CFG((encode_lane_kernel<uint32_t, kHuge>), s32)
-    RDX_CFG((decode_lane_kernel<uint16_t, kHuge>), s16)   RDX_CFG((decode_lane_kernel<uint32_t, kHuge>), s32)
-    // tuned kernels (redux_lane_al.cuh): <entry type, class, full tree values, code_bits == 32>.
-    // NARROW (c + f <= 30) implies at most 16,126 updates: always u16 entries with full values.
-    // The narrow decoder comes twice: code_bits <= 16 runs the STAGED window refill (redux_lane_al.cuh, BitWindow).
-    RDX_CFG((encode_lane_al_kernel<uint16_t, kNarrow, true, false>), s16)
-    RDX_CFG((decode_lane_al_kernel<uint16_t, kNarrow, true, false, true>), s16)
-    RDX_CFG((decode_lane_al_kernel<uint16_t, kNarrow, true, false, false>), s16)
-#define RDX_CFG_WIDE(C32) \
-    RDX_CFG((encode_lane_al_kernel<uint16_t, kWide, true, C32>), s16)  RDX_CFG((decode_lane_al_kernel<uint16_t, kWide, true, C32, false>), s16) \
-    RDX_CFG((encode_lane_al_kernel<uint16_t, kWide, false, C32>), s16) RDX_CFG((decode_lane_al_kernel<uint16_t, kWide, false, C32, false>), s16) \
-    RDX_CFG((encode_lane_al_kernel<uint32_t, kWide, true, C32>), s32)  RDX_CFG((decode_lane_al_kernel<uint32_t, kWide, true, C32, false>), s32)
-    RDX_CFG_WIDE(false) RDX_CFG_WIDE(true)
-#undef RDX_CFG_WIDE
-    // WIDE_D (double-reciprocal division, redux_common.cuh MagicD)
-#define RDX_CFG_WIDED(FULL, C32) \
-    RDX_CFG((encode_lane_al_kernel<uint16_t, kWideD, FULL, C32>), s16) RDX_CFG((decode_lane_al_kernel<uint16_t, kWideD, FULL, C32, false>), s16)
-    RDX_CFG_WIDED(true, false) RDX_CFG_WIDED(true, true) RDX_CFG_WIDED(false, false) RDX_CFG_WIDED(false, true)
-#undef RDX_CFG_WIDED
-    RDX_CFG((encode_lane_al_kernel<uint32_t, kWideD, true, false>), s32) RDX_CFG((decode_lane_al_kernel<uint32_t, kWideD, true, false, false>), s32)
-    RDX_CFG((encode_lane_al_kernel<uint32_t, kWideD, true, true>), s32)  RDX_CFG((decode_lane_al_kernel<uint32_t, kWideD, true, true, false>), s32)
-    // generic kernels: Fenwick columns of alphabets up to 7 bits in shared memory (66 KB per CTA at 7 bits)
-    RDX_CFG(encode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits))
-    RDX_CFG(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits))
+#define RDX_CFG(id, name, kernel, TW) if ((e = allow_smem(kernel, lane_smem<TW>())) != cudaSuccess) return e;
+    RDX_LANE_ENCODERS(RDX_CFG) RDX_LANE_DECODERS(RDX_CFG)
 #undef RDX_CFG
-    return cudaSuccess;
+    // generic kernels: Fenwick columns of alphabets up to 7 bits in shared memory (66 KB per CTA at 7 bits)
+    if ((e = allow_smem(encode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits))) != cudaSuccess) return e;
+    return allow_smem(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits));
 }
 
 // Shape of one launch derived from the parameters and the longest block.
@@ -356,17 +340,13 @@ struct Plan {
 // wins (29 corpus files: 31 MB/s against 62 lane and 86 split), so AUTO falls back to the lane mapping, not to it.
 constexpr uint64_t kWarpAutoMaxBlocks = 512;
 
-bool choose_warp(const redux_ctx *ctx, uint64_t)
-{
-    return ctx->sched == REDUX_SCHED_WARP || ctx->sched == REDUX_SCHED_SPLIT;
-}
-
-// Decode: REDUX_SCHED_AUTO always takes the lane mapping.  Since the decoder's output sink is phase-free (round 2) a
-// lane decodes every class faster than a cooperating warp at every batch size measured, ragged corpus batches
-// included (profiles/r02_small_batches_corpora.json: 29 files 28.6 vs 20.0 MB/s, 12 x 1 MiB 51.3 vs 35.9 MB/s at
-// (8,14,16); 15.2 vs 13.6 and 27.3 vs 24.3 MB/s at (8,30,32); one stream 4.9 vs 3.4 / 2.6 vs 2.3 MB/s).  The warp
-// decoder stays selectable (REDUX_SCHED_WARP / REDUX_SCHED_SPLIT).
-bool choose_warp_decode(const redux_ctx *ctx, uint64_t)
+// One stream per warp, encode and decode: only when the caller asks for it (REDUX_SCHED_WARP / REDUX_SCHED_SPLIT; the
+// split schedule decodes with the warp mapping).  REDUX_SCHED_AUTO decodes with the lane mapping: since the decoder's
+// output sink is phase-free (round 2) a lane decodes every class faster than a cooperating warp at every batch size
+// measured, ragged corpus batches included (profiles/r02_small_batches_corpora.json: 29 files 28.6 vs 20.0 MB/s,
+// 12 x 1 MiB 51.3 vs 35.9 MB/s at (8,14,16); 15.2 vs 13.6 and 27.3 vs 24.3 MB/s at (8,30,32); one stream 4.9 vs 3.4 /
+// 2.6 vs 2.3 MB/s).
+bool choose_warp(const redux_ctx *ctx)
 {
     return ctx->sched == REDUX_SCHED_WARP || ctx->sched == REDUX_SCHED_SPLIT;
 }
@@ -524,84 +504,68 @@ GenericJob generic_job(const Plan &pl)
     return g;
 }
 
-// Every launch_* function returns the KernelId of the kernel it started.
-// code_bits > 32: the generic kernels
-template <typename TW>
-int launch_encode(const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+// The fields LaneEncJob and LaneDecJob take from the plan.
+template <typename J>
+void set_plan_fields(J &job, const Plan &pl, const void *magic)
 {
-    encode_lane_kernel<TW, kHuge><<<grid, kLaneThreads, smem, s>>>(job);
-    return sizeof(TW) == 4 ? kEncHugeU32 : kEncHugeU16;
-}
-template <typename TW>
-int launch_decode(const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
-{
-    decode_lane_kernel<TW, kHuge><<<grid, kLaneThreads, smem, s>>>(job);
-    return sizeof(TW) == 4 ? kDecHugeU32 : kDecHugeU16;
+    job.magic = lane_magic(pl, magic); job.f = pl.f; job.c = pl.c; job.tcap = pl.tcap;
+    job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
+    job.init_tree = pl.pretrained ? pl.gen_init : nullptr; job.count0 = pl.count0; job.eof_freq = pl.eof_freq;
+    job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
 }
 
-// code_bits <= 32: the tuned kernels
-template <bool C32>
-int launch_encode_wide(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+// The lane or warp coder kernel a plan runs (the split and generic kernels are launched on their own).
+KernelId pick_encoder(const Plan &pl)
 {
-    if (pl.wide_table)      { encode_lane_al_kernel<uint32_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideU32C32 : kEncWideU32; }
-    else if (pl.full_table) { encode_lane_al_kernel<uint16_t, kWide, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideU16FullC32 : kEncWideU16Full; }
-    else                    { encode_lane_al_kernel<uint16_t, kWide, false, C32><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kEncWideU16C32 : kEncWideU16; }
+    const bool c32 = pl.c == 32;
+    if (pl.warp) return pl.cls == kNarrow ? kEncWarpNarrow : pl.cls == kWide ? kEncWarpWide : kEncWarpHuge;
+    if (!pl.aligned) return pl.wide_table ? kEncHugeU32 : kEncHugeU16;
+    if (pl.lane_cls == kNarrow) return kEncNarrow;
+    if (pl.lane_cls == kWide) return c32 ? kEncWideU32C32 : kEncWideU32;
+    if (pl.wide_table) return c32 ? kEncWideDU32C32 : kEncWideDU32;
+    if (pl.full_table) return c32 ? kEncWideDU16FullC32 : kEncWideDU16Full;
+    return c32 ? kEncWideDU16C32 : kEncWideDU16;
 }
-template <bool C32>
-int launch_decode_wide(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+KernelId pick_decoder(const Plan &pl)
 {
-    if (pl.wide_table)      { decode_lane_al_kernel<uint32_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideU32C32 : kDecWideU32; }
-    else if (pl.full_table) { decode_lane_al_kernel<uint16_t, kWide, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideU16FullC32 : kDecWideU16Full; }
-    else                    { decode_lane_al_kernel<uint16_t, kWide, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kDecWideU16C32 : kDecWideU16; }
+    const bool c32 = pl.c == 32;
+    if (pl.warp) return pl.cls == kNarrow ? kDecWarpNarrow : pl.cls == kHuge ? kDecWarpHuge : c32 ? kDecWarpWideC32 : kDecWarpWide;
+    if (!pl.aligned) return pl.wide_table ? kDecHugeU32 : kDecHugeU16;
+    if (pl.lane_cls == kNarrow) return pl.c <= 16 ? kDecNarrowStg : kDecNarrow;
+    if (pl.lane_cls == kWide) return c32 ? kDecWideU32C32 : kDecWideU32;
+    if (pl.wide_table) return c32 ? kDecWideDU32C32 : kDecWideDU32;
+    if (pl.full_table) return c32 ? kDecWideDU16FullC32 : kDecWideDU16Full;
+    return c32 ? kDecWideDU16C32 : kDecWideDU16;
 }
-template <bool C32>
-int launch_encode_wided(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
+
+// Starts lane or warp kernel `id` on job.n_blocks streams; false if `id` is not one of them.
+#define RDX_LAUNCH_LANE(id, name, kernel, TW) case id: kernel<<<lane_grid, kLaneThreads, lane_smem<TW>(), s>>>(job); return true;
+#define RDX_LAUNCH_WARP(id, name, kernel) case id: kernel<<<warp_grid, kWarpCtaThreads, 0, s>>>(job); return true;
+bool launch_coder(KernelId id, const LaneEncJob &job, cudaStream_t s)
 {
-    if (pl.wide_table)      { encode_lane_al_kernel<uint32_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideDU32C32 : kEncWideDU32; }
-    else if (pl.full_table) { encode_lane_al_kernel<uint16_t, kWideD, true, C32><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kEncWideDU16FullC32 : kEncWideDU16Full; }
-    else                    { encode_lane_al_kernel<uint16_t, kWideD, false, C32><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kEncWideDU16C32 : kEncWideDU16; }
-}
-template <bool C32>
-int launch_decode_wided(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
-{
-    if (pl.wide_table)      { decode_lane_al_kernel<uint32_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideDU32C32 : kDecWideDU32; }
-    else if (pl.full_table) { decode_lane_al_kernel<uint16_t, kWideD, true, C32, false><<<grid, kLaneThreads, smem, s>>>(job);  return C32 ? kDecWideDU16FullC32 : kDecWideDU16Full; }
-    else                    { decode_lane_al_kernel<uint16_t, kWideD, false, C32, false><<<grid, kLaneThreads, smem, s>>>(job); return C32 ? kDecWideDU16C32 : kDecWideDU16; }
-}
-int launch_encode_al(const Plan &pl, const LaneEncJob &job, uint32_t grid, size_t smem, cudaStream_t s)
-{
-    if (pl.lane_cls == kWideD) return pl.c == 32 ? launch_encode_wided<true>(pl, job, grid, smem, s) : launch_encode_wided<false>(pl, job, grid, smem, s);
-    if (pl.cls == kNarrow) { encode_lane_al_kernel<uint16_t, kNarrow, true, false><<<grid, kLaneThreads, smem, s>>>(job); return kEncNarrow; }
-    return pl.c == 32 ? launch_encode_wide<true>(pl, job, grid, smem, s) : launch_encode_wide<false>(pl, job, grid, smem, s);
-}
-int launch_decode_al(const Plan &pl, const LaneDecJob &job, uint32_t grid, size_t smem, cudaStream_t s)
-{
-    if (pl.lane_cls == kWideD) return pl.c == 32 ? launch_decode_wided<true>(pl, job, grid, smem, s) : launch_decode_wided<false>(pl, job, grid, smem, s);
-    if (pl.cls == kNarrow) {
-        if (pl.c <= 16) { decode_lane_al_kernel<uint16_t, kNarrow, true, false, true><<<grid, kLaneThreads, smem, s>>>(job);  return kDecNarrowStg; }
-        else            { decode_lane_al_kernel<uint16_t, kNarrow, true, false, false><<<grid, kLaneThreads, smem, s>>>(job); return kDecNarrow; }
+    const uint32_t lane_grid = (uint32_t)((job.n_blocks + kLaneThreads - 1) / kLaneThreads);
+    const uint32_t warp_grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
+    switch (id) {
+    RDX_LANE_ENCODERS(RDX_LAUNCH_LANE)
+    RDX_WARP_ENCODERS(RDX_LAUNCH_WARP)
+    default: return false;
     }
-    return pl.c == 32 ? launch_decode_wide<true>(pl, job, grid, smem, s) : launch_decode_wide<false>(pl, job, grid, smem, s);
 }
-
-int launch_encode_warp(int cls, const LaneEncJob &job, cudaStream_t s)
+bool launch_coder(KernelId id, const LaneDecJob &job, cudaStream_t s)
 {
-    const uint32_t grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
-    if (cls == kNarrow)    { encode_warp_kernel<kNarrow><<<grid, kWarpCtaThreads, 0, s>>>(job); return kEncWarpNarrow; }
-    else if (cls == kWide) { encode_warp_kernel<kWide><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kEncWarpWide; }
-    else                   { encode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kEncWarpHuge; }
+    const uint32_t lane_grid = (uint32_t)((job.n_blocks + kLaneThreads - 1) / kLaneThreads);
+    const uint32_t warp_grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
+    switch (id) {
+    RDX_LANE_DECODERS(RDX_LAUNCH_LANE)
+    RDX_WARP_DECODERS(RDX_LAUNCH_WARP)
+    default: return false;
+    }
 }
-int launch_decode_warp(int cls, const LaneDecJob &job, cudaStream_t s)
-{
-    const uint32_t grid = (uint32_t)((job.n_blocks + kWarpCtaWarps - 1) / kWarpCtaWarps);
-    if (cls == kNarrow)     { decode_warp_al_kernel<kNarrow, false><<<grid, kWarpCtaThreads, 0, s>>>(job); return kDecWarpNarrow; }
-    else if (cls == kHuge)  { decode_warp_kernel<kHuge><<<grid, kWarpCtaThreads, 0, s>>>(job);            return kDecWarpHuge; }
-    else if (job.c == 32)   { decode_warp_al_kernel<kWide, true><<<grid, kWarpCtaThreads, 0, s>>>(job);    return kDecWarpWideC32; }
-    else                    { decode_warp_al_kernel<kWide, false><<<grid, kWarpCtaThreads, 0, s>>>(job);   return kDecWarpWide; }
-}
+#undef RDX_LAUNCH_LANE
+#undef RDX_LAUNCH_WARP
 
 // Split encoder: model phase over all chunks of all streams, then one coder warp per stream (its KernelId in *kid).
-int launch_encode_split(redux_ctx *ctx, DeviceState *d, const Plan &pl, const LaneEncJob &job, cudaStream_t s, int *kid)
+int launch_encode_split(redux_ctx *ctx, DeviceState *d, const Plan &pl, const LaneEncJob &job, cudaStream_t s, KernelId *kid)
 {
     if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
     SplitJob sj;
@@ -773,8 +737,8 @@ extern "C" int redux_debug_lane_occupancy(int *enc_ctas_per_sm, int *dec_ctas_pe
 
 extern "C" const char *redux_debug_kernel_name(int id)
 {
-#define RDX_KERNEL_NAME(id, name) name,
-    static const char *const names[] = { RDX_KERNEL_IDS(RDX_KERNEL_NAME) };
+#define RDX_KERNEL_NAME(id, name, ...) name,
+    static const char *const names[] = { RDX_ALL_KERNELS(RDX_KERNEL_NAME) };
 #undef RDX_KERNEL_NAME
     return id >= 0 && id < kKernelIdCount ? names[id] : nullptr;
 }
@@ -996,15 +960,10 @@ int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     job.in = d_in; job.in_off = d_in_off; job.n_blocks = n_blocks;
     job.slots = slots; job.slot_stride = pl.slot_stride;
     job.sizes = sizes; job.status = d_status;
-    job.magic = lane_magic(pl, magic); job.f = pl.f; job.c = pl.c; job.tcap = pl.tcap;
-    job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
-    job.init_tree = pl.pretrained ? pl.gen_init : nullptr; job.count0 = pl.count0; job.eof_freq = pl.eof_freq;
-    job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
-    const uint32_t grid = (uint32_t)((n_blocks + kLaneThreads - 1) / kLaneThreads);
-    const size_t smem = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * (pl.wide_table ? 4 : 2) + kTabPadBytes;
+    set_plan_fields(job, pl, magic);
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_ENCODE);
-        int kid;
+        KernelId kid;
         if (pl.generic) {
             GenericJob g = generic_job(pl);
             g.in = d_in; g.in_off = d_in_off; g.n_blocks = n_blocks;
@@ -1017,10 +976,10 @@ int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
             int rc = launch_encode_split(ctx, d, pl, job, s, &kid);
             if (rc) return rc;
         }
-        else if (pl.warp)       kid = launch_encode_warp(pl.cls, job, s);
-        else if (pl.aligned)    kid = launch_encode_al(pl, job, grid, smem, s);
-        else if (pl.wide_table) kid = launch_encode<uint32_t>(job, grid, smem, s);
-        else                    kid = launch_encode<uint16_t>(job, grid, smem, s);
+        else {
+            kid = pick_encoder(pl);
+            if (!launch_coder(kid, job, s)) return fail(ctx, REDUX_CUDA_ERROR, "no encoder for the plan");
+        }
         ctx->note_kernel(kid);
     }
     ctx->launches++;
@@ -1050,15 +1009,11 @@ int decode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     LaneDecJob job;
     job.comp = d_comp; job.comp_off = d_comp_off; job.n_blocks = n_blocks;
     job.raw = d_raw; job.raw_off = d_raw_off; job.raw_len = d_raw_lens; job.consumed = d_consumed;
-    job.status = d_status; job.magic = lane_magic(pl, magic); job.f = pl.f; job.c = pl.c; job.tcap = pl.tcap;
-    job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
-    job.init_tree = pl.pretrained ? pl.gen_init : nullptr; job.count0 = pl.count0; job.eof_freq = pl.eof_freq;
-    job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
-    const uint32_t grid = (uint32_t)((n_blocks + kLaneThreads - 1) / kLaneThreads);
-    const size_t smem = (size_t)kLaneWarpsPerCta * kTabNodes * 32 * (pl.wide_table ? 4 : 2) + kTabPadBytes;
+    job.status = d_status;
+    set_plan_fields(job, pl, magic);
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_DECODE);
-        int kid;
+        KernelId kid;
         if (pl.generic) {
             GenericJob g = generic_job(pl);
             g.in = d_comp; g.in_off = d_comp_off; g.n_blocks = n_blocks;
@@ -1066,10 +1021,10 @@ int decode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
             decode_generic_kernel<<<pl.gen_threads / kGenericThreads, kGenericThreads, generic_smem_bytes(pl.s), s>>>(g);
             kid = pl.s <= kGenericSmemSymbolBits ? kDecGenericSmem : kDecGenericGlobal;
         }
-        else if (pl.warp)       kid = launch_decode_warp(pl.cls, job, s);
-        else if (pl.aligned)    kid = launch_decode_al(pl, job, grid, smem, s);
-        else if (pl.wide_table) kid = launch_decode<uint32_t>(job, grid, smem, s);
-        else                    kid = launch_decode<uint16_t>(job, grid, smem, s);
+        else {
+            kid = pick_decoder(pl);
+            if (!launch_coder(kid, job, s)) return fail(ctx, REDUX_CUDA_ERROR, "no decoder for the plan");
+        }
         ctx->note_kernel(kid);
     }
     ctx->launches++;
@@ -1090,7 +1045,7 @@ extern "C" int redux_encode_batch_device(redux_ctx_t *ctx, int device, void *str
     if ((rc = check_kind(ctx, model_kind))) return rc;
     Plan pl;
     if ((rc = make_plan(ctx, params, max_block_len, &pl))) return rc;
-    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx, n_blocks);
+    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx);
     pl.split = !pl.generic && !pl.pretrained && choose_split(ctx, n_blocks, pl.cls, max_block_len);
     DeviceState *d = find_dev(ctx, device);
     if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
@@ -1127,7 +1082,7 @@ extern "C" int redux_decode_batch_device(redux_ctx_t *ctx, int device, void *str
     if ((rc = check_kind(ctx, model_kind))) return rc;
     Plan pl;
     if ((rc = make_plan(ctx, params, max_block_len, &pl))) return rc;
-    pl.warp = !pl.generic && !pl.pretrained && choose_warp_decode(ctx, n_blocks);
+    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx);
     DeviceState *d = find_dev(ctx, device);
     if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
     if (n_blocks == 0) return REDUX_OK;
@@ -1440,11 +1395,10 @@ struct EncShardOut {
     uint64_t total = 0;
 };
 
-int encode_shard(redux_ctx *ctx, DeviceState *d, int kind, const redux_params_t *p, const uint8_t *in,
+int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const uint8_t *in,
                  const uint64_t *in_off, Shard sh, uint8_t *out, uint64_t out_cap,
                  int32_t *status, EncShardOut *res, ShardSync *sync, size_t g_index)
 {
-    (void)kind;
     const bool streaming = !sync || g_index == 0;          // the shard's base is known up front
     Trace tr;
     DeviceGuard g(d->device);
@@ -1459,7 +1413,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, int kind, const redux_params_t 
     Plan pl;
     int rc = make_plan(ctx, p, max_len, &pl);
     if (rc) return rc;
-    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx, sh.count);
+    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx);
     pl.split = !pl.generic && !pl.pretrained && choose_split(ctx, sh.count, pl.cls, max_len);
     // chunks of the generic path would share the Fenwick columns (and split chunks the range workspace): one chunk
     res->chunks = (pl.generic || pl.split) ? std::vector<Shard>{{0, sh.count}} : make_chunks(sh.count, +1);
@@ -1628,7 +1582,7 @@ extern "C" int redux_encode_batch(redux_ctx_t *ctx, int model_kind, const redux_
     std::vector<int> rcs(nd, REDUX_OK);
     ShardSync sync(nd);
     for_each_device(ctx, nd, rcs, [&](redux_ctx *view, DeviceState *d, size_t g) {
-        const int r = encode_shard(view, d, model_kind, params, in, in_offsets, shards[g], out, out_capacity,
+        const int r = encode_shard(view, d, params, in, in_offsets, shards[g], out, out_capacity,
                                    status + shards[g].first, &res[g], nd > 1 ? &sync : nullptr, g);
         if (r != REDUX_OK) sync.abort();
         return r;
@@ -1655,11 +1609,10 @@ namespace {
 // One device's shard of redux_decode_batch: chunk k runs
 //     H2D(compressed bytes) -> decode -> D2H(decoded slots) -> D2H(lengths, consumed, status)
 // (H2D on the shared h2d stream, the rest on the chunk's own stream); nothing depends on another chunk or shard.
-int decode_shard(redux_ctx *ctx, DeviceState *d, int kind, const redux_params_t *p, const uint8_t *comp,
+int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const uint8_t *comp,
                  const uint64_t *comp_off, Shard sh, uint8_t *raw, const uint64_t *raw_off,
                  uint64_t *raw_lens, uint64_t *consumed, int32_t *status)
 {
-    (void)kind;
     Trace tr;
     DeviceGuard g(d->device);
     const uint64_t cbase = comp_off[sh.first], cbytes = comp_off[sh.first + sh.count] - cbase;
@@ -1678,7 +1631,7 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, int kind, const redux_params_t 
     Plan pl;
     int rc = make_plan(ctx, p, max_len, &pl);
     if (rc) return rc;
-    pl.warp = !pl.generic && !pl.pretrained && choose_warp_decode(ctx, sh.count);
+    pl.warp = !pl.generic && !pl.pretrained && choose_warp(ctx);
     const std::vector<Shard> chunks = pl.generic ? std::vector<Shard>{{0, sh.count}} : make_chunks(sh.count, -1);
     const size_t nc = chunks.size();
     CU_TRY(ctx, d->st_in.reserve(cbytes + 32));
@@ -1797,7 +1750,7 @@ extern "C" int redux_decode_batch(redux_ctx_t *ctx, int model_kind, const redux_
     std::vector<Shard> shards = make_shards(n_blocks, nd);
     std::vector<int> rcs(nd, REDUX_OK);
     for_each_device(ctx, nd, rcs, [&](redux_ctx *view, DeviceState *d, size_t g) {
-        return decode_shard(view, d, model_kind, params, comp, comp_offsets, shards[g], raw, raw_offsets,
+        return decode_shard(view, d, params, comp, comp_offsets, shards[g], raw, raw_offsets,
                             raw_lens, consumed, status);
     });
     for (size_t g = 0; g < nd; ++g) if (rcs[g]) return rcs[g];

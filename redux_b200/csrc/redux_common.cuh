@@ -232,6 +232,9 @@ RDX_HD LanePlan lane_plan(uint32_t f, uint32_t c, uint64_t max_block_len, uint32
     pl.full_table = pretrained || pl.wide_table || updates + 256 <= 65535;   // cum(i) <= 256 + updates must fit u16
     // every total of the launch below the bound: the double-reciprocal division (see MagicD)
     if (pl.cls == kWide && (uint64_t)count0 + updates < kWideDMaxCount) pl.cls = kWideD;
+    // plain WIDE: totals reach kWideDMaxCount > 65,535, so the table takes u32 entries with full values (the
+    // conditions above already say so; stated here so that no threshold change can pair WIDE with u16 entries)
+    if (pl.cls == kWide) pl.wide_table = pl.full_table = true;
     pl.gf_m = 0; pl.gf_sh = 0;
     if (pl.cls == kNarrow)    { const Magic32 g = make_magic32((uint32_t)fmax, f + c); pl.gf_m = g.m; pl.gf_sh = g.sh; }
     else if (pl.cls == kWide) { const Magic64 g = make_magic64(fmax, f + c); pl.gf_m = g.m; pl.gf_sh = g.sh; }

@@ -1,6 +1,8 @@
 // redux_lane_codec.cuh -- throughput mapping: ONE STREAM PER LANE, 32 independent streams per warp.
 //
-// What the reference does per stream on one CPU thread (src/codec.rs:55-176 over
+// The pieces every lane kernel shares (jobs, arithmetic class traits, table layout, bit and byte I/O) and the lane
+// kernels of the HUGE class (code_bits > 32: 64-bit coder state).  The tuned lane kernels for code_bits <= 32 are in
+// redux_lane_al.cuh.  What the reference does per stream on one CPU thread (src/codec.rs:55-176 over
 // src/model/adaptive_tree.rs) runs here in every lane of every warp:
 //   * the stream's Fenwick table lives in shared memory, LANE-INTERLEAVED so that lane l only ever
 //     touches bank l: whatever nodes the 32 data-dependent walks visit, an access is one wavefront.
@@ -12,14 +14,13 @@
 //     adaptive_tree.rs:86-89) equals the number of updates so far and node 257 (EOF) is constant 1:
 //     neither is stored.  256 x u16 per stream = 512 B -> 14 warps (448 streams) per SM, which is
 //     what lets 65,536 blocks be resident on 148 SMs in ONE wave (443 streams per SM);
-//   * walks are flattened: the nodes of a prefix path are s & (0xFF << b) for the set bits b of s and
-//     the nodes of an update path are (s | (2^k - 1)) + 1 for the clear bits k-1 of s, so every load
-//     address is independent of every other load (no pointer chasing) and absent nodes read the
-//     always-zero node 0 instead of branching;
+//   * the encoder loads one node per tree level for the range query and the update together
+//     (LaneTable2::query, redux_lane_al.cuh); the decoder descends four ways per round on 32-bit residuals
+//     of the quotient value = X / range and increments the nodes where it turns left (LaneDecoder::run);
 //   * count_t = min(257 + t, FMAX) depends on the position only (SURVEY.md A.5), so the two divisions
-//     by count (src/codec.rs:59-60) are multiplications by a per-position magic shared by all streams,
-//     and the loop splits into an adaptive phase (t < FMAX-257) and a frozen phase (no updates,
-//     constant reciprocal);
+//     by count (src/codec.rs:59-60) are multiplications by a per-position 65-bit magic shared by all
+//     streams, and the loop splits into an adaptive phase (t < FMAX-257) and a frozen phase (no updates,
+//     constant reciprocal; the encoder rewrites its table as the cumulative array);
 //   * renormalisation (src/codec.rs:62-89 / :140-158) is the closed form of redux_common.cuh;
 //   * bits are packed into a 64-bit register and leave as whole big-endian 32-bit words
 //     (MSB-first bytes, src/bitio/mod.rs:148-198) into the stream's private output slot; raw bytes
@@ -155,79 +156,8 @@ struct LaneTable {
         for (int i = 0; i < kWords; ++i) w[i * 32] = 0;
     }
 
-    // (cum(s), cum(s+1)) for a data symbol s in 0..255: the paired walk of adaptive_tree.rs:63-80
-    // flattened.  Bits of s below its lowest zero bit belong to cum(s) only, bits above to both,
-    // node s+1 to cum(s+1) only.  `updates` = increments of the unstored node 256.
-    __device__ __forceinline__ void query(uint32_t s, uint32_t updates, uint32_t &cl, uint32_t &ch) const {
-        const uint32_t S = s << 5;
-        const uint32_t lowmask = s & ~(s + 1);                  // trailing ones of s
-        const uint32_t odd = s & 1u;
-        // b = 0: node s itself when s is odd (an odd node); belongs to cum(s) only
-        uint32_t total = t[odd ? (int)S + kOddAdj : 0];
-        uint32_t both = 0;
-#pragma unroll
-        for (int b = 1; b < 8; ++b) {
-            const uint32_t bit = 1u << b;
-            const uint32_t v = t[(s & bit) ? (S & (0x1FE0u << b)) : 0u];   // even node s & (0xFF<<b)
-            total += v;
-            both += (lowmask & bit) ? 0u : v;
-        }
-        // node s+1: odd when s is even; node 256 is not stored
-        const uint32_t it = (s == 255u) ? 0u : (odd ? S + 32u : (uint32_t)((int)S + 32 + kOddAdj));
-        const uint32_t top = t[it] + ((s == 255u) ? updates : 0u);
-        cl = s + total;
-        ch = s + 1u + top + both;
-    }
-
-    // update(s+1) of adaptive_tree.rs:83-92 minus the two unstored nodes: node s+1, then for every
-    // clear bit k-1 of s the node (s | (2^k-1)) + 1, while below 256.  The surviving levels are exactly
-    // the set bits of ~s below its highest one (the highest clear bit of s leads to node 256).
-    __device__ __forceinline__ void update(uint32_t s) {
-        const uint32_t S = s << 5;
-        const uint32_t q = ~s & 255u;
-        const uint32_t levels = q ? (q ^ (1u << (31 - clz32(q)))) : 0u;
-        if (q) {                                                        // s != 255
-            const uint32_t i0 = (s & 1u) ? S + 32u : (uint32_t)((int)S + 32 + kOddAdj);
-            t[i0] = (TW)(t[i0] + 1);
-        }
-#pragma unroll
-        for (int k = 1; k < 8; ++k) {
-            if (levels & (1u << (k - 1))) {
-                const uint32_t i = (S | (((1u << k) - 1u) << 5)) + 32u;   // ((s | mask_k) + 1) * 32, an even node
-                t[i] = (TW)(t[i] + 1);
-            }
-        }
-    }
-
     // index (in TW units from t) of node n, either parity
     static __device__ __forceinline__ int node_index(uint32_t n) { return (int)(n << 5) + ((n & 1u) ? kOddAdj : 0); }
-
-    // Once the model is frozen (adaptive_tree.rs:84) the tree is read-only: rewrite it in place as the
-    // plain cumulative array C[i] = cum(i) - i (the layout of AdaptiveLinearModel, adaptive_linear.rs:26-28),
-    // so that a lookup is two loads.  Descending i only reads nodes <= i, which are still Fenwick nodes.
-    __device__ __forceinline__ void freeze_to_cumulative() {
-        for (uint32_t i = 255; i >= 1; --i) {
-            uint32_t sum = 0;
-            for (uint32_t x = i; x; x &= x - 1) sum += t[node_index(x)];
-            t[node_index(i)] = (TW)sum;
-        }
-    }
-    // (cum(s), cum(s+1)) from the cumulative array; total = count
-    __device__ __forceinline__ void query_frozen(uint32_t s, uint32_t count, uint32_t &cl, uint32_t &ch) const {
-        if (sizeof(TW) == 2) {
-            // node pairs (2m, 2m+1) share word m: one or two aligned 32-bit loads
-            const uint32_t *w = reinterpret_cast<const uint32_t *>(t);
-            const uint32_t w0 = w[(s >> 1) << 5], w1 = w[(((s + 1) >> 1) & 127u) << 5];
-            const bool odd = s & 1u;
-            cl = s + (odd ? (w0 >> 16) : (w0 & 0xFFFFu));
-            const uint32_t hi = odd ? (w1 & 0xFFFFu) : (w0 >> 16);
-            ch = (s == 255u) ? count - 1 : s + 1 + hi;
-        } else {
-            cl = s + t[s << 5];
-            const uint32_t hi = t[((s + 1) & 255u) << 5];
-            ch = (s == 255u) ? count - 1 : s + 1 + hi;
-        }
-    }
 };
 
 // ------------------------------------------------------------------ bit packer (encoder output)
@@ -348,6 +278,8 @@ __device__ __forceinline__ uint32_t encode_step(typename Cls<CLS>::S &low, typen
 template <typename TW, bool FULL> struct LaneTable2;       // redux_lane_al.cuh: one-walk query + update
 
 // ------------------------------------------------------------------ encoder
+// The library launches these kernels (encoder and decoder) with CLS = kHuge only; code_bits <= 32 runs the tuned
+// kernels of redux_lane_al.cuh.  The bodies use nothing but the class traits, so CLS stays a parameter.
 template <typename TW, int CLS>
 __global__ void __launch_bounds__(kLaneThreads, 2)
 encode_lane_kernel(const LaneEncJob job)
@@ -529,84 +461,38 @@ struct LaneDecoder {
             const S rm1 = high - low;
             const P X = C::mulr(count, (S)(value - low)) - 1;
             // step m = 256: node 256 = count-1 (adaptive_tree.rs:119-127 with the unstored node)
-            P plo = 0, phi = C::mulr(count - 1, rm1);
+            const bool is_eof = X >= C::mulr(count - 1, rm1);
+            // Quotient first, as the 64-bit-product class of redux_lane_al.cuh: the reference's
+            // value = X / range (src/codec.rs:131) from a double estimate made exact by one remainder check
+            // (div_by_range64), then the 4-ary descent on plain 32-bit values in the residual domain --
+            // R = v - lo, N = v - hi < 0, each round's three sign bits move the position, unsigned min / max
+            // pick the new bounds -- with the model update on the left turns.  Four dependent table round trips
+            // of 32-bit adds instead of eight of 64-bit multiply-adds and 64-bit comparisons.  A step that ends
+            // the stream afterwards (EOF symbol, bits ran out, sink full) leaves a table nobody reads again.
+            const uint32_t v = div_by_range64((uint64_t)X, (uint64_t)rm1 + 1u);
+            uint32_t R = v, N = v - (count - 1u);                 // node 256 = count - 1
             uint32_t I = 0;                                       // i * 32
-            const bool is_eof = X >= phi;
-            if (CLS == kNarrow) {
-                // Two tree levels per round (adaptive_tree.rs:119-127 unrolled by two): the three candidate
-                // nodes i+m, i+m/2 and i+m+m/2 are loaded together, so the descent is 4 dependent
-                // shared-memory round trips instead of 8 (measured 41.5 -> 37.6 ms; with 64-bit products
-                // the extra speculative multiply costs more than the shorter chain saves).
 #pragma unroll
-                for (int m = 128; m >= 2; m >>= 2) {
-                    const int h = m >> 1;
-                    const int oddadj = (h == 1) ? LaneTable<TW>::kOddAdj : 0;      // nodes i+1, i+3 are odd
-                    const uint32_t a = (uint32_t)m + tab.t[I + (uint32_t)(m << 5)];
-                    const uint32_t b = (uint32_t)h + tab.t[(int)I + (h << 5) + oddadj];
-                    const uint32_t cc = (uint32_t)h + tab.t[(int)I + ((m + h) << 5) + oddadj];
-                    const P pa = C::mul_add(a, rm1, plo);
-                    const P pb = C::mul_add(b, rm1, plo);
-                    const P pc = C::mul_add(cc, rm1, pa);
-                    const bool ra = X >= pa, rb = X >= pb, rc = X >= pc;
-                    const bool r2 = ra ? rc : rb;                                   // second-level decision
-                    const P p2 = ra ? pc : pb;                                      // second-level boundary
-                    const P base = ra ? pa : plo;
-                    phi = r2 ? (ra ? phi : pa) : p2;
-                    plo = r2 ? p2 : base;
-                    I += (ra ? (uint32_t)(m << 5) : 0u) + (r2 ? (uint32_t)(h << 5) : 0u);
+            for (int m = 128; m >= 2; m >>= 2) {
+                const int h = m >> 1;
+                const int oddadj = (h == 1) ? LaneTable<TW>::kOddAdj : 0;      // nodes i+1, i+3 are odd
+                const uint32_t ia = I + (uint32_t)(m << 5), ib = (uint32_t)((int)I + (h << 5) + oddadj),
+                               ic = (uint32_t)((int)I + ((m + h) << 5) + oddadj);
+                const uint32_t ar = tab.t[ia], br = tab.t[ib], cr = tab.t[ic];
+                const uint32_t da = R - ((uint32_t)m + ar), db = R - ((uint32_t)h + br), dc = da - ((uint32_t)h + cr);
+                const uint32_t ma = (uint32_t)((int32_t)da >> 31), mb = (uint32_t)((int32_t)db >> 31), mc = (uint32_t)((int32_t)dc >> 31);
+                if (ADAPT) {                                      // + 1 where the descent turns left (node c: only after a right turn)
+                    tab.t[ia] = (TW)(ar - ma);
+                    tab.t[ib] = (TW)(br - mb);
+                    tab.t[ic] = (TW)(cr - mc + ma);
                 }
-            } else if (CLS == kHuge) {
-                // Quotient first, as the 64-bit-product class of redux_lane_al.cuh: the reference's
-                // value = X / range (src/codec.rs:131) from a double estimate made exact by one remainder check
-                // (div_by_range64), then the 4-ary descent on plain 32-bit values in the residual domain --
-                // R = v - lo, N = v - hi < 0, each round's three sign bits move the position, unsigned min / max
-                // pick the new bounds -- with the model update on the left turns.  Four dependent table round trips
-                // of 32-bit adds instead of eight of 64-bit multiply-adds and 64-bit comparisons.
-                const uint32_t v = div_by_range64((uint64_t)X, (uint64_t)rm1 + 1u);
-                uint32_t R = v, N = v - (count - 1u);             // node 256 = count - 1
-#pragma unroll
-                for (int m = 128; m >= 2; m >>= 2) {
-                    const int h = m >> 1;
-                    const int oddadj = (h == 1) ? LaneTable<TW>::kOddAdj : 0;
-                    const uint32_t ia = I + (uint32_t)(m << 5), ib = (uint32_t)((int)I + (h << 5) + oddadj),
-                                   ic = (uint32_t)((int)I + ((m + h) << 5) + oddadj);
-                    const uint32_t ar = tab.t[ia], br = tab.t[ib], cr = tab.t[ic];
-                    const uint32_t da = R - ((uint32_t)m + ar), db = R - ((uint32_t)h + br), dc = da - ((uint32_t)h + cr);
-                    const uint32_t ma = (uint32_t)((int32_t)da >> 31), mb = (uint32_t)((int32_t)db >> 31), mc = (uint32_t)((int32_t)dc >> 31);
-                    if (ADAPT) {                                  // + 1 where the descent turns left (node c: only after a right turn)
-                        tab.t[ia] = (TW)(ar - ma);
-                        tab.t[ib] = (TW)(br - mb);
-                        tab.t[ic] = (TW)(cr - mc + ma);
-                    }
-                    const uint32_t r1 = da < dc ? da : dc, r2 = R < db ? R : db;
-                    const uint32_t n1 = da > dc ? da : dc, n2 = N > db ? N : db;
-                    R = r1 < r2 ? r1 : r2;
-                    N = n1 > n2 ? n1 : n2;
-                    I += (3u + ma + mb + mc) * (uint32_t)(h << 5);
-                }
-                plo = C::mulr(v - R, rm1);
-                phi = C::mulr(v - N, rm1);
-            } else {
-#pragma unroll
-                // The model update rides on the descent (as in redux_lane_al.cuh): the nodes update(s+1) increments
-                // (adaptive_tree.rs:83-92) are exactly the nodes at which the descent to s turns left, and their
-                // values have just been loaded.  A step that ends the stream afterwards (EOF symbol, bits ran out,
-                // sink full) leaves a table nobody reads again.
-                for (int m = 128; m >= 2; m >>= 1) {              // even nodes i + m
-                    const uint32_t raw = tab.t[I + (uint32_t)(m << 5)];
-                    const P p = C::mul_add((uint32_t)m + raw, rm1, plo);
-                    const bool right = X >= p;
-                    if (ADAPT && !right) tab.t[I + (uint32_t)(m << 5)] = (TW)(raw + 1u);
-                    if (right) { I += (uint32_t)(m << 5); plo = p; } else { phi = p; }
-                }
-                {                                                 // m = 1: odd node i + 1
-                    const uint32_t raw = tab.t[(int)I + 32 + LaneTable<TW>::kOddAdj];
-                    const P p = C::mul_add(1u + raw, rm1, plo);
-                    const bool right = X >= p;
-                    if (ADAPT && !right) tab.t[(int)I + 32 + LaneTable<TW>::kOddAdj] = (TW)(raw + 1u);
-                    if (right) { I += 32u; plo = p; } else { phi = p; }
-                }
+                const uint32_t r1 = da < dc ? da : dc, r2 = R < db ? R : db;
+                const uint32_t n1 = da > dc ? da : dc, n2 = N > db ? N : db;
+                R = r1 < r2 ? r1 : r2;
+                N = n1 > n2 ? n1 : n2;
+                I += (3u + ma + mb + mc) * (uint32_t)(h << 5);
             }
+            const P plo = C::mulr(v - R, rm1), phi = C::mulr(v - N, rm1);
             if (is_eof) {                                         // src/codec.rs:136-138: no renorm, no reads
                 st = -1;
                 return;
@@ -615,7 +501,6 @@ struct LaneDecoder {
             // src/codec.rs:133-134
             high = low + (S)C::divc(phi, g, count) - 1;
             low = low + (S)C::divc(plo, g, count);
-            if (ADAPT && CLS == kNarrow) tab.update(sym);         // (the narrow rounds above keep the separate walk)
             // src/codec.rs:140-158 in closed form
             const Renorm<S> r = renorm<S>(low, high, c);
             const uint32_t n = r.n1 + r.k;

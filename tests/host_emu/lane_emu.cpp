@@ -69,17 +69,6 @@ void run_grid(K kernel, const J &job, uint64_t n_blocks)
 
 }  // namespace
 
-namespace {
-// the plan without the double-reciprocal class (forced 32-bit tables, the generic kernels)
-void plain_wide(LanePlan &pl)
-{
-    if (pl.cls != kWideD) return;
-    pl.cls = kWide;
-    const Magic64 g = make_magic64(((uint64_t)1 << pl.f) - 1, pl.f + pl.c);
-    pl.gf_m = g.m; pl.gf_sh = g.sh;
-}
-}  // namespace
-
 extern "C" uint64_t emu_slot_stride(uint32_t f, uint32_t c, uint64_t max_block_len)
 {
     return lane_plan(f, c, max_block_len).slot_stride;
@@ -92,8 +81,7 @@ extern "C" void emu_lane_plan(uint32_t f, uint32_t c, uint64_t max_block_len, ui
     out[0] = (uint32_t)pl.cls; out[1] = pl.wide_table; out[2] = pl.full_table; out[3] = pl.aligned; out[4] = pl.tcap;
 }
 
-// force_wide_table: -1 = as the front end would choose, 0 = u16 entries, 1 = u32 entries; +2 = force the
-// generic kernels (redux_lane_codec.cuh) where the tuned ones (redux_lane_al.cuh) would be chosen
+// force_wide_table: -1 = as the front end would choose, 0 = u16 entries, 1 = u32 entries
 namespace {
 // start state of a trained byte model for the tuned lane kernels: tree[0..257], total, EOF frequency
 struct LaneStart { std::vector<uint32_t> tree; uint32_t count0 = kNsym, eof_freq = 1; bool on = false; };
@@ -124,10 +112,7 @@ extern "C" int emu_encode_lane_ex(uint32_t f, uint32_t c, uint64_t max_block_len
 {
     const LaneStart st0 = lane_start(freq);
     LanePlan pl = lane_plan(f, c, max_block_len, st0.count0, st0.on);
-    const bool legacy = force_wide_table >= 2;            // 2/3: the generic kernels of redux_lane_codec.cuh
-    if (force_wide_table >= 2) force_wide_table -= 2;
     if (force_wide_table >= 0) { pl.wide_table = force_wide_table != 0; if (pl.wide_table) pl.full_table = true; }
-    if (legacy) plain_wide(pl);
     std::vector<uint8_t> magic = build_magic(pl);
     LaneEncJob job;
     job.in = in; job.in_off = in_off; job.n_blocks = n_blocks;
@@ -136,22 +121,17 @@ extern "C" int emu_encode_lane_ex(uint32_t f, uint32_t c, uint64_t max_block_len
     job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
     job.init_tree = st0.on ? st0.tree.data() : nullptr; job.count0 = st0.count0; job.eof_freq = st0.eof_freq;
     job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
-#define RUN(TW) \
-    (pl.cls == kNarrow ? run_grid(encode_lane_kernel<TW, kNarrow>, job, n_blocks) : \
-     pl.cls == kWide   ? run_grid(encode_lane_kernel<TW, kWide>, job, n_blocks)   : \
-                         run_grid(encode_lane_kernel<TW, kHuge>, job, n_blocks))
 #define RUN_AL(TW, FULL) \
     (pl.cls == kWideD && pl.c == 32 ? run_grid(encode_lane_al_kernel<TW, kWideD, FULL, true>, job, n_blocks) : \
      pl.cls == kWideD  ? run_grid(encode_lane_al_kernel<TW, kWideD, FULL, false>, job, n_blocks) : \
      pl.cls == kNarrow ? run_grid(encode_lane_al_kernel<TW, kNarrow, FULL, false>, job, n_blocks) : \
      pl.c == 32        ? run_grid(encode_lane_al_kernel<TW, kWide, FULL, true>, job, n_blocks) : \
                          run_grid(encode_lane_al_kernel<TW, kWide, FULL, false>, job, n_blocks))
-    if (pl.aligned && !legacy) {
-        if (pl.wide_table) RUN_AL(uint32_t, true);
-        else if (pl.full_table) RUN_AL(uint16_t, true);
-        else RUN_AL(uint16_t, false);
-    } else if (pl.wide_table) RUN(uint32_t); else RUN(uint16_t);
-#undef RUN
+    if (!pl.aligned && pl.wide_table) run_grid(encode_lane_kernel<uint32_t, kHuge>, job, n_blocks);
+    else if (!pl.aligned) run_grid(encode_lane_kernel<uint16_t, kHuge>, job, n_blocks);
+    else if (pl.wide_table) RUN_AL(uint32_t, true);
+    else if (pl.full_table) RUN_AL(uint16_t, true);
+    else RUN_AL(uint16_t, false);
 #undef RUN_AL
     return 0;
 }
@@ -170,10 +150,7 @@ extern "C" int emu_decode_lane_ex(uint32_t f, uint32_t c, uint64_t max_block_len
 {
     const LaneStart st0 = lane_start(freq);
     LanePlan pl = lane_plan(f, c, max_block_len, st0.count0, st0.on);
-    const bool legacy = force_wide_table >= 2;            // 2/3: the generic kernels of redux_lane_codec.cuh
-    if (force_wide_table >= 2) force_wide_table -= 2;
     if (force_wide_table >= 0) { pl.wide_table = force_wide_table != 0; if (pl.wide_table) pl.full_table = true; }
-    if (legacy) plain_wide(pl);
     std::vector<uint8_t> magic = build_magic(pl);
     LaneDecJob job;
     job.comp = comp; job.comp_off = comp_off; job.n_blocks = n_blocks;
@@ -182,10 +159,6 @@ extern "C" int emu_decode_lane_ex(uint32_t f, uint32_t c, uint64_t max_block_len
     job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
     job.init_tree = st0.on ? st0.tree.data() : nullptr; job.count0 = st0.count0; job.eof_freq = st0.eof_freq;
     job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
-#define RUN(TW) \
-    (pl.cls == kNarrow ? run_grid(decode_lane_kernel<TW, kNarrow>, job, n_blocks) : \
-     pl.cls == kWide   ? run_grid(decode_lane_kernel<TW, kWide>, job, n_blocks)   : \
-                         run_grid(decode_lane_kernel<TW, kHuge>, job, n_blocks))
 #define RUN_AL(TW, FULL) \
     (pl.cls == kWideD && pl.c == 32 ? run_grid(decode_lane_al_kernel<TW, kWideD, FULL, true, false>, job, n_blocks) : \
      pl.cls == kWideD  ? run_grid(decode_lane_al_kernel<TW, kWideD, FULL, false, false>, job, n_blocks) : \
@@ -193,12 +166,11 @@ extern "C" int emu_decode_lane_ex(uint32_t f, uint32_t c, uint64_t max_block_len
      pl.cls == kNarrow ? run_grid(decode_lane_al_kernel<TW, kNarrow, FULL, false, false>, job, n_blocks) : \
      pl.c == 32        ? run_grid(decode_lane_al_kernel<TW, kWide, FULL, true, false>, job, n_blocks) : \
                          run_grid(decode_lane_al_kernel<TW, kWide, FULL, false, false>, job, n_blocks))
-    if (pl.aligned && !legacy) {
-        if (pl.wide_table) RUN_AL(uint32_t, true);
-        else if (pl.full_table) RUN_AL(uint16_t, true);
-        else RUN_AL(uint16_t, false);
-    } else if (pl.wide_table) RUN(uint32_t); else RUN(uint16_t);
-#undef RUN
+    if (!pl.aligned && pl.wide_table) run_grid(decode_lane_kernel<uint32_t, kHuge>, job, n_blocks);
+    else if (!pl.aligned) run_grid(decode_lane_kernel<uint16_t, kHuge>, job, n_blocks);
+    else if (pl.wide_table) RUN_AL(uint32_t, true);
+    else if (pl.full_table) RUN_AL(uint16_t, true);
+    else RUN_AL(uint16_t, false);
 #undef RUN_AL
     return 0;
 }

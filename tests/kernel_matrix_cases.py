@@ -1,10 +1,11 @@
 """The kernel matrix: one row per (parameters, model, schedule, block shapes) that selects a given coder kernel.
 
-The device path chooses among ~45 kernel instantiations (redux_b200/csrc/redux_capi.cu, launch_*): by arithmetic class,
-table entry width, FULL (u16 entries hold full tree values), code_bits == 32, code_bits <= 16 (staged decoder window),
-lane / warp / split mapping, generic kernels, and whether the model was trained.  Encode plans from the longest block,
-decode from the largest output slot.  Every row names the encode and decode kernel it must reach (checked on the GPU by
-redux_debug_launched_kernels) and is chosen to reach the phase that matters: adaptive, frozen, or both in one block.
+The device path chooses among 37 coder kernels (redux_b200/csrc/redux_capi.cu: pick_encoder / pick_decoder, the split
+and generic launches) by arithmetic class, table entry width, FULL (u16 entries hold full tree values), code_bits ==
+32, code_bits <= 16 (staged decoder window), lane / warp / split mapping, generic kernels, and whether the model was
+trained.  Encode plans from the longest block, decode from the largest output slot.  Every row names the encode and
+decode kernel it must reach (checked on the GPU by redux_debug_launched_kernels) and is chosen to reach the phase that
+matters: adaptive, frozen, or both in one block.  Together the rows reach every kernel of the library.
 
 Imported by test_gpu_kernel_matrix.py (GPU, every row), test_kernel_coverage.py (no GPU: completeness, the plan
 behind each lane row, and the lane rows in the host emulation) -- plain data and helpers, no test in here.
@@ -111,11 +112,6 @@ CASES = [
     C("generic_trained_c34", (8, 30, 34), "encode_generic<global>", "decode_generic<global>", train=3000,
       big=[(5000, "mix")]),
 ]
-
-# Configured and compiled, never launched: kWide survives lane_plan only when count0 + updates >= 349,525, which is
-# more than 65,535 and so always takes u32 entries (test_kernel_coverage.py proves it over the whole plan space).
-UNREACHABLE = [e for tw_full in (("u16", True), ("u16", False)) for c32 in (False, True)
-               for e in lane(tw_full[0], "Wide", tw_full[1], c32)]
 
 
 def expected_kernels():

@@ -29,7 +29,7 @@ def lane_plan(emu, f, c, max_len, count0=km.NSYM, pretrained=False):
 
 
 def lane_kernels(emu, case, max_len):
-    """(encode, decode) kernel names the lane launch switches of redux_capi.cu pick for lane_plan's result."""
+    """(encode, decode) kernel names pick_encoder / pick_decoder of redux_capi.cu choose for lane_plan's result."""
     _, f, c = case.params
     p = lane_plan(emu, f, c, max_len, int(km.trained_freq(case).sum()), case.train > 0)
     tw = "u32" if p["wide_table"] else "u16"
@@ -44,23 +44,23 @@ def is_lane_row(case):
     return case.enc.startswith("encode_lane")
 
 
-def test_every_kernel_has_a_row():
-    """The rows' kernels plus the unreachable ones are exactly the kernels the library can launch: a kernel added
-    without a row, or a row deleted that was the only one reaching its kernel, fails here."""
+def test_rows_reach_exactly_the_library_kernels():
+    """The rows' kernels are exactly the kernels the library can launch: a kernel added without a row, or a row
+    deleted that was the only one reaching its kernel, fails here."""
     names = rb.kernel_names()
-    assert len(names) == len(set(names)) >= 45
-    expected, unreachable = km.expected_kernels(), set(km.UNREACHABLE)
-    assert len(unreachable) == 8 and not expected & unreachable
-    assert expected | unreachable == set(names), ("no row for %s" % sorted(set(names) - expected - unreachable),
-                                                  "not a kernel: %s" % sorted(expected - set(names)))
+    assert len(names) == len(set(names)) == 37
+    expected = km.expected_kernels()
+    assert expected == set(names), ("no row for %s" % sorted(set(names) - expected),
+                                    "not a kernel: %s" % sorted(expected - set(names)))
     assert len({c.name for c in km.CASES}) == len(km.CASES)
 
 
-def test_u16_wide_kernels_are_unreachable(emu):
+def test_wide_class_plans_take_u32_entries(emu):
     """lane_plan keeps the plain WIDE class (64-bit magics) only when count0 + updates >= 349,525 > 65,535, which
-    always takes u32 entries: the eight u16 WIDE kernels are never launched.  Swept over every byte-symbol (f, c)
-    with c <= 32, block lengths at every threshold +-1 and fresh / trained start totals around 65,535 and 349,525.
-    NARROW plans are always u16 entries with full values (its launch switch has no other kernel)."""
+    always takes u32 entries: the library has no u16 WIDE lane kernel, and lane_plan states the rule outright so
+    that no threshold change can ask for one.  Swept over every byte-symbol (f, c) with c <= 32, block lengths at
+    every threshold +-1 and fresh / trained start totals around 65,535 and 349,525.  NARROW plans are always u16
+    entries with full values (the library has no other NARROW lane kernel)."""
     wide = 0
     for f in range(10, 31):
         fmax = (1 << f) - 1
