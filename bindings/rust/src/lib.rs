@@ -65,6 +65,15 @@ extern "C" {
                                  model_freq: *const u32, comp: *const u8, comp_offsets: *const u64, n_blocks: u64,
                                  raw: *mut u8, raw_offsets: *const u64, raw_lens: *mut u64,
                                  consumed: *mut u64, status: *mut i32) -> c_int;
+    pub fn redux_encode_batch_models(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t,
+                                     model_freqs: *const u32, n_models: u32, block_model: *const u32,
+                                     input: *const u8, in_offsets: *const u64, n_blocks: u64,
+                                     out: *mut u8, out_cap: u64, out_offsets: *mut u64, status: *mut i32) -> c_int;
+    pub fn redux_decode_batch_models(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t,
+                                     model_freqs: *const u32, n_models: u32, block_model: *const u32,
+                                     comp: *const u8, comp_offsets: *const u64, n_blocks: u64,
+                                     raw: *mut u8, raw_offsets: *const u64, raw_lens: *mut u64,
+                                     consumed: *mut u64, status: *mut i32) -> c_int;
     pub fn redux_encode_batch_device(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, model_kind: c_int,
                                      p: *const redux_params_t, d_in: *const u8, d_in_offsets: *const u64,
                                      n_blocks: u64, max_block_len: u64, d_out: *mut u8, out_cap: u64,
@@ -73,6 +82,16 @@ extern "C" {
                                      p: *const redux_params_t, d_comp: *const u8, d_comp_offsets: *const u64,
                                      n_blocks: u64, max_block_len: u64, d_raw: *mut u8, d_raw_offsets: *const u64,
                                      d_raw_lens: *mut u64, d_consumed: *mut u64, d_status: *mut i32) -> c_int;
+    pub fn redux_encode_batch_device_models(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, model_kind: c_int,
+                                            p: *const redux_params_t, model_freqs: *const u32, n_models: u32,
+                                            d_block_model: *const u32, d_in: *const u8, d_in_offsets: *const u64,
+                                            n_blocks: u64, max_block_len: u64, d_out: *mut u8, out_cap: u64,
+                                            d_out_offsets: *mut u64, d_status: *mut i32) -> c_int;
+    pub fn redux_decode_batch_device_models(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, model_kind: c_int,
+                                            p: *const redux_params_t, model_freqs: *const u32, n_models: u32,
+                                            d_block_model: *const u32, d_comp: *const u8, d_comp_offsets: *const u64,
+                                            n_blocks: u64, max_block_len: u64, d_raw: *mut u8, d_raw_offsets: *const u64,
+                                            d_raw_lens: *mut u64, d_consumed: *mut u64, d_status: *mut i32) -> c_int;
     pub fn redux_ctx_synchronize(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void) -> c_int;
 }
 

@@ -179,6 +179,27 @@ int redux_decode_batch_ex(redux_ctx_t *ctx, int model_kind, const redux_params_t
                           uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
                           uint64_t *consumed, int32_t *status);
 
+/* ---- a start model per block.  A batch of compress() calls that each get their own Box<Model>, trained or fresh,
+ * is one call: model_freqs holds n_models frequency vectors of symbol_count entries back to back (host memory; each row
+ * validated like model_freq above, an invalid row gives REDUX_INVALID_INPUT and redux_ctx_last_error names it; a fresh
+ * model is a row of ones), and block i starts from row block_model[i].  block_model == NULL is allowed only when
+ * n_models == 1 (every block uses row 0); n_models == 0 is REDUX_INVALID_INPUT.  A block whose row index is >= n_models
+ * gets status REDUX_INVALID_INPUT and an empty stream / empty output; the other blocks are unaffected.  The start trees
+ * take n_models x (symbol_count + 1) x 4 bytes of device memory; a table larger than REDUX_MAX_MODEL_TABLE_BYTES
+ * returns REDUX_UNSUPPORTED.  One model kind and one set of parameters per call.  Blocks of one launch that start from
+ * different totals freeze at different positions, which can cost time (DESIGN.md 3.8).  The _ex calls are the
+ * n_models == 1 case.  Otherwise identical to redux_encode_batch / redux_decode_batch. */
+#define REDUX_MAX_MODEL_TABLE_BYTES ((uint64_t)256 << 20)
+int redux_encode_batch_models(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                              const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                              const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                              uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status);
+int redux_decode_batch_models(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                              const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                              const uint8_t *comp, const uint64_t *comp_offsets, uint64_t n_blocks,
+                              uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
+                              uint64_t *consumed, int32_t *status);
+
 /* ---- batch, device-resident buffers (kernel-only timing; all pointers are device memory on
  * `device`, which must be one of the context's devices; work is enqueued on `stream` (a
  * cudaStream_t; NULL = the CUDA default stream) and is asynchronous to the host).
@@ -216,6 +237,22 @@ int redux_decode_batch_device_ex(redux_ctx_t *ctx, int device, void *stream, int
                                  uint64_t max_block_len,
                                  uint8_t *d_raw, const uint64_t *d_raw_offsets, uint64_t *d_raw_lens,
                                  uint64_t *d_consumed, int32_t *d_status);
+/* The same with a start model per block (see redux_encode_batch_models): model_freqs is a HOST pointer, copied during
+ * the call; d_block_model is a DEVICE pointer [n_blocks] (NULL only when n_models == 1), read by the kernels. */
+int redux_encode_batch_device_models(redux_ctx_t *ctx, int device, void *stream, int model_kind,
+                                     const redux_params_t *params, const uint32_t *model_freqs, uint32_t n_models,
+                                     const uint32_t *d_block_model,
+                                     const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_blocks,
+                                     uint64_t max_block_len,
+                                     uint8_t *d_out, uint64_t out_capacity, uint64_t *d_out_offsets,
+                                     int32_t *d_status);
+int redux_decode_batch_device_models(redux_ctx_t *ctx, int device, void *stream, int model_kind,
+                                     const redux_params_t *params, const uint32_t *model_freqs, uint32_t n_models,
+                                     const uint32_t *d_block_model,
+                                     const uint8_t *d_comp, const uint64_t *d_comp_offsets, uint64_t n_blocks,
+                                     uint64_t max_block_len,
+                                     uint8_t *d_raw, const uint64_t *d_raw_offsets, uint64_t *d_raw_lens,
+                                     uint64_t *d_consumed, int32_t *d_status);
 /* Waits for the work enqueued on `stream` of `device`. */
 int redux_ctx_synchronize(redux_ctx_t *ctx, int device, void *stream);
 

@@ -152,6 +152,10 @@ def lib():
     L.redux_host_unregister.argtypes = [vp]
     L.redux_encode_batch_device_ex.argtypes = [vp, i32, vp, i32, pp, vp, vp, vp, u64, u64, vp, u64, vp, vp]
     L.redux_decode_batch_device_ex.argtypes = [vp, i32, vp, i32, pp, vp, vp, vp, u64, u64, vp, vp, vp, vp, vp]
+    L.redux_encode_batch_models.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, u64, vp, vp]
+    L.redux_decode_batch_models.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, vp, vp, vp, vp]
+    L.redux_encode_batch_device_models.argtypes = [vp, i32, vp, i32, pp, vp, u32, vp, vp, vp, u64, u64, vp, u64, vp, vp]
+    L.redux_decode_batch_device_models.argtypes = [vp, i32, vp, i32, pp, vp, u32, vp, vp, vp, u64, u64, vp, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -310,6 +314,30 @@ class AdaptiveLinearModel(Model):
 class AdaptiveTreeModel(Model):
     """AdaptiveTreeModel::new (src/model/adaptive_tree.rs:36-48)."""
     kind = MODEL_TREE
+
+
+def _model_table(models):
+    """(kind, C parameters, uint32[n_models, symbol_count] frequency table) of a sequence of models: one model kind and
+    one Parameters for all of them (InvalidInput otherwise); a fresh model is a row of ones."""
+    models = list(models)
+    if not models:
+        raise InvalidInput("no models")
+    kind, p = models[0].kind, models[0].params
+    key = (p.symbol_bits, p.freq_bits, p.code_bits)
+    for m in models:
+        if m.kind != kind:
+            raise InvalidInput("models of different kinds in one call")
+        if (m.params.symbol_bits, m.params.freq_bits, m.params.code_bits) != key:
+            raise InvalidInput("models with different Parameters in one call")
+    table = np.ones((len(models), p.symbol_count), dtype=np.uint32)
+    for i, m in enumerate(models):
+        if m.freq is not None:
+            table[i] = m.freq
+    return kind, p._c(), table
+
+
+def _block_model(block_model):
+    return None if block_model is None else np.ascontiguousarray(block_model, dtype=np.uint32)
 
 
 def _ptr(x):
@@ -479,6 +507,51 @@ class Context:
             _raise(rc, self)
         return raw, raw_lens[:n], consumed[:n], status[:n]
 
+    def encode_batch_models(self, data, offsets, models, block_model, out=None, check=True):
+        """encode_batch with a start model per block: block i starts from models[block_model[i]] (block_model None:
+        only with one model).  models: AdaptiveLinearModel / AdaptiveTreeModel of one kind and one Parameters, fresh or
+        trained.  A block whose index is out of range gets status InvalidInput and an empty stream.  Returns
+        (out uint8 array view, out_offsets, status)."""
+        kind, pc, table = _model_table(models)
+        bm = _block_model(block_model)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        if out is None:
+            lens = offsets[1:] - offsets[:-1]
+            nsym = lens * np.uint64(8) // np.uint64(pc.symbol_bits) + np.uint64(1)
+            cap = int((nsym * np.uint64(pc.code_bits) + np.uint64(7)).sum() // 8) + 8 * n
+            out = np.empty(max(cap, 1), dtype=np.uint8)
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        rc = lib().redux_encode_batch_models(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(bm),
+                                             _ptr(data), _ptr(offsets), n, _ptr(out), out.size, _ptr(out_off),
+                                             _ptr(status))
+        if check:
+            _raise(rc, self)
+        return out[:int(out_off[n])], out_off, status[:n]
+
+    def decode_batch_models(self, comp, comp_offsets, raw_offsets, models, block_model, raw=None, check=True):
+        """decode_batch with a start model per block (see encode_batch_models).  Returns (raw uint8 array, raw_lens,
+        consumed, status)."""
+        kind, pc, table = _model_table(models)
+        bm = _block_model(block_model)
+        comp = np.ascontiguousarray(comp, dtype=np.uint8)
+        comp_offsets = np.ascontiguousarray(comp_offsets, dtype=np.uint64)
+        raw_offsets = np.ascontiguousarray(raw_offsets, dtype=np.uint64)
+        n = comp_offsets.size - 1
+        if raw is None:
+            raw = np.zeros(max(int(raw_offsets[-1]), 1), dtype=np.uint8)
+        raw_lens = np.zeros(max(n, 1), dtype=np.uint64)
+        consumed = np.zeros(max(n, 1), dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        rc = lib().redux_decode_batch_models(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(bm),
+                                             _ptr(comp), _ptr(comp_offsets), n, _ptr(raw), _ptr(raw_offsets),
+                                             _ptr(raw_lens), _ptr(consumed), _ptr(status))
+        if check:
+            _raise(rc, self)
+        return raw, raw_lens[:n], consumed[:n], status[:n]
+
     # ---- batch, device-resident (tensors or raw device addresses); asynchronous on `stream`
     def encode_batch_device(self, d_in, d_in_offsets, n_blocks, max_block_len, d_out, out_capacity,
                             d_out_offsets, d_status, model, device=0, stream=None):
@@ -494,6 +567,25 @@ class Context:
                                                   _ptr(d_comp), _ptr(d_comp_offsets), n_blocks, max_block_len,
                                                   _ptr(d_raw), _ptr(d_raw_offsets), _ptr(d_raw_lens), _ptr(d_consumed),
                                                   _ptr(d_status)), self)
+
+    def encode_batch_device_models(self, d_in, d_in_offsets, n_blocks, max_block_len, d_out, out_capacity,
+                                   d_out_offsets, d_status, models, d_block_model, device=0, stream=None):
+        """encode_batch_device with a start model per block: d_block_model is a device uint32 tensor (or address) of
+        n_blocks row indices, None only with one model."""
+        kind, pc, table = _model_table(models)
+        _raise(lib().redux_encode_batch_device_models(self._h, device, stream, kind, C.byref(pc), _ptr(table),
+                                                      table.shape[0], _ptr(d_block_model), _ptr(d_in), _ptr(d_in_offsets),
+                                                      n_blocks, max_block_len, _ptr(d_out), out_capacity,
+                                                      _ptr(d_out_offsets), _ptr(d_status)), self)
+
+    def decode_batch_device_models(self, d_comp, d_comp_offsets, n_blocks, max_block_len, d_raw, d_raw_offsets,
+                                   d_raw_lens, d_consumed, d_status, models, d_block_model, device=0, stream=None):
+        kind, pc, table = _model_table(models)
+        _raise(lib().redux_decode_batch_device_models(self._h, device, stream, kind, C.byref(pc), _ptr(table),
+                                                      table.shape[0], _ptr(d_block_model), _ptr(d_comp),
+                                                      _ptr(d_comp_offsets), n_blocks, max_block_len, _ptr(d_raw),
+                                                      _ptr(d_raw_offsets), _ptr(d_raw_lens), _ptr(d_consumed),
+                                                      _ptr(d_status)), self)
 
     def set_text_corpus(self, corpus):
         """bytes / uint8 array (or None): the corpus the synthetic generator cuts its text-class blocks from."""

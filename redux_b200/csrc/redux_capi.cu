@@ -234,9 +234,11 @@ struct DeviceState {
     cudaStream_t h2d = nullptr;           // host-to-device stream: input copies never queue behind kernels
     HostBuf pin_off, pin_status, pin_aux0, pin_aux1;
     DevBuf slots, sizes, flag;                 // encoder workspace
-    DevBuf st_in, st_off, st_out, st_ooff, st_status, st_aux0, st_aux1, st_roff;   // host-API staging
+    DevBuf st_in, st_off, st_bmod, st_out, st_ooff, st_status, st_aux0, st_aux1, st_roff;   // host-API staging
     DevBuf split_hist, split_pairs;            // split encoder: chunk histograms, per-position ranges
-    DevBuf gen_tabs, gen_init, gen_freq, gen_magic;   // generic path: Fenwick columns, start tree, uploaded frequencies, reciprocals
+    // start models (trained models and the generic path): Fenwick columns of the generic kernels, start trees,
+    // uploaded frequencies, {total, EOF frequency} per model, reciprocals of the generic kernels
+    DevBuf gen_tabs, gen_init, gen_freq, gen_start, gen_magic;
     uint8_t *text_lut = nullptr;
     DevBuf corpus; uint64_t corpus_len = 0;    // text-class corpus of the synthetic generator (redux_ctx_set_text_corpus)
     std::vector<MagicEntry> magics;
@@ -255,13 +257,18 @@ struct DeviceState {
 
 struct TimedSpan { cudaEvent_t a, b; int kind; int device; };
 
+// The start models of the running *_models call (redux_encode_batch_models): on = false for a fresh model.
+// freqs: n rows of symbol_count frequencies (host memory); block_model: the row of each block, NULL = row 0 for every
+// block (host memory in the host-buffer calls, device memory in the device-resident ones).
+struct ModelArgs { bool on = false; const uint32_t *freqs = nullptr; uint32_t n = 0; const uint32_t *block_model = nullptr; };
+
 struct redux_ctx {
     std::vector<DeviceState> devs;
     int sched = REDUX_SCHED_AUTO;
     std::string last_error;
     uint64_t launches = 0;
     bool timing = false;                  // bracket every kernel with CUDA events (bench.py)
-    const uint32_t *model_freq = nullptr;  // pre-trained start state of the running *_ex call (host pointer)
+    ModelArgs models;                     // start models of the running call
     std::vector<TimedSpan> spans;
     StagingConfig staging;
     CopyPool *pool = nullptr;              // created by the first call that meets pageable memory
@@ -324,11 +331,15 @@ struct Plan {
     int lane_cls = kNarrow;                     // class of the tuned lane kernels (kWideD where the plan allows it)
     uint64_t gf_m_wide = 0; uint32_t gf_sh_wide = 0;   // frozen reciprocal of the plain WIDE class (warp / split paths)
     // generic path (redux_generic_codec.cuh): symbol_bits != 8 or a pre-trained model
-    bool generic = false; uint32_t s = 8, gen_threads = 0, gen_total = 0;
-    // byte symbols, code_bits <= 32, model trained before the call: the tuned lane kernels start from its tree
-    bool pretrained = false; uint32_t count0 = kNsym, eof_freq = 1;
-    uint32_t *gen_tabs = nullptr; const uint32_t *gen_init = nullptr;
-    const Magic64 *gen_magic = nullptr; uint32_t gen_magic_len = 0;
+    bool generic = false; uint32_t s = 8, gen_threads = 0;
+    // byte symbols, code_bits <= 32, models trained before the call: the tuned lane kernels start each block from its
+    // model's tree
+    bool pretrained = false;
+    std::vector<uint2> starts;              // {total, EOF frequency} of every start model (a fresh one: symbol_count, 1)
+    BlockModels models{};                   // the start models on the device (prepare_models); none for a fresh model
+    const uint32_t *gen_init = nullptr;      // the start trees (prepare_models)
+    uint32_t *gen_tabs = nullptr;
+    const Magic64 *gen_magic = nullptr; uint32_t gen_magic_len = 0, gen_magic_base = 0;
     bool warp = false;      // one stream per warp (latency mapping) instead of one per lane
     bool split = false;     // encode only: parallel model phase + one-warp coder chain (redux_split_encoder.cuh)
     uint64_t max_len = 0;   // longest block of the launch
@@ -362,6 +373,33 @@ bool choose_split(const redux_ctx *ctx, uint64_t n_blocks, int cls, uint64_t max
     return n_blocks * stride * sizeof(uint2) <= kSplitMaxPairBytes;
 }
 
+// {total, EOF frequency} of every row of the running call's model table, after checking the table: every entry >= 1
+// and the sum <= freq_max (the observable state of a trained reference model: every symbol at least once, a total
+// that starts at symbol_count and stops growing at freq_max, adaptive_tree.rs:84).
+int model_starts(redux_ctx *ctx, const redux_params_t *p, std::vector<uint2> *starts)
+{
+    const ModelArgs &ma = ctx->models;
+    if (ma.n == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_models is 0");
+    if (!ma.freqs) return fail(ctx, REDUX_INVALID_INPUT, "model_freqs is NULL");
+    if (!ma.block_model && ma.n > 1) return fail(ctx, REDUX_INVALID_INPUT, "block_model is NULL but n_models > 1");
+    const uint64_t nsym = ((uint64_t)1 << p->symbol_bits) + 1, fmax = ((uint64_t)1 << p->freq_bits) - 1;
+    if ((uint64_t)ma.n * (nsym + 1) * sizeof(uint32_t) > REDUX_MAX_MODEL_TABLE_BYTES)
+        return fail(ctx, REDUX_UNSUPPORTED, "n_models x (symbol_count + 1) start-tree entries exceed REDUX_MAX_MODEL_TABLE_BYTES");
+    starts->resize(ma.n);
+    char msg[96];
+    for (uint32_t m = 0; m < ma.n; ++m) {
+        const uint32_t *fr = ma.freqs + (size_t)m * nsym;
+        uint64_t total = 0;
+        for (uint64_t i = 0; i < nsym; ++i) {
+            if (fr[i] < 1) { snprintf(msg, sizeof msg, "model row %u: frequency below 1", m); return fail(ctx, REDUX_INVALID_INPUT, msg); }
+            total += fr[i];
+        }
+        if (total > fmax) { snprintf(msg, sizeof msg, "model row %u: total exceeds freq_max", m); return fail(ctx, REDUX_INVALID_INPUT, msg); }
+        (*starts)[m] = make_uint2((uint32_t)total, fr[nsym - 1]);
+    }
+    return REDUX_OK;
+}
+
 int make_plan(redux_ctx *ctx, const redux_params_t *p, uint64_t max_block_len, Plan *pl)
 {
     if (!p) return fail(ctx, REDUX_INVALID_INPUT, "params is NULL");
@@ -374,20 +412,12 @@ int make_plan(redux_ctx *ctx, const redux_params_t *p, uint64_t max_block_len, P
     pl->s = p->symbol_bits;
     pl->max_len = max_block_len;
     const bool huge = arith_class(p->freq_bits, p->code_bits) == kHuge;
-    pl->generic = p->symbol_bits != (uint32_t)kSymbolBits || (ctx->model_freq != nullptr && huge);
-    uint64_t total0 = ((uint64_t)1 << p->symbol_bits) + 1;
-    if (ctx->model_freq) {
-        // the observable state of a trained reference model: every symbol at least once, total <= freq_max
-        // (it starts at symbol_count and stops growing at freq_max, adaptive_tree.rs:84)
-        const uint64_t nsym = total0, fmax = ((uint64_t)1 << p->freq_bits) - 1;
-        total0 = 0;
-        for (uint64_t i = 0; i < nsym; ++i) {
-            if (ctx->model_freq[i] < 1) return fail(ctx, REDUX_INVALID_INPUT, "model frequency below 1");
-            total0 += ctx->model_freq[i];
-        }
-        if (total0 > fmax) return fail(ctx, REDUX_INVALID_INPUT, "model total exceeds freq_max");
+    pl->generic = p->symbol_bits != (uint32_t)kSymbolBits || (ctx->models.on && huge);
+    pl->starts.assign(1, make_uint2((1u << p->symbol_bits) + 1, 1u));
+    if (ctx->models.on) {
+        int rc = model_starts(ctx, p, &pl->starts);
+        if (rc) return rc;
     }
-    pl->gen_total = (uint32_t)total0;
     if (pl->generic) {
         // worst case: every coded symbol (floor(8 len / s) data symbols + EOF) emits code_bits bits
         pl->f = p->freq_bits; pl->c = p->code_bits; pl->cls = kHuge; pl->tcap = 0; pl->wide_table = true;
@@ -396,10 +426,16 @@ int make_plan(redux_ctx *ctx, const redux_params_t *p, uint64_t max_block_len, P
         pl->slot_stride = ((bound + 15) & ~(uint64_t)15) + 16;
         return REDUX_OK;
     }
-    // (trained) tuned lane kernels: count_t = min(count0 + t, FMAX), full tree values in the table
-    pl->pretrained = ctx->model_freq != nullptr;
-    pl->count0 = (uint32_t)total0; pl->eof_freq = ctx->model_freq ? ctx->model_freq[kEof] : 1u;
-    const LanePlan lp = lane_plan(p->freq_bits, p->code_bits, max_block_len, pl->count0, pl->pretrained);
+    // (trained) tuned lane kernels: count_t = min(count0 + t, FMAX), full tree values in the table.  Blocks may start
+    // from different models; the launch is planned for the largest start total.  Every choice lane_plan makes from
+    // count0 holds for every smaller one: the totals a block reaches, min(count0 + len, FMAX), grow with count0, so u32
+    // entries, a total below the WIDE_D bound and the reciprocal table's length (entry t <-> 257 + t; a lane reads
+    // it from count0 - 257 on) that serve the largest also serve the others.  The frozen total is FMAX for all of them.
+    // tests/test_block_models_emu.py checks this over lane_plan.
+    pl->pretrained = ctx->models.on;
+    uint32_t count0 = 0;
+    for (const uint2 &st : pl->starts) count0 = std::max(count0, st.x);
+    const LanePlan lp = lane_plan(p->freq_bits, p->code_bits, max_block_len, count0, pl->pretrained);
     pl->lane_cls = lp.cls;
     pl->f = lp.f; pl->c = lp.c; pl->cls = lp.cls == kWideD ? (int)kWide : lp.cls; pl->tcap = lp.tcap; pl->wide_table = lp.wide_table;
     pl->magic_len = lp.magic_len; pl->slot_stride = lp.slot_stride;
@@ -441,38 +477,54 @@ int get_magic(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const Plan &p
     return REDUX_OK;
 }
 
-// Generic path set-up: uploads the start frequencies (if any), builds the start tree on the device and
-// sizes the per-thread Fenwick columns.  At most ~2 GB of columns; a thread codes several blocks in turn.
-int prepare_generic(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const redux_params_t *p, uint64_t n_blocks, Plan *pl)
+// Start models on the device (trained models, generic path): uploads the frequency table and the {total, EOF frequency}
+// of every model, builds all start trees in one launch (a fresh model: one tree, gen_init) and, for the generic path,
+// sizes the per-thread Fenwick columns (at most ~2 GB; a thread codes several blocks in turn) and builds the
+// reciprocals.  pl->models.block_model stays NULL: the launches set it.
+int prepare_models(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const redux_params_t *p, uint64_t n_blocks, Plan *pl)
 {
     if (!pl->generic && !pl->pretrained) return REDUX_OK;
     const uint32_t nsym = (1u << p->symbol_bits) + 1;
+    const uint32_t n_models = (uint32_t)pl->starts.size();
     const uint32_t *d_freq = nullptr;
-    if (ctx->model_freq) {                                   // validated by make_plan
-        CU_TRY(ctx, d->gen_freq.reserve(nsym * sizeof(uint32_t)));
-        CU_TRY(ctx, cudaMemcpyAsync(d->gen_freq.p, ctx->model_freq, nsym * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    if (ctx->models.on) {                                    // validated by make_plan
+        const size_t bytes = (size_t)n_models * nsym * sizeof(uint32_t);
+        CU_TRY(ctx, d->gen_freq.reserve(bytes));
+        CU_TRY(ctx, cudaMemcpyAsync(d->gen_freq.p, ctx->models.freqs, bytes, cudaMemcpyHostToDevice, stream));
         d_freq = (const uint32_t *)d->gen_freq.p;
     }
-    CU_TRY(ctx, d->gen_init.reserve((nsym + 1) * sizeof(uint32_t)));
-    build_tree_kernel<<<(nsym + 1 + 255) / 256, 256, 0, stream>>>(d_freq, nsym, (uint32_t *)d->gen_init.p);
+    const uint64_t nodes = (uint64_t)n_models * (nsym + 1);
+    CU_TRY(ctx, d->gen_init.reserve(nodes * sizeof(uint32_t)));
+    build_tree_kernel<<<(uint32_t)((nodes + 255) / 256), 256, 0, stream>>>(d_freq, nsym, (uint32_t *)d->gen_init.p, n_models);
     ctx->launches++;
     CU_TRY(ctx, cudaGetLastError());
     pl->gen_init = (const uint32_t *)d->gen_init.p;
-    if (!pl->generic) {                                      // tuned lane kernels: only the start tree is needed
+    if (ctx->models.on) {
+        CU_TRY(ctx, d->gen_start.reserve(n_models * sizeof(uint2)));
+        CU_TRY(ctx, cudaMemcpyAsync(d->gen_start.p, pl->starts.data(), n_models * sizeof(uint2), cudaMemcpyHostToDevice, stream));
+        pl->models.trees = pl->gen_init;
+        pl->models.start = (const uint2 *)d->gen_start.p;
+        pl->models.n_models = n_models;
+    }
+    if (!pl->generic) {                                      // tuned lane kernels: only the start trees are needed
+        // the trees must be complete before kernels on other streams read them; the upload buffers are reused
         CU_TRY(ctx, cudaStreamSynchronize(stream));
         return REDUX_OK;
     }
-    // reciprocals of every total a block of this call can reach: init_total .. min(freq_max, init_total + symbols)
+    // reciprocals of every total a block of this call can reach: smallest start total .. min(freq_max, largest start
+    // total + symbols)
     {
+        uint32_t lo = pl->starts[0].x, hi = lo;
+        for (const uint2 &st : pl->starts) { lo = std::min(lo, st.x); hi = std::max(hi, st.x); }
         const uint64_t fmax = ((uint64_t)1 << p->freq_bits) - 1;
         const uint64_t syms = pl->max_len * 8 / p->symbol_bits + 1;                     // data symbols + EOF
-        const uint64_t top = std::min<uint64_t>(fmax, (uint64_t)pl->gen_total + syms);
-        const uint32_t len = (uint32_t)(top - pl->gen_total + 2);
+        const uint64_t top = std::min<uint64_t>(fmax, (uint64_t)hi + syms);
+        const uint32_t len = (uint32_t)(top - lo + 2);
         CU_TRY(ctx, d->gen_magic.reserve((size_t)len * sizeof(Magic64)));
-        build_magic_kernel<Magic64><<<(len + 255) / 256, 256, 0, stream>>>((Magic64 *)d->gen_magic.p, len, 0u, pl->gen_total);
+        build_magic_kernel<Magic64><<<(len + 255) / 256, 256, 0, stream>>>((Magic64 *)d->gen_magic.p, len, 0u, lo);
         ctx->launches++;
         CU_TRY(ctx, cudaGetLastError());
-        pl->gen_magic = (const Magic64 *)d->gen_magic.p; pl->gen_magic_len = len;
+        pl->gen_magic = (const Magic64 *)d->gen_magic.p; pl->gen_magic_len = len; pl->gen_magic_base = lo;
     }
     const uint64_t col_bytes = (uint64_t)(nsym + 1) * sizeof(uint32_t);
     uint64_t threads = std::min<uint64_t>((n_blocks + kGenericThreads - 1) / kGenericThreads * kGenericThreads,
@@ -480,37 +532,36 @@ int prepare_generic(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const r
     const uint64_t budget = (uint64_t)2 << 30;
     if (threads * col_bytes > budget) threads = std::max<uint64_t>(budget / col_bytes / kGenericThreads, 1) * kGenericThreads;
     CU_TRY(ctx, d->gen_tabs.reserve(threads * col_bytes));
-    // the start tree must be complete before kernels on other streams read it; the upload buffer is reused
+    // the start trees must be complete before kernels on other streams read them; the upload buffers are reused
     CU_TRY(ctx, cudaStreamSynchronize(stream));
     pl->gen_threads = (uint32_t)threads;
     pl->gen_tabs = (uint32_t *)d->gen_tabs.p;
     return REDUX_OK;
 }
 
-// Reciprocal table as the kernels index it: entry t <-> count0 + t (the table itself starts at count 257).
-const void *lane_magic(const Plan &pl, const void *magic)
-{
-    if (!magic || !pl.pretrained) return magic;
-    const size_t esz = magic_entry_size(magic_class(pl));
-    return (const uint8_t *)magic + (size_t)(pl.count0 - kNsym) * esz;
-}
-
-GenericJob generic_job(const Plan &pl)
+// block_model: the row of each block of the launch (NULL: row 0)
+GenericJob generic_job(const Plan &pl, const uint32_t *block_model)
 {
     GenericJob g{};
-    g.tabs = pl.gen_tabs; g.init_tree = pl.gen_init; g.init_total = pl.gen_total;
+    g.tabs = pl.gen_tabs; g.init_tree = pl.gen_init; g.init_total = pl.gen_magic_base;
+    g.models = pl.models; g.models.block_model = pl.models.start ? block_model : nullptr;
     g.s = pl.s; g.f = pl.f; g.c = pl.c; g.n_threads = pl.gen_threads;
     g.magic = pl.gen_magic; g.magic_len = pl.gen_magic_len;
     return g;
 }
 
-// The fields LaneEncJob and LaneDecJob take from the plan.
+// The fields LaneEncJob and LaneDecJob take from the plan.  The job's own start model is the fresh one (257 / 1, the
+// reciprocal table from count 257 on); trained models come as the table of pl.models, whose rows the kernels offset
+// from it (StreamStart).
 template <typename J>
-void set_plan_fields(J &job, const Plan &pl, const void *magic)
+void set_plan_fields(J &job, const Plan &pl, const void *magic, const uint32_t *block_model)
 {
-    job.magic = lane_magic(pl, magic); job.f = pl.f; job.c = pl.c; job.tcap = pl.tcap;
+    job.magic = magic; job.f = pl.f; job.c = pl.c;
+    job.tcap = pl.pretrained ? (uint32_t)(((uint64_t)1 << pl.f) - 1 - kNsym) : pl.tcap;
     job.one = pl.c <= 32 ? 1u << (32 - pl.c) : 0u;
-    job.init_tree = pl.pretrained ? pl.gen_init : nullptr; job.count0 = pl.count0; job.eof_freq = pl.eof_freq;
+    job.init_tree = nullptr; job.count0 = kNsym; job.eof_freq = 1;
+    job.models = pl.models;
+    job.models.block_model = pl.models.start ? block_model : nullptr;
     job.gf_m = pl.gf_m; job.gf_sh = pl.gf_sh;
 }
 
@@ -860,8 +911,9 @@ extern "C" void redux_ctx_destroy(redux_ctx_t *ctx)
         if (d.h2d) cudaStreamDestroy(d.h2d);
         for (int i = 0; i < kPipeStreams; ++i) if (d.pipe[i]) cudaStreamDestroy(d.pipe[i]);
         for (HostBuf *b : {&d.pin_off, &d.pin_status, &d.pin_aux0, &d.pin_aux1}) b->release();
-        for (DevBuf *b : {&d.slots, &d.sizes, &d.flag, &d.st_in, &d.st_off, &d.st_out, &d.st_ooff,
-                          &d.st_status, &d.st_aux0, &d.st_aux1, &d.st_roff, &d.corpus, &d.gen_magic, &d.gen_tabs, &d.gen_init, &d.gen_freq, &d.split_hist, &d.split_pairs}) b->release();
+        for (DevBuf *b : {&d.slots, &d.sizes, &d.flag, &d.st_in, &d.st_off, &d.st_bmod, &d.st_out, &d.st_ooff,
+                          &d.st_status, &d.st_aux0, &d.st_aux1, &d.st_roff, &d.corpus, &d.gen_magic, &d.gen_tabs, &d.gen_init,
+                          &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs}) b->release();
         for (auto &m : d.magics) cudaFree(m.ptr);
         if (d.text_lut) cudaFree(d.text_lut);
         for (StageRing *r : {d.ring_up, d.ring_down}) if (r) { r->release(); delete r; }
@@ -952,7 +1004,7 @@ namespace {
 // Enqueues encode + size scan + compaction for n_blocks blocks on stream s.  Workspace slices are given
 // explicitly so that several chunks of one batch can be in flight on different streams.
 int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, const void *magic,
-                  const uint8_t *d_in, const uint64_t *d_in_off, uint64_t n_blocks,
+                  const uint8_t *d_in, const uint64_t *d_in_off, const uint32_t *d_block_model, uint64_t n_blocks,
                   uint8_t *d_out, uint64_t out_capacity, uint64_t *d_out_off, int32_t *d_status,
                   uint8_t *slots, uint32_t *sizes, int32_t *flag)
 {
@@ -960,12 +1012,12 @@ int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     job.in = d_in; job.in_off = d_in_off; job.n_blocks = n_blocks;
     job.slots = slots; job.slot_stride = pl.slot_stride;
     job.sizes = sizes; job.status = d_status;
-    set_plan_fields(job, pl, magic);
+    set_plan_fields(job, pl, magic, d_block_model);
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_ENCODE);
         KernelId kid;
         if (pl.generic) {
-            GenericJob g = generic_job(pl);
+            GenericJob g = generic_job(pl, d_block_model);
             g.in = d_in; g.in_off = d_in_off; g.n_blocks = n_blocks;
             g.slots = slots; g.slot_stride = pl.slot_stride; g.sizes = sizes; g.status = d_status;
             encode_generic_kernel<<<pl.gen_threads / kGenericThreads, kGenericThreads, generic_smem_bytes(pl.s), s>>>(g);
@@ -1002,7 +1054,7 @@ int encode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
 }
 
 int decode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, const void *magic,
-                  const uint8_t *d_comp, const uint64_t *d_comp_off, uint64_t n_blocks,
+                  const uint8_t *d_comp, const uint64_t *d_comp_off, const uint32_t *d_block_model, uint64_t n_blocks,
                   uint8_t *d_raw, const uint64_t *d_raw_off, uint64_t *d_raw_lens, uint64_t *d_consumed,
                   int32_t *d_status)
 {
@@ -1010,12 +1062,12 @@ int decode_launch(redux_ctx *ctx, int device, cudaStream_t s, const Plan &pl, co
     job.comp = d_comp; job.comp_off = d_comp_off; job.n_blocks = n_blocks;
     job.raw = d_raw; job.raw_off = d_raw_off; job.raw_len = d_raw_lens; job.consumed = d_consumed;
     job.status = d_status;
-    set_plan_fields(job, pl, magic);
+    set_plan_fields(job, pl, magic, d_block_model);
     {
         KernelTimer kt(ctx, device, s, REDUX_KERNEL_DECODE);
         KernelId kid;
         if (pl.generic) {
-            GenericJob g = generic_job(pl);
+            GenericJob g = generic_job(pl, d_block_model);
             g.in = d_comp; g.in_off = d_comp_off; g.n_blocks = n_blocks;
             g.raw = d_raw; g.raw_off = d_raw_off; g.raw_len = d_raw_lens; g.consumed = d_consumed; g.status = d_status;
             decode_generic_kernel<<<pl.gen_threads / kGenericThreads, kGenericThreads, generic_smem_bytes(pl.s), s>>>(g);
@@ -1059,11 +1111,11 @@ extern "C" int redux_encode_batch_device(redux_ctx_t *ctx, int device, void *str
     CU_TRY(ctx, ws_acquire(d, s));              // the previous device call may still be using the workspace
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, s, pl, &magic))) return rc;
-    if ((rc = prepare_generic(ctx, d, s, params, n_blocks, &pl))) return rc;
+    if ((rc = prepare_models(ctx, d, s, params, n_blocks, &pl))) return rc;
     CU_TRY(ctx, d->slots.reserve(n_blocks * pl.slot_stride));
     CU_TRY(ctx, d->sizes.reserve(n_blocks * sizeof(uint32_t)));
     CU_TRY(ctx, d->flag.reserve(sizeof(int32_t)));
-    rc = encode_launch(ctx, device, s, pl, magic, d_in, d_in_offsets, n_blocks, d_out, out_capacity,
+    rc = encode_launch(ctx, device, s, pl, magic, d_in, d_in_offsets, ctx->models.block_model, n_blocks, d_out, out_capacity,
                        d_out_offsets, d_status, (uint8_t *)d->slots.p, (uint32_t *)d->sizes.p,
                        (int32_t *)d->flag.p);
     CU_TRY(ctx, ws_release(d, s));
@@ -1093,8 +1145,8 @@ extern "C" int redux_decode_batch_device(redux_ctx_t *ctx, int device, void *str
     CU_TRY(ctx, ws_acquire(d, s));
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, s, pl, &magic))) return rc;
-    if ((rc = prepare_generic(ctx, d, s, params, n_blocks, &pl))) return rc;
-    rc = decode_launch(ctx, device, s, pl, magic, d_comp, d_comp_offsets, n_blocks, d_raw, d_raw_offsets,
+    if ((rc = prepare_models(ctx, d, s, params, n_blocks, &pl))) return rc;
+    rc = decode_launch(ctx, device, s, pl, magic, d_comp, d_comp_offsets, ctx->models.block_model, n_blocks, d_raw, d_raw_offsets,
                        d_raw_lens, d_consumed, d_status);
     CU_TRY(ctx, ws_release(d, s));
     return rc;
@@ -1222,7 +1274,7 @@ void for_each_device(redux_ctx *ctx, size_t nd, std::vector<int> &rcs, F fn)
     std::vector<uint64_t> launches(nd, 0);
     std::vector<std::vector<TimedSpan>> spans(nd);
     for (size_t g = 0; g < nd; ++g) th.emplace_back([&, g] {
-        redux_ctx view; view.sched = ctx->sched; view.timing = ctx->timing; view.model_freq = ctx->model_freq;
+        redux_ctx view; view.sched = ctx->sched; view.timing = ctx->timing; view.models = ctx->models;
         view.staging = ctx->staging; view.pool = ctx->pool;
         view.devs.push_back(ctx->devs[g]);
         rcs[g] = fn(&view, &view.devs[0], g);
@@ -1237,6 +1289,20 @@ void for_each_device(redux_ctx *ctx, size_t nd, std::vector<int> &rcs, F fn)
         ctx->spans.insert(ctx->spans.end(), spans[g].begin(), spans[g].end());
         if (rcs[g]) ctx->last_error = errs[g];
     }
+}
+
+// The shard's slice of the call's block-to-model index (host memory) goes to the device on the h2d stream, beside the
+// offsets, so every chunk's kernel (which waits for its input on that stream) finds it; *d_bmod stays NULL when the
+// call has no index.
+int upload_block_models(redux_ctx *ctx, DeviceState *d, Shard sh, const uint32_t **d_bmod)
+{
+    *d_bmod = nullptr;
+    if (!ctx->models.on || !ctx->models.block_model) return REDUX_OK;
+    CU_TRY(ctx, d->st_bmod.reserve(sh.count * sizeof(uint32_t)));
+    CU_TRY(ctx, cudaMemcpyAsync(d->st_bmod.p, ctx->models.block_model + sh.first, sh.count * sizeof(uint32_t),
+                                cudaMemcpyHostToDevice, d->h2d));
+    *d_bmod = (const uint32_t *)d->st_bmod.p;
+    return REDUX_OK;
 }
 
 // Waits for everything this device still has in flight (used on error paths before buffers are reused).
@@ -1444,7 +1510,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     CU_TRY(ctx, d->pin_status.reserve(sh.count * sizeof(int32_t)));
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, d->h2d, pl, &magic))) return rc;
-    if ((rc = prepare_generic(ctx, d, d->h2d, p, sh.count, &pl))) return rc;
+    if ((rc = prepare_models(ctx, d, d->h2d, p, sh.count, &pl))) return rc;
     EventSet evs;                       // [0, nc): chunk done; [nc, 2nc): chunk input on the device
     CU_TRY(ctx, evs.create(2 * nc));
     // pageable caller memory goes through the pinned rings (CopyPool); then the enqueue loop below runs on a feeder
@@ -1454,6 +1520,8 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     if (stage_in) CU_TRY(ctx, ensure_ring(ctx, &d->ring_up));
     if (stage_out) CU_TRY(ctx, ensure_ring(ctx, &d->ring_down));
     CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, rel.data(), rel.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, d->h2d));
+    const uint32_t *d_bmod = nullptr;
+    if ((rc = upload_block_models(ctx, d, sh, &d_bmod))) return rc;
 
     uint8_t *d_in = (uint8_t *)d->st_in.p, *d_out = (uint8_t *)d->st_out.p;
     uint64_t *d_off = (uint64_t *)d->st_off.p, *d_ooff = (uint64_t *)d->st_ooff.p;
@@ -1475,7 +1543,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
             if (e == cudaSuccess) e = cudaEventRecord(evs.ev[nc + k], d->h2d);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(s, evs.ev[nc + k], 0);
             if (e == cudaSuccess)
-                rc2 = encode_launch(ctx, d->device, s, pl, magic, d_in, d_off + c.first, c.count,
+                rc2 = encode_launch(ctx, d->device, s, pl, magic, d_in, d_off + c.first, d_bmod ? d_bmod + c.first : nullptr, c.count,
                                     d_out + res->chunk_base[k], chunk_cap[k], d_ooff + c.first + k,
                                     d_status + c.first, (uint8_t *)d->slots.p + c.first * pl.slot_stride,
                                     (uint32_t *)d->sizes.p + c.first, (int32_t *)d->flag.p + k);
@@ -1645,7 +1713,7 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     CU_TRY(ctx, d->pin_status.reserve(sh.count * sizeof(int32_t)));
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, d->pipe[0], pl, &magic))) return rc;
-    if ((rc = prepare_generic(ctx, d, d->pipe[0], p, sh.count, &pl))) return rc;
+    if ((rc = prepare_models(ctx, d, d->pipe[0], p, sh.count, &pl))) return rc;
     EventSet evs;                       // [0, nc): chunk input on the device; [nc, 2nc): chunk decoded
     CU_TRY(ctx, evs.create(2 * nc));
     // pageable caller memory: see encode_shard
@@ -1654,6 +1722,8 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     if (stage_in) CU_TRY(ctx, ensure_ring(ctx, &d->ring_up));
     if (stage_out) CU_TRY(ctx, ensure_ring(ctx, &d->ring_down));
     CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, rel.data(), rel.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, d->h2d));
+    const uint32_t *d_bmod = nullptr;
+    if ((rc = upload_block_models(ctx, d, sh, &d_bmod))) return rc;
     uint8_t *d_comp = (uint8_t *)d->st_in.p, *d_raw = (uint8_t *)d->st_out.p;
     uint64_t *d_coff = (uint64_t *)d->st_off.p, *d_roff = d_coff + sh.count + 1;
     uint64_t *d_len = (uint64_t *)d->st_aux0.p, *d_cons = (uint64_t *)d->st_aux1.p;
@@ -1675,7 +1745,7 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
             if (e == cudaSuccess) e = cudaEventRecord(evs.ev[k], d->h2d);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(s, evs.ev[k], 0);
             if (e == cudaSuccess)
-                rc2 = decode_launch(ctx, d->device, s, pl, magic, d_comp, d_coff + c.first, c.count, d_raw,
+                rc2 = decode_launch(ctx, d->device, s, pl, magic, d_comp, d_coff + c.first, d_bmod ? d_bmod + c.first : nullptr, c.count, d_raw,
                                     d_roff + c.first, d_len + c.first, d_cons + c.first, d_status + c.first);
             // the whole slot range of the chunk goes back; bytes beyond raw_lens[i] inside a slot are unspecified
             // (into pageable memory: by the drainer below, through the ring)
@@ -1793,18 +1863,76 @@ extern "C" int redux_decompress(redux_ctx_t *ctx, int model_kind, const redux_pa
 }
 
 // ================================================================== pre-trained models (8(f) rank 4)
+// A call with start models runs the plain call with ctx->models set: make_plan validates them, prepare_models puts them
+// on the device, the launches hand each block its row.  The _ex forms are the one-model case.
+
+namespace {
+struct ModelScope {
+    redux_ctx *ctx;
+    ModelScope(redux_ctx *c, const uint32_t *freqs, uint32_t n, const uint32_t *block_model) : ctx(c) {
+        ctx->models.on = true; ctx->models.freqs = freqs; ctx->models.n = n; ctx->models.block_model = block_model;
+    }
+    ~ModelScope() { ctx->models = ModelArgs{}; }
+};
+}  // namespace
+
+extern "C" int redux_encode_batch_models(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                         const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                         const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                         uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status)
+{
+    if (!ctx) return REDUX_INVALID_INPUT;
+    ModelScope ms(ctx, model_freqs, n_models, block_model);
+    return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
+}
+
+extern "C" int redux_decode_batch_models(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                         const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                         const uint8_t *comp, const uint64_t *comp_offsets, uint64_t n_blocks,
+                                         uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
+                                         uint64_t *consumed, int32_t *status)
+{
+    if (!ctx) return REDUX_INVALID_INPUT;
+    ModelScope ms(ctx, model_freqs, n_models, block_model);
+    return redux_decode_batch(ctx, model_kind, params, comp, comp_offsets, n_blocks, raw, raw_offsets, raw_lens,
+                              consumed, status);
+}
+
+extern "C" int redux_encode_batch_device_models(redux_ctx_t *ctx, int device, void *stream, int model_kind,
+                                                const redux_params_t *params, const uint32_t *model_freqs,
+                                                uint32_t n_models, const uint32_t *d_block_model,
+                                                const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_blocks,
+                                                uint64_t max_block_len, uint8_t *d_out, uint64_t out_capacity,
+                                                uint64_t *d_out_offsets, int32_t *d_status)
+{
+    if (!ctx) return REDUX_INVALID_INPUT;
+    ModelScope ms(ctx, model_freqs, n_models, d_block_model);
+    return redux_encode_batch_device(ctx, device, stream, model_kind, params, d_in, d_in_offsets, n_blocks,
+                                     max_block_len, d_out, out_capacity, d_out_offsets, d_status);
+}
+
+extern "C" int redux_decode_batch_device_models(redux_ctx_t *ctx, int device, void *stream, int model_kind,
+                                                const redux_params_t *params, const uint32_t *model_freqs,
+                                                uint32_t n_models, const uint32_t *d_block_model,
+                                                const uint8_t *d_comp, const uint64_t *d_comp_offsets, uint64_t n_blocks,
+                                                uint64_t max_block_len, uint8_t *d_raw, const uint64_t *d_raw_offsets,
+                                                uint64_t *d_raw_lens, uint64_t *d_consumed, int32_t *d_status)
+{
+    if (!ctx) return REDUX_INVALID_INPUT;
+    ModelScope ms(ctx, model_freqs, n_models, d_block_model);
+    return redux_decode_batch_device(ctx, device, stream, model_kind, params, d_comp, d_comp_offsets, n_blocks,
+                                     max_block_len, d_raw, d_raw_offsets, d_raw_lens, d_consumed, d_status);
+}
 
 extern "C" int redux_encode_batch_ex(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
                                      const uint32_t *model_freq, const uint8_t *in, const uint64_t *in_offsets,
                                      uint64_t n_blocks, uint8_t *out, uint64_t out_capacity,
                                      uint64_t *out_offsets, int32_t *status)
 {
-    if (!ctx) return REDUX_INVALID_INPUT;
-    ctx->model_freq = model_freq;
-    const int rc = redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity,
-                                      out_offsets, status);
-    ctx->model_freq = nullptr;
-    return rc;
+    if (!model_freq) return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity,
+                                               out_offsets, status);
+    return redux_encode_batch_models(ctx, model_kind, params, model_freq, 1, nullptr, in, in_offsets, n_blocks, out,
+                                     out_capacity, out_offsets, status);
 }
 
 extern "C" int redux_decode_batch_ex(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
@@ -1812,12 +1940,10 @@ extern "C" int redux_decode_batch_ex(redux_ctx_t *ctx, int model_kind, const red
                                      uint64_t n_blocks, uint8_t *raw, const uint64_t *raw_offsets,
                                      uint64_t *raw_lens, uint64_t *consumed, int32_t *status)
 {
-    if (!ctx) return REDUX_INVALID_INPUT;
-    ctx->model_freq = model_freq;
-    const int rc = redux_decode_batch(ctx, model_kind, params, comp, comp_offsets, n_blocks, raw, raw_offsets,
-                                      raw_lens, consumed, status);
-    ctx->model_freq = nullptr;
-    return rc;
+    if (!model_freq) return redux_decode_batch(ctx, model_kind, params, comp, comp_offsets, n_blocks, raw, raw_offsets,
+                                               raw_lens, consumed, status);
+    return redux_decode_batch_models(ctx, model_kind, params, model_freq, 1, nullptr, comp, comp_offsets, n_blocks, raw,
+                                     raw_offsets, raw_lens, consumed, status);
 }
 
 extern "C" int redux_encode_batch_device_ex(redux_ctx_t *ctx, int device, void *stream, int model_kind,
@@ -1826,12 +1952,12 @@ extern "C" int redux_encode_batch_device_ex(redux_ctx_t *ctx, int device, void *
                                             uint64_t max_block_len, uint8_t *d_out, uint64_t out_capacity,
                                             uint64_t *d_out_offsets, int32_t *d_status)
 {
-    if (!ctx) return REDUX_INVALID_INPUT;
-    ctx->model_freq = model_freq;               // HOST pointer; uploaded and turned into the start tree on `stream`
-    const int rc = redux_encode_batch_device(ctx, device, stream, model_kind, params, d_in, d_in_offsets, n_blocks,
-                                             max_block_len, d_out, out_capacity, d_out_offsets, d_status);
-    ctx->model_freq = nullptr;
-    return rc;
+    // model_freq: HOST pointer; uploaded and turned into the start tree on `stream`
+    if (!model_freq) return redux_encode_batch_device(ctx, device, stream, model_kind, params, d_in, d_in_offsets,
+                                                      n_blocks, max_block_len, d_out, out_capacity, d_out_offsets, d_status);
+    return redux_encode_batch_device_models(ctx, device, stream, model_kind, params, model_freq, 1, nullptr, d_in,
+                                            d_in_offsets, n_blocks, max_block_len, d_out, out_capacity, d_out_offsets,
+                                            d_status);
 }
 
 extern "C" int redux_decode_batch_device_ex(redux_ctx_t *ctx, int device, void *stream, int model_kind,
@@ -1840,10 +1966,10 @@ extern "C" int redux_decode_batch_device_ex(redux_ctx_t *ctx, int device, void *
                                             uint64_t max_block_len, uint8_t *d_raw, const uint64_t *d_raw_offsets,
                                             uint64_t *d_raw_lens, uint64_t *d_consumed, int32_t *d_status)
 {
-    if (!ctx) return REDUX_INVALID_INPUT;
-    ctx->model_freq = model_freq;
-    const int rc = redux_decode_batch_device(ctx, device, stream, model_kind, params, d_comp, d_comp_offsets, n_blocks,
-                                             max_block_len, d_raw, d_raw_offsets, d_raw_lens, d_consumed, d_status);
-    ctx->model_freq = nullptr;
-    return rc;
+    if (!model_freq) return redux_decode_batch_device(ctx, device, stream, model_kind, params, d_comp, d_comp_offsets,
+                                                      n_blocks, max_block_len, d_raw, d_raw_offsets, d_raw_lens,
+                                                      d_consumed, d_status);
+    return redux_decode_batch_device_models(ctx, device, stream, model_kind, params, model_freq, 1, nullptr, d_comp,
+                                            d_comp_offsets, n_blocks, max_block_len, d_raw, d_raw_offsets, d_raw_lens,
+                                            d_consumed, d_status);
 }

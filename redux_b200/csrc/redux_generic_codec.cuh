@@ -46,16 +46,18 @@ struct GenericJob {
     int32_t *status;
     uint32_t *tabs;             // [nsym + 1][n_threads] Fenwick columns
     const uint32_t *init_tree;  // [nsym + 1] tree every block starts from (fresh: tree[i] = lowbit(i))
-    uint32_t init_total;        // its total frequency
+    uint32_t init_total;        // its total frequency; with `models`: the smallest start total of the call
+    BlockModels models;         // a start model per block: block i starts from its row instead of init_tree
     uint32_t s, f, c;
     uint32_t n_threads;
-    // 65-bit reciprocals (redux_common.cuh, make_magic65) of the totals init_total .. init_total + magic_len - 1: the
-    // total is a function of the position only, so the two divisions by it (src/codec.rs:59-60 / :133-134) are two
-    // multiplications; the decoder's division by the range (:131) stays a division
+    // 65-bit reciprocals (redux_common.cuh, make_magic65) of the totals init_total .. init_total + magic_len - 1: a
+    // block's total is a function of its start total and its position, so the two divisions by it
+    // (src/codec.rs:59-60 / :133-134) are two multiplications; the decoder's division by the range (:131) stays a
+    // division
     const Magic64 *magic; uint32_t magic_len;
 };
 
-// reciprocal of the total `count` (init_total <= count < init_total + magic_len by construction of the table)
+// reciprocal of the total `count` (magic_base <= count < magic_base + magic_len by construction of the table)
 __device__ __forceinline__ Magic64 generic_magic(const GenericJob &job, uint32_t count) {
     uint32_t i = count - job.init_total;
     if (i >= job.magic_len) i = job.magic_len - 1;      // only if the caller's max_block_len understated a block: stay in bounds
@@ -64,18 +66,26 @@ __device__ __forceinline__ Magic64 generic_magic(const GenericJob &job, uint32_t
     return g;
 }
 
+// Row of block blk (0 without a table), or false when its index is out of range.
+__device__ __forceinline__ bool generic_row(const GenericJob &job, uint64_t blk, uint32_t &m) {
+    m = 0;
+    return !job.models.start || block_row(job.models, blk, m);
+}
+
 // The reference's AdaptiveTreeModel over one column of `tabs`.
 struct GenericTree {
     uint32_t *t; uint32_t stride;       // node i at t[i * stride]
     uint32_t nsym, eof, total, fmax;
 
-    __device__ __forceinline__ void reset(const GenericJob &job, uint32_t tid, uint32_t *smem_cols) {
+    // start from row m of the call's models (generic_row checked it), or from init_tree without a table
+    __device__ __forceinline__ void reset(const GenericJob &job, uint32_t tid, uint32_t *smem_cols, uint32_t m) {
         if (job.s <= kGenericSmemSymbolBits) { t = smem_cols + threadIdx.x; stride = kGenericThreads; }
         else                                 { t = job.tabs + tid; stride = job.n_threads; }
         eof = 1u << job.s; nsym = eof + 1;
         fmax = (uint32_t)(((uint64_t)1 << job.f) - 1);
-        total = job.init_total;
-        for (uint32_t i = 0; i <= nsym; ++i) t[(size_t)i * stride] = job.init_tree[i];
+        total = job.models.start ? job.models.start[m].x : job.init_total;
+        const uint32_t *init = job.models.start ? job.models.trees + (size_t)m * (nsym + 1) : job.init_tree;
+        for (uint32_t i = 0; i <= nsym; ++i) t[(size_t)i * stride] = init[i];
     }
     // get_frequency_single (adaptive_tree.rs:51-59)
     __device__ __forceinline__ uint32_t prefix(uint32_t i) const {
@@ -126,10 +136,12 @@ encode_generic_kernel(const GenericJob job)
     const uint64_t maxv = (c == 64) ? ~(uint64_t)0 : ((((uint64_t)1) << c) - 1);
     GenericTree tree;
     for (uint64_t blk = tid; blk < job.n_blocks; blk += job.n_threads) {
+        uint32_t m;
+        if (!generic_row(job, blk, m)) { job.sizes[blk] = 0; job.status[blk] = kStatusInvalidInput; continue; }
         const uint64_t off = job.in_off[blk];
         const uint64_t len = job.in_off[blk + 1] - off;
         if (len >= (1ull << 29)) { job.sizes[blk] = 0; job.status[blk] = 5; continue; }
-        tree.reset(job, tid, gen_cols);
+        tree.reset(job, tid, gen_cols, m);
         BitSource src;                                       // read_bits(symbol_bits) over the raw bytes
         src.init(job.in + off, (uint32_t)len);
         BitSink sink;
@@ -173,11 +185,16 @@ decode_generic_kernel(const GenericJob job)
     const uint64_t body = maxv >> 1, half = body + 1;
     GenericTree tree;
     for (uint64_t blk = tid; blk < job.n_blocks; blk += job.n_threads) {
+        uint32_t m;
+        if (!generic_row(job, blk, m)) {
+            job.raw_len[blk] = 0; job.consumed[blk] = 0; job.status[blk] = kStatusInvalidInput;
+            continue;
+        }
         const uint64_t coff = job.in_off[blk];
         const uint64_t clen = job.in_off[blk + 1] - coff;
         const uint64_t roff = job.raw_off[blk];
         if (clen >= (1ull << 29)) { job.raw_len[blk] = 0; job.consumed[blk] = 0; job.status[blk] = 5; continue; }
-        tree.reset(job, tid, gen_cols);
+        tree.reset(job, tid, gen_cols, m);
         BitSource src;
         src.init(job.in + coff, (uint32_t)clen);
         SymbolSink out;
@@ -215,19 +232,21 @@ decode_generic_kernel(const GenericJob job)
     }
 }
 
-// Fenwick tree of a frequency vector freq[0..nsym) (adaptive_tree.rs layout: node i covers the lowbit(i)
-// symbols ending at symbol i-1).  init_tree has nsym + 1 entries; returns nothing, total is summed by the
-// host.  One thread per node; tiny, runs once per call.
-__global__ void build_tree_kernel(const uint32_t *freq, uint32_t nsym, uint32_t *tree)
+// Fenwick trees of n_models frequency vectors freq[m * nsym ..][0..nsym) (adaptive_tree.rs layout: node i covers the
+// lowbit(i) symbols ending at symbol i-1) into tree[m * (nsym + 1) ..], nsym + 1 entries each; freq == NULL: one fresh
+// model (every frequency 1).  The totals are summed by the host.  One thread per node; tiny, runs once per call.
+__global__ void build_tree_kernel(const uint32_t *freq, uint32_t nsym, uint32_t *tree, uint32_t n_models = 1)
 {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i > nsym) return;
+    const uint64_t k = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= (uint64_t)n_models * (nsym + 1)) return;
+    const uint32_t m = (uint32_t)(k / (nsym + 1)), i = (uint32_t)(k % (nsym + 1));
+    const uint32_t *fm = freq ? freq + (size_t)m * nsym : nullptr;
     uint32_t sum = 0;
     if (i > 0) {
         const uint32_t lb = i & (0u - i);
-        for (uint32_t j = i - lb; j < i; ++j) sum += freq ? freq[j] : 1u;
+        for (uint32_t j = i - lb; j < i; ++j) sum += fm ? fm[j] : 1u;
     }
-    tree[i] = sum;
+    tree[k] = sum;
 }
 
 }  // namespace rdx

@@ -475,6 +475,39 @@ __device__ __forceinline__ BitSink2::Code encode_core_al(uint32_t &L, uint32_t &
     return cd;
 }
 
+// ------------------------------------------------------------------ start state of one stream
+// The job's start model (a fresh one: 257 / 1, tree[i] = lowbit(i)), or the block's row of the call's model table
+// (BlockModels).  The job's reciprocal table and freeze point belong to the job's count0; a lane that starts from
+// total count0' reads the table from entry count0' - count0 on (entry t <-> count0' + t) and freezes after
+// tcap + count0 - count0' = FMAX - count0' updates.  The frozen total is FMAX for every model, so the frozen reciprocal
+// stays a launch constant.  false: the block's row index is out of range; the start state is then row 0's, so that
+// every address the kernel forms stays in the table, and the kernel codes an empty block and reports
+// REDUX_INVALID_INPUT.  (The kernels keep one exit: an early return for such a block costs the encoder's table loads
+// their uniform shared-memory base operand.)
+template <typename M>
+struct StreamStart {
+    uint32_t count0, eof_freq, tcap;
+    const uint32_t *tree;       // NULL: fresh
+    const M *magic;
+    template <typename J>
+    __device__ __forceinline__ bool init(const J &job, uint64_t blk) {
+        count0 = job.count0; eof_freq = job.eof_freq; tree = job.init_tree; tcap = job.tcap;
+        magic = reinterpret_cast<const M *>(job.magic);
+        bool ok = true;
+        if (job.models.start) {
+            uint32_t m;
+            ok = block_row(job.models, blk, m);
+            if (!ok) m = 0;
+            const uint2 s = __ldg(job.models.start + m);
+            count0 = s.x; eof_freq = s.y;
+            tree = job.models.trees + (size_t)m * (kNsym + 1);
+            magic += (int32_t)(count0 - job.count0);
+            tcap = job.tcap + job.count0 - count0;
+        }
+        return ok;
+    }
+};
+
 // ------------------------------------------------------------------ encoder
 template <typename TW, int CLS, bool FULL, bool C32>
 __global__ void __launch_bounds__(kLaneThreads, 2)
@@ -487,17 +520,19 @@ encode_lane_al_kernel(const LaneEncJob job)
     const uint64_t blk = (uint64_t)blockIdx.x * kLaneThreads + threadIdx.x;
     if (blk >= job.n_blocks) return;
 
+    StreamStart<M> st;
+    const bool valid = st.init(job, blk);    // false: code an empty block, report it
     LaneTable2<TW, FULL> tab;
     tab.init(smem_u4, warp, lane);
-    tab.reset(job.init_tree);
+    tab.reset(st.tree);
 
     const uint64_t off = job.in_off[blk];
-    const uint32_t len = (uint32_t)(job.in_off[blk + 1] - off);
+    const uint32_t len = valid ? (uint32_t)(job.in_off[blk + 1] - off) : 0u;
     const uint32_t c = job.c, sh = 32 - c;
     const uint32_t one = pinned(job.one, off);
-    const uint32_t count0 = job.count0, eof_freq = job.eof_freq;   // 257 and 1 for a fresh model
-    const M *magic = reinterpret_cast<const M *>(job.magic);
-    const uint32_t tcap = job.tcap;
+    const uint32_t count0 = st.count0, eof_freq = st.eof_freq;
+    const M *magic = st.magic;
+    const uint32_t tcap = st.tcap;
 
     ByteSource3 src;
     src.init(job.in + off, len, lane_stage_slot<TW>(smem_u4));
@@ -590,8 +625,9 @@ encode_lane_al_kernel(const LaneEncJob job)
     const uint32_t shifts = encode_step_al<CLS, C32>(L, H, pend, sink, cum256f, countf, countf, gf, sh, one);
     const uint32_t extra = c - shifts;
     sink.put_code(top_bits(L, extra), extra, pend, 0);
-    job.sizes[blk] = sink.finish();
-    job.status[blk] = 0;
+    const uint32_t bytes = sink.finish();
+    job.sizes[blk] = valid ? bytes : 0u;
+    job.status[blk] = valid ? 0 : kStatusInvalidInput;
     StageSlot::wait<0>();                                  // nothing of this thread may still be in flight at exit
 }
 
@@ -1074,12 +1110,14 @@ decode_lane_al_kernel(const LaneDecJob job)
         __syncthreads();
     }
     if (blk >= job.n_blocks) return;
-    d.tab.reset(job.init_tree);
+    StreamStart<M> st;
+    const bool valid = st.init(job, blk);    // false: decode an empty stream, report it
+    d.tab.reset(st.tree);
 
     const uint64_t coff = job.comp_off[blk];
-    const uint64_t clen = job.comp_off[blk + 1] - coff;
+    const uint64_t clen = valid ? job.comp_off[blk + 1] - coff : 0u;     // no bits: nothing is read or written
     const uint64_t roff = job.raw_off[blk];
-    const uint64_t cap64 = job.raw_off[blk + 1] - roff;
+    const uint64_t cap64 = valid ? job.raw_off[blk + 1] - roff : 0u;
     if (clen >= (1ull << 29)) {                 // 32-bit bit counters; such a stream is not lane work
         job.raw_len[blk] = 0; job.consumed[blk] = 0; job.status[blk] = 5;
         return;
@@ -1087,13 +1125,13 @@ decode_lane_al_kernel(const LaneDecJob job)
     const uint32_t c = job.c;
     const uint32_t cap = cap64 > 0xFFFFFFFEull ? 0xFFFFFFFEu : (uint32_t)cap64;
     const uint32_t total_bits = (uint32_t)clen * 8;
-    d.sh = 32 - c; d.one = job.one; d.count0 = job.count0; d.eof_freq = job.eof_freq;
+    d.sh = 32 - c; d.one = job.one; d.count0 = st.count0; d.eof_freq = st.eof_freq;
     uint32_t *scratch = reinterpret_cast<uint32_t *>(job.consumed + blk);   // this thread's own word until the end
     d.out.init(job.raw + roff, scratch);
     d.st = 0; d.t = 0;
     d.L = 0; d.H = 0xFFFFFFFFu; d.V = 0; d.left = 0;
-    const M *magic = reinterpret_cast<const M *>(job.magic);
-    const uint32_t tcap = job.tcap;
+    const M *magic = st.magic;
+    const uint32_t tcap = st.tcap;
 
     // src/codec.rs:124-127: prime code_bits bits (Err(Eof) if the stream is shorter)
     if (total_bits < c) {
@@ -1115,7 +1153,7 @@ decode_lane_al_kernel(const LaneDecJob job)
     d.out.finish(scratch);
     job.raw_len[blk] = d.t;
     job.consumed[blk] = (total_bits - d.left + 7) >> 3;
-    job.status[blk] = d.st < 0 ? 0 : d.st;
+    job.status[blk] = !valid ? kStatusInvalidInput : d.st < 0 ? 0 : d.st;
     StageSlot::wait<0>();                                  // nothing of this thread may still be in flight at exit
 }
 

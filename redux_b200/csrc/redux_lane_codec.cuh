@@ -45,6 +45,24 @@ constexpr int kTabNodes = 256;                      // nodes 0..255 (node 0 stay
 constexpr int kTabZeroRowBytes = 128;
 constexpr int kTabPadBytes = kTabZeroRowBytes + kLaneThreads * 4;
 
+// The models the blocks of a call start from (trained models: the tuned lane kernels and the generic kernels).  Row m
+// is one model: trees[m * (symbol_count + 1) ..] is its Fenwick tree (adaptive_tree.rs layout, build_tree_kernel) and
+// start[m] = {total frequency, frequency of EOF}.  Block i of the launch starts from row block_model[i] (NULL: row 0);
+// a row index >= n_models makes the block fail with REDUX_INVALID_INPUT before anything is read from the table.
+struct BlockModels {
+    const uint32_t *trees = nullptr;
+    const uint2 *start = nullptr;        // NULL: no table, every block starts from the job's own start model
+    const uint32_t *block_model = nullptr;
+    uint32_t n_models = 0;
+};
+constexpr int32_t kStatusInvalidInput = 2;          // REDUX_INVALID_INPUT
+
+// Row of block blk, or false when its index is out of range.
+__device__ __forceinline__ bool block_row(const BlockModels &bm, uint64_t blk, uint32_t &m) {
+    m = bm.block_model ? __ldg(bm.block_model + blk) : 0u;
+    return m < bm.n_models;
+}
+
 struct LaneEncJob {
     const uint8_t *in;          // raw bytes
     const uint64_t *in_off;     // [n_blocks+1]
@@ -53,14 +71,17 @@ struct LaneEncJob {
     uint64_t slot_stride;
     uint32_t *sizes;            // [n_blocks] compressed bytes
     int32_t *status;            // [n_blocks]
-    const void *magic;          // Magic32/Magic64 [magic_len], entry tt <-> count 257+tt
+    const void *magic;          // Magic32/Magic64 [magic_len], entry tt <-> count count0 + tt
     uint32_t f, c;
-    uint32_t tcap;              // FMAX - NSYM: number of model updates before the freeze
+    uint32_t tcap;              // FMAX - count0: number of model updates before the freeze
     uint32_t one;               // 1 << (32 - c) for c <= 32 (redux_lane_al.cuh), else 0
-    // pre-trained start state (tuned kernels only): NULL / 257 / 1 for a fresh model
+    // the start model every block starts from (tuned kernels only): NULL / 257 / 1 for a fresh model
     const uint32_t *init_tree;  // tree[0..255] of the start model (adaptive_tree.rs layout), or NULL
-    uint32_t count0;            // its total frequency; `magic` entry t <-> count0 + t, tcap = FMAX - count0
+    uint32_t count0;            // its total frequency
     uint32_t eof_freq;          // frequency of the EOF symbol: cum(256) = total - eof_freq
+    // a start model per block (tuned kernels only): block i starts from its row instead; `magic` and `tcap` stay
+    // those of count0 above, and the kernel offsets them by the row's total (StreamStart, redux_lane_al.cuh)
+    BlockModels models;
     // reciprocal of the frozen total FMAX (= magic[tcap]) as launch constants: the frozen loops read it from the
     // constant bank, so no in-loop instruction depends on a global load's scoreboard (tuned kernels only)
     uint64_t gf_m; uint32_t gf_sh;
@@ -81,6 +102,7 @@ struct LaneDecJob {
     uint32_t one;               // as in LaneEncJob
     const uint32_t *init_tree;  // as in LaneEncJob
     uint32_t count0, eof_freq;
+    BlockModels models;         // as in LaneEncJob
     uint64_t gf_m; uint32_t gf_sh;   // as in LaneEncJob
 };
 
