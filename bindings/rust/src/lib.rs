@@ -92,6 +92,14 @@ extern "C" {
                                             d_block_model: *const u32, d_comp: *const u8, d_comp_offsets: *const u64,
                                             n_blocks: u64, max_block_len: u64, d_raw: *mut u8, d_raw_offsets: *const u64,
                                             d_raw_lens: *mut u64, d_consumed: *mut u64, d_status: *mut i32) -> c_int;
+    // one trained frequency row per sample (n_samples x symbol_count); model_freqs / sample_model are host memory
+    pub fn redux_train_models(ctx: *mut redux_ctx_t, p: *const redux_params_t, model_freqs: *const u32, n_models: u32,
+                              sample_model: *const u32, input: *const u8, in_offsets: *const u64, n_samples: u64,
+                              out_freqs: *mut u32) -> c_int;
+    pub fn redux_train_models_device(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, p: *const redux_params_t,
+                                     model_freqs: *const u32, n_models: u32, sample_model: *const u32,
+                                     d_in: *const u8, d_in_offsets: *const u64, n_samples: u64, max_sample_len: u64,
+                                     d_out_freqs: *mut u32) -> c_int;
     pub fn redux_ctx_synchronize(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void) -> c_int;
 }
 

@@ -200,6 +200,29 @@ int redux_decode_batch_models(redux_ctx_t *ctx, int model_kind, const redux_para
                               uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
                               uint64_t *consumed, int32_t *status);
 
+/* ---- training start models on the device.  Sample i (in[in_offsets[i] .. in_offsets[i+1])) trains a copy of start
+ * row sample_model[i] exactly as the reference's Model::get_frequency(sym) (src/model/mod.rs:23-25) would for every
+ * symbol its BitReader yields from the sample (symbol_bits at a time, MSB-first, a trailing partial symbol dropped:
+ * src/bitio/mod.rs:94-108): the start row plus the histogram of the first min(n_sym, freq_max - total(row)) symbols,
+ * n_sym = floor(8 * len / symbol_bits).  The EOF entry never changes.  Both model kinds train to the same vector, so
+ * there is no model_kind argument.  out_freqs receives n_samples rows of symbol_count entries.
+ * model_freqs / n_models / sample_model follow redux_encode_batch_models (host memory in both forms; each row checked
+ * the same way, and an invalid row or an index >= n_models gives REDUX_INVALID_INPUT before anything launches, named
+ * by redux_ctx_last_error); model_freqs == NULL with n_models == 0 starts every sample from a fresh model.
+ * symbol_bits > 16 gives REDUX_UNSUPPORTED; n_samples == 0 does nothing.  The host form runs on the context's first
+ * device and returns when out_freqs is written.  Without a device both return REDUX_CUDA_ERROR. */
+int redux_train_models(redux_ctx_t *ctx, const redux_params_t *params,
+                       const uint32_t *model_freqs, uint32_t n_models, const uint32_t *sample_model,
+                       const uint8_t *in, const uint64_t *in_offsets, uint64_t n_samples,
+                       uint32_t *out_freqs);
+/* The same on device-resident buffers (d_in under the alignment contract below, d_in_offsets[n_samples+1],
+ * d_out_freqs[n_samples x symbol_count]; model_freqs and sample_model stay HOST pointers, copied during the call),
+ * enqueued on `stream` like the other _device calls.  max_sample_len: an upper bound of every sample's length. */
+int redux_train_models_device(redux_ctx_t *ctx, int device, void *stream, const redux_params_t *params,
+                              const uint32_t *model_freqs, uint32_t n_models, const uint32_t *sample_model,
+                              const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_samples,
+                              uint64_t max_sample_len, uint32_t *d_out_freqs);
+
 /* ---- batch, device-resident buffers (kernel-only timing; all pointers are device memory on
  * `device`, which must be one of the context's devices; work is enqueued on `stream` (a
  * cudaStream_t; NULL = the CUDA default stream) and is asynchronous to the host).

@@ -156,6 +156,8 @@ def lib():
     L.redux_decode_batch_models.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, vp, vp, vp, vp]
     L.redux_encode_batch_device_models.argtypes = [vp, i32, vp, i32, pp, vp, u32, vp, vp, vp, u64, u64, vp, u64, vp, vp]
     L.redux_decode_batch_device_models.argtypes = [vp, i32, vp, i32, pp, vp, u32, vp, vp, vp, u64, u64, vp, vp, vp, vp, vp]
+    L.redux_train_models.argtypes = [vp, pp, vp, u32, vp, vp, vp, u64, vp]
+    L.redux_train_models_device.argtypes = [vp, i32, vp, pp, vp, u32, vp, vp, vp, u64, u64, vp]
     _lib = L
     return L
 
@@ -338,6 +340,33 @@ def _model_table(models):
 
 def _block_model(block_model):
     return None if block_model is None else np.ascontiguousarray(block_model, dtype=np.uint32)
+
+
+def _train_start(start, n):
+    """(class, Parameters, C parameters, start table or None, n_models, sample_model or None) of the `start` argument of
+    train_models: one model for every sample (None table when it is fresh), or a list of n models, sample i starting
+    from start[i]."""
+    if isinstance(start, Model):
+        p = start.params
+        if start.freq is None:
+            return type(start), p, p._c(), None, 0, None
+        return type(start), p, p._c(), np.ascontiguousarray(start.freq, dtype=np.uint32)[None, :], 1, None
+    start = list(start)
+    if len(start) != n:
+        raise InvalidInput("train_models: %d start models for %d samples" % (len(start), n))
+    if n == 0:
+        raise InvalidInput("train_models: an empty list of start models names no Parameters")
+    _, pc, table = _model_table(start)
+    return type(start[0]), start[0].params, pc, table, n, np.arange(n, dtype=np.uint32)
+
+
+def _trained_models(cls, params, rows):
+    out = []
+    for r in rows:
+        m = cls(params)
+        m.freq = r.copy()
+        out.append(m)
+    return out
 
 
 def _ptr(x):
@@ -551,6 +580,30 @@ class Context:
         if check:
             _raise(rc, self)
         return raw, raw_lens[:n], consumed[:n], status[:n]
+
+    # ---- training start models on the device (redux_train_models, DESIGN.md 3.9)
+    def train_models(self, data, offsets, start):
+        """One new model per sample: sample i = data[offsets[i]:offsets[i+1]] trains a copy of its start model exactly
+        as get_frequency() of every symbol the reference's reader yields from it would.  start: one model (fresh or
+        trained) for every sample, or a list of n models, sample i starting from start[i].  The models passed in are
+        not modified.  Returns a list of n models of start's kind and Parameters."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        cls, params, pc, table, n_models, sm = _train_start(start, n)
+        out = np.zeros((max(n, 1), params.symbol_count), dtype=np.uint32)
+        _raise(lib().redux_train_models(self._h, C.byref(pc), _ptr(table), n_models, _ptr(sm),
+                                        _ptr(data) if data.size else None, _ptr(offsets), n, _ptr(out)), self)
+        return _trained_models(cls, params, out[:n])
+
+    def train_models_device(self, d_in, d_in_offsets, n_samples, max_sample_len, d_out_freqs, start, device=0,
+                            stream=None):
+        """train_models on device-resident buffers: d_out_freqs (uint32, n_samples x symbol_count) receives the rows.
+        Asynchronous on `stream`; `start` as in train_models (host models)."""
+        _, _, pc, table, n_models, sm = _train_start(start, n_samples)
+        _raise(lib().redux_train_models_device(self._h, device, stream, C.byref(pc), _ptr(table), n_models, _ptr(sm),
+                                               _ptr(d_in), _ptr(d_in_offsets), n_samples, max_sample_len,
+                                               _ptr(d_out_freqs)), self)
 
     # ---- batch, device-resident (tensors or raw device addresses); asynchronous on `stream`
     def encode_batch_device(self, d_in, d_in_offsets, n_blocks, max_block_len, d_out, out_capacity,

@@ -27,6 +27,7 @@
 #include "redux_generic_codec.cuh"
 #include "redux_warp_codec.cuh"
 #include "redux_split_encoder.cuh"
+#include "redux_train.cuh"
 
 using namespace rdx;
 
@@ -239,6 +240,7 @@ struct DeviceState {
     // start models (trained models and the generic path): Fenwick columns of the generic kernels, start trees,
     // uploaded frequencies, {total, EOF frequency} per model, reciprocals of the generic kernels
     DevBuf gen_tabs, gen_init, gen_freq, gen_start, gen_magic;
+    DevBuf train_rows, train_sample;           // redux_train_models: start rows, {row, room} per sample
     uint8_t *text_lut = nullptr;
     DevBuf corpus; uint64_t corpus_len = 0;    // text-class corpus of the synthetic generator (redux_ctx_set_text_corpus)
     std::vector<MagicEntry> magics;
@@ -320,6 +322,8 @@ cudaError_t configure_kernels()
 #undef RDX_CFG
     // generic kernels: Fenwick columns of alphabets up to 7 bits in shared memory (66 KB per CTA at 7 bits)
     if ((e = allow_smem(encode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits))) != cudaSuccess) return e;
+    // training: 64 KiB of sub-histograms per CTA (symbol_bits 11 .. 14)
+    if ((e = allow_smem(train_count_kernel, kTrainSmemWords * sizeof(uint32_t))) != cudaSuccess) return e;
     return allow_smem(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits));
 }
 
@@ -913,7 +917,7 @@ extern "C" void redux_ctx_destroy(redux_ctx_t *ctx)
         for (HostBuf *b : {&d.pin_off, &d.pin_status, &d.pin_aux0, &d.pin_aux1}) b->release();
         for (DevBuf *b : {&d.slots, &d.sizes, &d.flag, &d.st_in, &d.st_off, &d.st_bmod, &d.st_out, &d.st_ooff,
                           &d.st_status, &d.st_aux0, &d.st_aux1, &d.st_roff, &d.corpus, &d.gen_magic, &d.gen_tabs, &d.gen_init,
-                          &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs}) b->release();
+                          &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs, &d.train_rows, &d.train_sample}) b->release();
         for (auto &m : d.magics) cudaFree(m.ptr);
         if (d.text_lut) cudaFree(d.text_lut);
         for (StageRing *r : {d.ring_up, d.ring_down}) if (r) { r->release(); delete r; }
@@ -1972,4 +1976,157 @@ extern "C" int redux_decode_batch_device_ex(redux_ctx_t *ctx, int device, void *
     return redux_decode_batch_device_models(ctx, device, stream, model_kind, params, model_freq, 1, nullptr, d_comp,
                                             d_comp_offsets, n_blocks, max_block_len, d_raw, d_raw_offsets, d_raw_lens,
                                             d_consumed, d_status);
+}
+
+// ================================================================== training start models (DESIGN.md 3.9)
+// redux_train_models: one new frequency row per sample, from the sample's start row plus the histogram of its first
+// min(n_sym, freq_max - total) symbols (redux_train.cuh).  The host checks the rows and the indices before anything
+// launches; the device copies each start row into its output row and the counting kernel adds to it.
+
+namespace {
+
+// What the host hands the training kernels: the start rows (a row of ones when the caller gives none) and
+// {row, freq_max - total(row)} per sample.
+struct TrainSetup {
+    const uint32_t *rows = nullptr; uint32_t n_rows = 0;
+    std::vector<uint32_t> ones;
+    std::vector<uint2> sample;
+    uint32_t s = 8, nsym = 257, max_room = 0;
+};
+
+// A call without a context: no context exists without a device, so say which of the two is missing.
+int train_no_context()
+{
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) { (void)cudaGetLastError(); return REDUX_CUDA_ERROR; }
+    return REDUX_INVALID_INPUT;
+}
+
+int train_setup(redux_ctx *ctx, const redux_params_t *p, const uint32_t *model_freqs, uint32_t n_models,
+                const uint32_t *sample_model, uint64_t n_samples, TrainSetup *t)
+{
+    if (!p) return fail(ctx, REDUX_INVALID_INPUT, "params is NULL");
+    if (!params_valid(p->symbol_bits, p->freq_bits, p->code_bits))
+        return fail(ctx, REDUX_INVALID_INPUT, "Parameters::new rejects these parameters");
+    if (p->symbol_bits > kGenericMaxSymbolBits)
+        return fail(ctx, REDUX_UNSUPPORTED, "device path implements symbol_bits <= 16");
+    t->s = p->symbol_bits;
+    t->nsym = (1u << p->symbol_bits) + 1;
+    const uint32_t fmax = (uint32_t)(((uint64_t)1 << p->freq_bits) - 1);     // freq_bits <= 31
+    std::vector<uint2> starts;
+    if (!model_freqs && n_models == 0) {                     // every sample starts fresh
+        t->ones.assign(t->nsym, 1u);
+        t->rows = t->ones.data(); t->n_rows = 1;
+        starts.assign(1, make_uint2(t->nsym, 1u));
+    } else {
+        ModelScope ms(ctx, model_freqs, n_models, sample_model);   // the row check of the *_models calls
+        int rc = model_starts(ctx, p, &starts);
+        if (rc) return rc;
+        t->rows = model_freqs; t->n_rows = n_models;
+    }
+    t->sample.resize(n_samples);
+    t->max_room = 0;
+    char msg[96];
+    for (uint64_t i = 0; i < n_samples; ++i) {
+        const uint32_t m = sample_model ? sample_model[i] : 0u;
+        if (m >= t->n_rows) {
+            snprintf(msg, sizeof msg, "sample %llu: model index %u >= n_models", (unsigned long long)i, m);
+            return fail(ctx, REDUX_INVALID_INPUT, msg);
+        }
+        const uint32_t room = fmax - starts[m].x;
+        t->sample[i] = make_uint2(m, room);
+        t->max_room = std::max(t->max_room, room);
+    }
+    return REDUX_OK;
+}
+
+// Enqueues the start-row copy and the counting kernel on stream s of device d (one device call in flight, DESIGN.md 4).
+int train_enqueue(redux_ctx *ctx, DeviceState *d, cudaStream_t s, const TrainSetup &t, const uint8_t *d_in,
+                  const uint64_t *d_in_offsets, uint64_t n_samples, uint64_t max_sample_len, uint32_t *d_out)
+{
+    CU_TRY(ctx, ws_acquire(d, s));
+    const size_t row_bytes = (size_t)t.n_rows * t.nsym * sizeof(uint32_t);
+    CU_TRY(ctx, d->train_rows.reserve(row_bytes));
+    CU_TRY(ctx, d->train_sample.reserve(n_samples * sizeof(uint2)));
+    CU_TRY(ctx, cudaMemcpyAsync(d->train_rows.p, t.rows, row_bytes, cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(d->train_sample.p, t.sample.data(), n_samples * sizeof(uint2), cudaMemcpyHostToDevice, s));
+    TrainJob j;
+    j.in = d_in; j.in_off = d_in_offsets;
+    j.table = (const uint32_t *)d->train_rows.p; j.sample = (const uint2 *)d->train_sample.p;
+    j.out = d_out; j.n_samples = n_samples;
+    j.s = t.s; j.nsym = t.nsym;
+    j.chunk = kTrainChunk;
+    // positions any sample can count: below min(n_sym of the longest sample, the largest room)
+    const uint64_t limit = std::min<uint64_t>(max_sample_len * 8 / t.s, t.max_room);
+    j.chunks = (uint32_t)std::max<uint64_t>((limit + kTrainChunk - 1) / kTrainChunk, 1);
+    j.n_ctas = limit ? n_samples * j.chunks : 0;
+    j.copies = train_copies(t.s);
+    train_init_kernel<<<(uint32_t)std::min<uint64_t>(n_samples, 148 * 16), kTrainThreads, 0, s>>>(j);
+    ctx->launches++;
+    CU_TRY(ctx, cudaGetLastError());
+    if (j.n_ctas) {
+        const size_t smem = ((size_t)j.copies << t.s) * sizeof(uint32_t);
+        train_count_kernel<<<(uint32_t)std::min<uint64_t>(j.n_ctas, 0x7FFFFFFFull), kTrainThreads, smem, s>>>(j);
+        ctx->launches++;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    CU_TRY(ctx, ws_release(d, s));
+    return REDUX_OK;
+}
+
+}  // namespace
+
+extern "C" int redux_train_models_device(redux_ctx_t *ctx, int device, void *stream_, const redux_params_t *params,
+                                         const uint32_t *model_freqs, uint32_t n_models, const uint32_t *sample_model,
+                                         const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_samples,
+                                         uint64_t max_sample_len, uint32_t *d_out_freqs)
+{
+    if (!ctx) return train_no_context();
+    TrainSetup t;
+    int rc = train_setup(ctx, params, model_freqs, n_models, sample_model, n_samples, &t);
+    if (rc) return rc;
+    DeviceState *d = find_dev(ctx, device);
+    if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
+    if (n_samples == 0) return REDUX_OK;
+    if (!d_in_offsets || !d_out_freqs || (!d_in && max_sample_len))
+        return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    DeviceGuard g(device);
+    return train_enqueue(ctx, d, (cudaStream_t)stream_, t, d_in, d_in_offsets, n_samples, max_sample_len, d_out_freqs);
+}
+
+extern "C" int redux_train_models(redux_ctx_t *ctx, const redux_params_t *params, const uint32_t *model_freqs,
+                                  uint32_t n_models, const uint32_t *sample_model, const uint8_t *in,
+                                  const uint64_t *in_offsets, uint64_t n_samples, uint32_t *out_freqs)
+{
+    if (!ctx) return train_no_context();
+    TrainSetup t;
+    int rc = train_setup(ctx, params, model_freqs, n_models, sample_model, n_samples, &t);
+    if (rc) return rc;
+    if (n_samples == 0) return REDUX_OK;
+    if (!in_offsets || !out_freqs) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    uint64_t max_len = 0;
+    for (uint64_t i = 0; i < n_samples; ++i) {
+        if (in_offsets[i + 1] < in_offsets[i]) return fail(ctx, REDUX_INVALID_INPUT, "in_offsets decrease");
+        max_len = std::max(max_len, in_offsets[i + 1] - in_offsets[i]);
+    }
+    const uint64_t first = in_offsets[0], total = in_offsets[n_samples] - first;
+    if (!in && total) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    // the context's first device; the work per sample is bounded by freq_max, so one device serves any batch
+    DeviceState *d = &ctx->devs[0];
+    DeviceGuard g(d->device);
+    cudaStream_t s = d->stream;
+    std::vector<uint64_t> off(in_offsets, in_offsets + n_samples + 1);
+    for (uint64_t &o : off) o -= first;
+    const size_t out_bytes = (size_t)n_samples * t.nsym * sizeof(uint32_t);
+    CU_TRY(ctx, d->st_in.reserve(total + 16));               // + 16: the last aligned 16-byte load
+    CU_TRY(ctx, d->st_off.reserve(off.size() * sizeof(uint64_t)));
+    CU_TRY(ctx, d->st_out.reserve(out_bytes));
+    if (total) CU_TRY(ctx, cudaMemcpyAsync(d->st_in.p, in + first, total, cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    rc = train_enqueue(ctx, d, s, t, (const uint8_t *)d->st_in.p, (const uint64_t *)d->st_off.p, n_samples, max_len,
+                       (uint32_t *)d->st_out.p);
+    if (rc) return rc;
+    CU_TRY(ctx, cudaMemcpyAsync(out_freqs, d->st_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
+    CU_TRY(ctx, cudaStreamSynchronize(s));
+    return REDUX_OK;
 }
