@@ -100,6 +100,19 @@ extern "C" {
                                      model_freqs: *const u32, n_models: u32, sample_model: *const u32,
                                      d_in: *const u8, d_in_offsets: *const u64, n_samples: u64, max_sample_len: u64,
                                      d_out_freqs: *mut u32) -> c_int;
+    // each block's start row chosen on the device by its ideal code length (cost_bits: null or n_blocks x n_models);
+    // model_freqs is host memory in every form
+    pub fn redux_select_models(ctx: *mut redux_ctx_t, p: *const redux_params_t, model_freqs: *const u32, n_models: u32,
+                               input: *const u8, in_offsets: *const u64, n_blocks: u64, block_model: *mut u32,
+                               cost_bits: *mut f64) -> c_int;
+    pub fn redux_select_models_device(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, p: *const redux_params_t,
+                                      model_freqs: *const u32, n_models: u32, d_in: *const u8, d_in_offsets: *const u64,
+                                      n_blocks: u64, max_block_len: u64, d_block_model: *mut u32,
+                                      d_cost_bits: *mut f64) -> c_int;
+    pub fn redux_encode_batch_select(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t, model_freqs: *const u32,
+                                     n_models: u32, input: *const u8, in_offsets: *const u64, n_blocks: u64,
+                                     out: *mut u8, out_capacity: u64, out_offsets: *mut u64, status: *mut i32,
+                                     block_model: *mut u32) -> c_int;
     pub fn redux_ctx_synchronize(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void) -> c_int;
 }
 

@@ -223,6 +223,41 @@ int redux_train_models_device(redux_ctx_t *ctx, int device, void *stream, const 
                               const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_samples,
                               uint64_t max_sample_len, uint32_t *d_out_freqs);
 
+/* ---- choosing each block's start model on the device (DESIGN.md 3.10).  Block i (in[in_offsets[i] ..
+ * in_offsets[i+1])) gets block_model[i] = the smallest k whose cost is the least of the block's row, where the cost of
+ * row k is the ideal code length in bits of what compress() codes from that start state: the block's
+ * n = floor(8 * len / symbol_bits) symbols (MSB-first, a trailing partial symbol dropped), the first
+ * m = min(n, freq_max - total) of them adaptively and the rest against the frozen row, then EOF against the frozen
+ * total.  It depends only on the block's symbol histograms; both model kinds give the same cost, so there is no
+ * model_kind argument.  It estimates the stream size; the coder's rounding makes the stream differ from it.
+ * model_freqs / n_models as redux_encode_batch_models (host memory in every form; n_models == 0 or an invalid row is
+ * REDUX_INVALID_INPUT, named by redux_ctx_last_error; a table over REDUX_MAX_MODEL_TABLE_BYTES is REDUX_UNSUPPORTED);
+ * these checks come before a device is needed.  symbol_bits > 16, and a block of 2^31 symbols or more, give
+ * REDUX_UNSUPPORTED.  Without a device every form returns REDUX_CUDA_ERROR.  Costs and choices are deterministic: the
+ * host form, the device form and redux_encode_batch_select give identical results for the same input.
+ * cost_bits: NULL, or n_blocks x n_models doubles (row-major).  The host form runs on the context's first device and
+ * returns when its outputs are written. */
+int redux_select_models(redux_ctx_t *ctx, const redux_params_t *params,
+                        const uint32_t *model_freqs, uint32_t n_models,
+                        const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                        uint32_t *block_model, double *cost_bits);
+/* The same on device-resident buffers (d_in under the alignment contract below, d_in_offsets[n_blocks+1],
+ * d_block_model[n_blocks], d_cost_bits NULL or [n_blocks x n_models]; model_freqs stays a HOST pointer, copied during
+ * the call), enqueued on `stream` like the other _device calls.  max_block_len: an upper bound of every block's length. */
+int redux_select_models_device(redux_ctx_t *ctx, int device, void *stream, const redux_params_t *params,
+                               const uint32_t *model_freqs, uint32_t n_models,
+                               const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_blocks,
+                               uint64_t max_block_len, uint32_t *d_block_model, double *d_cost_bits);
+/* redux_encode_batch_models with block_model chosen on the device as redux_select_models chooses it, in the same
+ * pipeline: each chunk's blocks are selected on the device after their bytes arrive and coded from the chosen rows,
+ * so the data crosses PCIe once.  block_model (host, n_blocks entries) receives the choice.  The streams and the
+ * index equal redux_select_models followed by redux_encode_batch_models with that index. */
+int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                              const uint32_t *model_freqs, uint32_t n_models,
+                              const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                              uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+                              uint32_t *block_model);
+
 /* ---- batch, device-resident buffers (kernel-only timing; all pointers are device memory on
  * `device`, which must be one of the context's devices; work is enqueued on `stream` (a
  * cudaStream_t; NULL = the CUDA default stream) and is asynchronous to the host).

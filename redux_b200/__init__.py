@@ -158,6 +158,9 @@ def lib():
     L.redux_decode_batch_device_models.argtypes = [vp, i32, vp, i32, pp, vp, u32, vp, vp, vp, u64, u64, vp, vp, vp, vp, vp]
     L.redux_train_models.argtypes = [vp, pp, vp, u32, vp, vp, vp, u64, vp]
     L.redux_train_models_device.argtypes = [vp, i32, vp, pp, vp, u32, vp, vp, vp, u64, u64, vp]
+    L.redux_select_models.argtypes = [vp, pp, vp, u32, vp, vp, u64, vp, vp]
+    L.redux_select_models_device.argtypes = [vp, i32, vp, pp, vp, u32, vp, vp, u64, u64, vp, vp]
+    L.redux_encode_batch_select.argtypes = [vp, i32, pp, vp, u32, vp, vp, u64, vp, u64, vp, vp, vp]
     _lib = L
     return L
 
@@ -604,6 +607,53 @@ class Context:
         _raise(lib().redux_train_models_device(self._h, device, stream, C.byref(pc), _ptr(table), n_models, _ptr(sm),
                                                _ptr(d_in), _ptr(d_in_offsets), n_samples, max_sample_len,
                                                _ptr(d_out_freqs)), self)
+
+    # ---- choosing each block's start model on the device (redux_select_models, DESIGN.md 3.10)
+    def select_models(self, data, offsets, models, costs=False):
+        """The start model of each block = data[offsets[i]:offsets[i+1]]: the index into `models` with the smallest
+        ideal code length of the block (the lowest such index on a tie).  models: as in encode_batch_models.  Returns
+        block_model (uint32[n]), or (block_model, costs float64[n, len(models)] in bits) when costs is true."""
+        _, pc, table = _model_table(models)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        block_model = np.zeros(max(n, 1), dtype=np.uint32)
+        cost = np.zeros((max(n, 1), table.shape[0]), dtype=np.float64) if costs else None
+        _raise(lib().redux_select_models(self._h, C.byref(pc), _ptr(table), table.shape[0],
+                                         _ptr(data) if data.size else None, _ptr(offsets), n, _ptr(block_model),
+                                         _ptr(cost)), self)
+        return (block_model[:n], cost[:n]) if costs else block_model[:n]
+
+    def select_models_device(self, d_in, d_in_offsets, n_blocks, max_block_len, models, d_block_model, d_costs=None,
+                             device=0, stream=None):
+        """select_models on device-resident buffers: d_block_model (uint32, n_blocks) receives the choice and d_costs
+        (float64, n_blocks x len(models)), if given, the costs.  Asynchronous on `stream`; models are host models."""
+        _, pc, table = _model_table(models)
+        _raise(lib().redux_select_models_device(self._h, device, stream, C.byref(pc), _ptr(table), table.shape[0],
+                                                _ptr(d_in), _ptr(d_in_offsets), n_blocks, max_block_len,
+                                                _ptr(d_block_model), _ptr(d_costs)), self)
+
+    def encode_batch_select(self, data, offsets, models, out=None, check=True):
+        """encode_batch_models with each block's model chosen on the device as select_models chooses it, in the same
+        pass over the data.  Returns (out uint8 array view, out_offsets, status, block_model)."""
+        kind, pc, table = _model_table(models)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        if out is None:
+            lens = offsets[1:] - offsets[:-1]
+            nsym = lens * np.uint64(8) // np.uint64(pc.symbol_bits) + np.uint64(1)
+            cap = int((nsym * np.uint64(pc.code_bits) + np.uint64(7)).sum() // 8) + 8 * n
+            out = np.empty(max(cap, 1), dtype=np.uint8)
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        block_model = np.zeros(max(n, 1), dtype=np.uint32)
+        rc = lib().redux_encode_batch_select(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(data),
+                                             _ptr(offsets), n, _ptr(out), out.size, _ptr(out_off), _ptr(status),
+                                             _ptr(block_model))
+        if check:
+            _raise(rc, self)
+        return out[:int(out_off[n])], out_off, status[:n], block_model[:n]
 
     # ---- batch, device-resident (tensors or raw device addresses); asynchronous on `stream`
     def encode_batch_device(self, d_in, d_in_offsets, n_blocks, max_block_len, d_out, out_capacity,

@@ -18,7 +18,9 @@ the row each block starts from in its segment's index.
     segment := u32 n_blocks  u32 last_block_raw_len  u32 model_index[n_blocks]  u32 comp_size[n_blocks]
                stream[n_blocks]
 A row is a model's frequency vector, fresh (all ones) or trained: every entry >= 1, total <= freq_max.  Block i's
-stream is compress() of the block with a model in that state.  pack / pack_stream still write version 1."""
+stream is compress() of the block with a model in that state.  pack / pack_stream still write version 1.
+pack_models / pack_stream_models take the index from the caller, pack_auto / pack_stream_auto let the device choose it
+(redux_encode_batch_select)."""
 import io
 import struct
 
@@ -121,21 +123,15 @@ def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=N
     return raw_total, out_total + 8
 
 
-def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_blocks=16384, context=None):
-    """pack_stream with a start model per block, as version 2: block i (counted over the whole input) is coded from
-    models[block_model[i]], each model fresh or trained (one kind and one Parameters, byte symbols).  Raises
-    ContainerError for an index out of range, and for a block_model shorter than the blocks of a batch before that batch
-    is coded.  Returns (raw_bytes, container_bytes)."""
-    models = list(models)
+def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode):
+    """Writes a version 2 container of fin's bytes: the header and model table of `models`, then one segment per batch
+    of `batch_blocks` blocks.  encode(data, offsets, first) codes a batch whose first block is block `first` of the
+    input and returns (streams, stream offsets, model index).  Returns (raw_bytes, container_bytes)."""
     kind, pc, table = rb._model_table(models)
     if pc.symbol_bits != 8:
         raise ContainerError("the container stores byte-symbol streams only (symbol_bits must be 8)")
     if table.shape[0] * (table.shape[1] + 1) * 4 > MAX_MODEL_TABLE_BYTES:
         raise ContainerError("model table larger than the library takes in one call")
-    bm = np.ascontiguousarray(block_model, dtype=np.int64).ravel()
-    if bm.size and (bm.min() < 0 or bm.max() >= len(models)):
-        raise ContainerError("block_model holds an index outside the %d models" % len(models))
-    bm = bm.astype(np.uint32)
     fout.write(HEADER.pack(MAGIC, 2, kind, pc.symbol_bits, pc.freq_bits, pc.code_bits, block_len))
     fout.write(struct.pack("<I", table.shape[0]))
     fout.write(table.astype("<u4").tobytes())
@@ -146,12 +142,8 @@ def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_bl
             break
         data = np.frombuffer(chunk, dtype=np.uint8)
         n = (data.size + block_len - 1) // block_len
-        if first + n > bm.size:
-            raise ContainerError("block_model has %d entries for at least %d blocks" % (bm.size, first + n))
-        idx = bm[first:first + n]
-        ctx = context or rb._ctx()
         off = np.minimum(np.arange(n + 1, dtype=np.uint64) * np.uint64(block_len), np.uint64(data.size))
-        comp, coff, _ = ctx.encode_batch_models(data, off, models, idx)
+        comp, coff, idx = encode(data, off, first)
         sizes = (coff[1:] - coff[:-1]).astype("<u4")
         fout.write(struct.pack("<II", n, data.size - (n - 1) * block_len))
         fout.write(idx.astype("<u4").tobytes())
@@ -162,6 +154,41 @@ def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_bl
         first += n
     fout.write(struct.pack("<II", 0, 0))
     return raw_total, out_total + 8
+
+
+def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_blocks=16384, context=None):
+    """pack_stream with a start model per block, as version 2: block i (counted over the whole input) is coded from
+    models[block_model[i]], each model fresh or trained (one kind and one Parameters, byte symbols).  Raises
+    ContainerError for an index out of range, and for a block_model shorter than the blocks of a batch before that batch
+    is coded.  Returns (raw_bytes, container_bytes)."""
+    models = list(models)
+    rb._model_table(models)
+    bm = np.ascontiguousarray(block_model, dtype=np.int64).ravel()
+    if bm.size and (bm.min() < 0 or bm.max() >= len(models)):
+        raise ContainerError("block_model holds an index outside the %d models" % len(models))
+    bm = bm.astype(np.uint32)
+
+    def encode(data, off, first):
+        n = off.size - 1
+        if first + n > bm.size:
+            raise ContainerError("block_model has %d entries for at least %d blocks" % (bm.size, first + n))
+        idx = bm[first:first + n]
+        comp, coff, _ = (context or rb._ctx()).encode_batch_models(data, off, models, idx)
+        return comp, coff, idx
+
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode)
+
+
+def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, context=None):
+    """pack_stream_models with each block's start model chosen on the device (Context.encode_batch_select): the model
+    with the smallest estimated compressed size of the block.  Writes version 2.  Returns (raw_bytes, container_bytes)."""
+    models = list(models)
+
+    def encode(data, off, first):
+        comp, coff, _, idx = (context or rb._ctx()).encode_batch_select(data, off, models)
+        return comp, coff, idx
+
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode)
 
 
 def unpack_stream(fin, fout, context=None):
@@ -232,6 +259,13 @@ def pack_models(data, models, block_model, block_len=65536, context=None):
         raise ContainerError("block_model has %d entries for %d blocks" % (len(block_model), n))
     out = io.BytesIO()
     pack_stream_models(io.BytesIO(data), out, models, block_model, block_len, context=context)
+    return out.getvalue()
+
+
+def pack_auto(data, models, block_len=65536, context=None):
+    """pack with each block's start model chosen on the device (version 2); see pack_stream_auto."""
+    out = io.BytesIO()
+    pack_stream_auto(io.BytesIO(bytes(data)), out, models, block_len, context=context)
     return out.getvalue()
 
 

@@ -27,7 +27,7 @@
 #include "redux_generic_codec.cuh"
 #include "redux_warp_codec.cuh"
 #include "redux_split_encoder.cuh"
-#include "redux_train.cuh"
+#include "redux_select.cuh"
 
 using namespace rdx;
 
@@ -241,6 +241,10 @@ struct DeviceState {
     // uploaded frequencies, {total, EOF frequency} per model, reciprocals of the generic kernels
     DevBuf gen_tabs, gen_init, gen_freq, gen_start, gen_magic;
     DevBuf train_rows, train_sample;           // redux_train_models: start rows, {row, room} per sample
+    // redux_select_models: candidate rows, SelectSetup::meta, {0, no limit} per block of a slice (the histogram pass's
+    // TrainJob::sample), histogram scratch of every stream
+    DevBuf sel_rows, sel_meta, sel_sample, sel_scratch;
+    HostBuf pin_bmod;                          // redux_encode_batch_select: the chosen rows on their way out
     uint8_t *text_lut = nullptr;
     DevBuf corpus; uint64_t corpus_len = 0;    // text-class corpus of the synthetic generator (redux_ctx_set_text_corpus)
     std::vector<MagicEntry> magics;
@@ -259,10 +263,16 @@ struct DeviceState {
 
 struct TimedSpan { cudaEvent_t a, b; int kind; int device; };
 
+namespace { struct SelectSetup; }
+
 // The start models of the running *_models call (redux_encode_batch_models): on = false for a fresh model.
 // freqs: n rows of symbol_count frequencies (host memory); block_model: the row of each block, NULL = row 0 for every
 // block (host memory in the host-buffer calls, device memory in the device-resident ones).
-struct ModelArgs { bool on = false; const uint32_t *freqs = nullptr; uint32_t n = 0; const uint32_t *block_model = nullptr; };
+// select (redux_encode_batch_select): the device chooses each block's row, and chosen (host memory) receives the choice.
+struct ModelArgs {
+    bool on = false; const uint32_t *freqs = nullptr; uint32_t n = 0; const uint32_t *block_model = nullptr;
+    const SelectSetup *select = nullptr; uint32_t *chosen = nullptr;
+};
 
 struct redux_ctx {
     std::vector<DeviceState> devs;
@@ -324,6 +334,8 @@ cudaError_t configure_kernels()
     if ((e = allow_smem(encode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits))) != cudaSuccess) return e;
     // training: 64 KiB of sub-histograms per CTA (symbol_bits 11 .. 14)
     if ((e = allow_smem(train_count_kernel, kTrainSmemWords * sizeof(uint32_t))) != cudaSuccess) return e;
+    // selection: the running histogram of alphabets up to 14 bits (64 KiB at 14 bits)
+    if ((e = allow_smem(select_cost_kernel, sizeof(uint32_t) << kSelectMaxSmemSymbolBits)) != cudaSuccess) return e;
     return allow_smem(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits));
 }
 
@@ -377,22 +389,20 @@ bool choose_split(const redux_ctx *ctx, uint64_t n_blocks, int cls, uint64_t max
     return n_blocks * stride * sizeof(uint2) <= kSplitMaxPairBytes;
 }
 
-// {total, EOF frequency} of every row of the running call's model table, after checking the table: every entry >= 1
+// {total, EOF frequency} of every row of a model table, after checking the table: every entry >= 1
 // and the sum <= freq_max (the observable state of a trained reference model: every symbol at least once, a total
 // that starts at symbol_count and stops growing at freq_max, adaptive_tree.rs:84).
-int model_starts(redux_ctx *ctx, const redux_params_t *p, std::vector<uint2> *starts)
+int check_rows(redux_ctx *ctx, const redux_params_t *p, const uint32_t *freqs, uint32_t n, std::vector<uint2> *starts)
 {
-    const ModelArgs &ma = ctx->models;
-    if (ma.n == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_models is 0");
-    if (!ma.freqs) return fail(ctx, REDUX_INVALID_INPUT, "model_freqs is NULL");
-    if (!ma.block_model && ma.n > 1) return fail(ctx, REDUX_INVALID_INPUT, "block_model is NULL but n_models > 1");
+    if (n == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_models is 0");
+    if (!freqs) return fail(ctx, REDUX_INVALID_INPUT, "model_freqs is NULL");
     const uint64_t nsym = ((uint64_t)1 << p->symbol_bits) + 1, fmax = ((uint64_t)1 << p->freq_bits) - 1;
-    if ((uint64_t)ma.n * (nsym + 1) * sizeof(uint32_t) > REDUX_MAX_MODEL_TABLE_BYTES)
+    if ((uint64_t)n * (nsym + 1) * sizeof(uint32_t) > REDUX_MAX_MODEL_TABLE_BYTES)
         return fail(ctx, REDUX_UNSUPPORTED, "n_models x (symbol_count + 1) start-tree entries exceed REDUX_MAX_MODEL_TABLE_BYTES");
-    starts->resize(ma.n);
+    starts->resize(n);
     char msg[96];
-    for (uint32_t m = 0; m < ma.n; ++m) {
-        const uint32_t *fr = ma.freqs + (size_t)m * nsym;
+    for (uint32_t m = 0; m < n; ++m) {
+        const uint32_t *fr = freqs + (size_t)m * nsym;
         uint64_t total = 0;
         for (uint64_t i = 0; i < nsym; ++i) {
             if (fr[i] < 1) { snprintf(msg, sizeof msg, "model row %u: frequency below 1", m); return fail(ctx, REDUX_INVALID_INPUT, msg); }
@@ -402,6 +412,16 @@ int model_starts(redux_ctx *ctx, const redux_params_t *p, std::vector<uint2> *st
         (*starts)[m] = make_uint2((uint32_t)total, fr[nsym - 1]);
     }
     return REDUX_OK;
+}
+
+// check_rows of the running call's model table, after the checks of its block index.
+int model_starts(redux_ctx *ctx, const redux_params_t *p, std::vector<uint2> *starts)
+{
+    const ModelArgs &ma = ctx->models;
+    if (ma.n == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_models is 0");
+    if (!ma.freqs) return fail(ctx, REDUX_INVALID_INPUT, "model_freqs is NULL");
+    if (!ma.block_model && !ma.select && ma.n > 1) return fail(ctx, REDUX_INVALID_INPUT, "block_model is NULL but n_models > 1");
+    return check_rows(ctx, p, ma.freqs, ma.n, starts);
 }
 
 int make_plan(redux_ctx *ctx, const redux_params_t *p, uint64_t max_block_len, Plan *pl)
@@ -914,10 +934,11 @@ extern "C" void redux_ctx_destroy(redux_ctx_t *ctx)
         if (d.copy) cudaStreamDestroy(d.copy);
         if (d.h2d) cudaStreamDestroy(d.h2d);
         for (int i = 0; i < kPipeStreams; ++i) if (d.pipe[i]) cudaStreamDestroy(d.pipe[i]);
-        for (HostBuf *b : {&d.pin_off, &d.pin_status, &d.pin_aux0, &d.pin_aux1}) b->release();
+        for (HostBuf *b : {&d.pin_off, &d.pin_status, &d.pin_aux0, &d.pin_aux1, &d.pin_bmod}) b->release();
         for (DevBuf *b : {&d.slots, &d.sizes, &d.flag, &d.st_in, &d.st_off, &d.st_bmod, &d.st_out, &d.st_ooff,
                           &d.st_status, &d.st_aux0, &d.st_aux1, &d.st_roff, &d.corpus, &d.gen_magic, &d.gen_tabs, &d.gen_init,
-                          &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs, &d.train_rows, &d.train_sample}) b->release();
+                          &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs, &d.train_rows, &d.train_sample,
+                          &d.sel_rows, &d.sel_meta, &d.sel_sample, &d.sel_scratch}) b->release();
         for (auto &m : d.magics) cudaFree(m.ptr);
         if (d.text_lut) cudaFree(d.text_lut);
         for (StageRing *r : {d.ring_up, d.ring_down}) if (r) { r->release(); delete r; }
@@ -1295,12 +1316,147 @@ void for_each_device(redux_ctx *ctx, size_t nd, std::vector<int> &rcs, F fn)
     }
 }
 
+// ---- selecting start models (redux_select_models, DESIGN.md 3.10)
+// Blocks go through the histogram pass and the cost kernel in slices whose scratch (the full histogram of every block,
+// plus the running histogram above 14 bits) stays under kSelectScratchBytes per stream.
+constexpr size_t kSelectScratchBytes = (size_t)64 << 20;
+constexpr uint64_t kSelectMaxSymbols = (uint64_t)1 << 31;   // a block's symbol count must stay below this (TrainJob)
+
+// What the host hands the selection kernels: the rows, and meta = {total, EOF entry} per model | the model indices by
+// split point freq_max - total ascending | n_groups + 1 group starts | n_groups distinct split points.
+struct SelectSetup {
+    const uint32_t *rows = nullptr; uint32_t n_models = 0;
+    uint32_t s = 8, nsym = 257, n_groups = 0;
+    std::vector<uint32_t> meta;
+    size_t block_bytes() const { return (size_t)nsym * 4 + (s > kSelectMaxSmemSymbolBits ? (size_t)4 << s : 0); }
+};
+
+// The checks of redux_encode_batch_models / redux_train_models on the parameters and the rows (ctx may be NULL).
+int select_setup(redux_ctx *ctx, const redux_params_t *p, const uint32_t *model_freqs, uint32_t n_models, SelectSetup *t)
+{
+    if (!p) return fail(ctx, REDUX_INVALID_INPUT, "params is NULL");
+    if (!params_valid(p->symbol_bits, p->freq_bits, p->code_bits))
+        return fail(ctx, REDUX_INVALID_INPUT, "Parameters::new rejects these parameters");
+    if (p->symbol_bits > kGenericMaxSymbolBits)
+        return fail(ctx, REDUX_UNSUPPORTED, "device path implements symbol_bits <= 16");
+    std::vector<uint2> starts;
+    int rc = check_rows(ctx, p, model_freqs, n_models, &starts);
+    if (rc) return rc;
+    t->rows = model_freqs; t->n_models = n_models;
+    t->s = p->symbol_bits; t->nsym = (1u << p->symbol_bits) + 1;
+    const uint32_t fmax = (uint32_t)(((uint64_t)1 << p->freq_bits) - 1);
+    std::vector<uint32_t> order(n_models);
+    for (uint32_t k = 0; k < n_models; ++k) order[k] = k;
+    std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return starts[a].x > starts[b].x; });
+    std::vector<uint32_t> group, split;
+    for (uint32_t q = 0; q < n_models; ++q) {
+        const uint32_t room = fmax - starts[order[q]].x;
+        if (split.empty() || split.back() != room) { group.push_back(q); split.push_back(room); }
+    }
+    group.push_back(n_models);
+    t->n_groups = (uint32_t)split.size();
+    t->meta.clear();
+    for (const uint2 &st : starts) { t->meta.push_back(st.x); t->meta.push_back(st.y); }
+    t->meta.insert(t->meta.end(), order.begin(), order.end());
+    t->meta.insert(t->meta.end(), group.begin(), group.end());
+    t->meta.insert(t->meta.end(), split.begin(), split.end());
+    return REDUX_OK;
+}
+
+// The selection's device tables on one device, and `streams` scratch areas of `slice` blocks each.
+struct SelectDev {
+    const uint32_t *rows = nullptr, *meta = nullptr;
+    const uint2 *sample = nullptr;
+    uint8_t *scratch = nullptr;
+    uint64_t slice = 0;
+};
+
+// Uploads the tables on `stream` (the rows too unless d_rows already holds them) for launches of up to max_blocks
+// blocks on up to `streams` streams at once.  Work on another stream must wait for `stream` before it reads them.
+int select_prepare(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const SelectSetup &t, const uint32_t *d_rows,
+                   uint64_t max_blocks, int streams, SelectDev *dev)
+{
+    if (!d_rows) {
+        const size_t bytes = (size_t)t.n_models * t.nsym * sizeof(uint32_t);
+        CU_TRY(ctx, d->sel_rows.reserve(bytes));
+        CU_TRY(ctx, cudaMemcpyAsync(d->sel_rows.p, t.rows, bytes, cudaMemcpyHostToDevice, stream));
+        d_rows = (const uint32_t *)d->sel_rows.p;
+    }
+    CU_TRY(ctx, d->sel_meta.reserve(t.meta.size() * sizeof(uint32_t)));
+    CU_TRY(ctx, cudaMemcpyAsync(d->sel_meta.p, t.meta.data(), t.meta.size() * sizeof(uint32_t), cudaMemcpyHostToDevice, stream));
+    dev->slice = std::max<uint64_t>(1, std::min<uint64_t>(max_blocks, kSelectScratchBytes / t.block_bytes()));
+    // the histogram pass counts every symbol of a block: start row 0 (unused), no limit below the block's own
+    const std::vector<uint2> sample(dev->slice, make_uint2(0u, (uint32_t)(kSelectMaxSymbols - 1)));
+    CU_TRY(ctx, d->sel_sample.reserve(dev->slice * sizeof(uint2)));
+    CU_TRY(ctx, cudaMemcpyAsync(d->sel_sample.p, sample.data(), dev->slice * sizeof(uint2), cudaMemcpyHostToDevice, stream));
+    CU_TRY(ctx, d->sel_scratch.reserve((size_t)streams * dev->slice * t.block_bytes()));
+    dev->rows = d_rows; dev->meta = (const uint32_t *)d->sel_meta.p;
+    dev->sample = (const uint2 *)d->sel_sample.p;
+    dev->scratch = (uint8_t *)d->sel_scratch.p;
+    return REDUX_OK;
+}
+
+// Enqueues the selection of n_blocks blocks on stream s with scratch area `slot`: per slice, the histogram pass
+// (train_count_kernel into zeroed rows) and select_cost_kernel.  d_cost: NULL or n_blocks x n_models doubles.
+int select_enqueue(redux_ctx *ctx, cudaStream_t s, const SelectSetup &t, const SelectDev &dev, int slot,
+                   const uint8_t *d_in, const uint64_t *d_in_off, uint64_t n_blocks, uint64_t max_block_len,
+                   uint32_t *d_block_model, double *d_cost)
+{
+    uint8_t *scratch = dev.scratch + (size_t)slot * dev.slice * t.block_bytes();
+    uint32_t *hist = (uint32_t *)scratch, *run = hist + dev.slice * t.nsym;
+    const uint64_t max_n = max_block_len * 8 / t.s;
+    const uint32_t *meta = dev.meta;
+    for (uint64_t first = 0; first < n_blocks; first += dev.slice) {
+        const uint64_t cnt = std::min<uint64_t>(dev.slice, n_blocks - first);
+        CU_TRY(ctx, cudaMemsetAsync(hist, 0, (size_t)cnt * t.nsym * sizeof(uint32_t), s));
+        TrainJob j;
+        j.in = d_in; j.in_off = d_in_off + first;
+        j.table = nullptr; j.sample = dev.sample;
+        j.out = hist; j.n_samples = cnt;
+        j.s = t.s; j.nsym = t.nsym;
+        j.chunk = kTrainChunk;
+        j.chunks = (uint32_t)std::max<uint64_t>((max_n + kTrainChunk - 1) / kTrainChunk, 1);
+        j.n_ctas = max_n ? cnt * j.chunks : 0;
+        j.copies = train_copies(t.s);
+        if (j.n_ctas) {
+            const size_t smem = ((size_t)j.copies << t.s) * sizeof(uint32_t);
+            train_count_kernel<<<(uint32_t)std::min<uint64_t>(j.n_ctas, 0x7FFFFFFFull), kTrainThreads, smem, s>>>(j);
+            ctx->launches++;
+            CU_TRY(ctx, cudaGetLastError());
+        }
+        SelectJob sj;
+        sj.in = d_in; sj.in_off = d_in_off + first;
+        sj.rows = dev.rows;
+        sj.start = (const uint2 *)meta;
+        sj.order = meta + 2 * t.n_models;
+        sj.group = sj.order + t.n_models;
+        sj.split = sj.group + t.n_groups + 1;
+        sj.hist = hist; sj.run = run;
+        sj.block_model = d_block_model + first;
+        sj.cost = d_cost ? d_cost + first * t.n_models : nullptr;
+        sj.n_blocks = cnt;
+        sj.n_models = t.n_models; sj.n_groups = t.n_groups; sj.s = t.s; sj.nsym = t.nsym;
+        const size_t smem = t.s <= kSelectMaxSmemSymbolBits ? sizeof(uint32_t) << t.s : 0;
+        select_cost_kernel<<<(uint32_t)std::min<uint64_t>(cnt, 0x7FFFFFFFull), kSelectThreads, smem, s>>>(sj);
+        ctx->launches++;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    return REDUX_OK;
+}
+
 // The shard's slice of the call's block-to-model index (host memory) goes to the device on the h2d stream, beside the
 // offsets, so every chunk's kernel (which waits for its input on that stream) finds it; *d_bmod stays NULL when the
-// call has no index.
+// call has no index.  When the device chooses the rows (redux_encode_batch_select), the chunks' selections write the
+// index in place, and nothing is uploaded.
 int upload_block_models(redux_ctx *ctx, DeviceState *d, Shard sh, const uint32_t **d_bmod)
 {
     *d_bmod = nullptr;
+    if (ctx->models.select) {
+        CU_TRY(ctx, d->st_bmod.reserve(sh.count * sizeof(uint32_t)));
+        CU_TRY(ctx, d->pin_bmod.reserve(sh.count * sizeof(uint32_t)));
+        *d_bmod = (const uint32_t *)d->st_bmod.p;
+        return REDUX_OK;
+    }
     if (!ctx->models.on || !ctx->models.block_model) return REDUX_OK;
     CU_TRY(ctx, d->st_bmod.reserve(sh.count * sizeof(uint32_t)));
     CU_TRY(ctx, cudaMemcpyAsync(d->st_bmod.p, ctx->models.block_model + sh.first, sh.count * sizeof(uint32_t),
@@ -1490,14 +1646,16 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     const size_t nc = res->chunks.size();
     res->chunk_base.assign(nc, 0); res->chunk_total.assign(nc, 0);
     res->local_off.assign(sh.count + 1, 0);
-    std::vector<uint64_t> chunk_cap(nc);
-    uint64_t dcap = 0;
+    std::vector<uint64_t> chunk_cap(nc), chunk_max(nc, 0);
+    uint64_t dcap = 0, chunk_blocks = 0;
     for (size_t k = 0; k < nc; ++k) {
         uint64_t w = 0;
         for (uint64_t i = 0; i < res->chunks[k].count; ++i) {
             const uint64_t b = res->chunks[k].first + i;
             w += redux_compress_bound_ex(rel[b + 1] - rel[b], pl.s, pl.c);
+            chunk_max[k] = std::max(chunk_max[k], rel[b + 1] - rel[b]);
         }
+        chunk_blocks = std::max(chunk_blocks, res->chunks[k].count);
         chunk_cap[k] = w;
         res->chunk_base[k] = dcap;
         dcap += (w + 15) & ~(uint64_t)15;
@@ -1515,6 +1673,11 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, d->h2d, pl, &magic))) return rc;
     if ((rc = prepare_models(ctx, d, d->h2d, p, sh.count, &pl))) return rc;
+    // redux_encode_batch_select: the rows are on the device already (prepare_models); every chunk stream gets scratch
+    const SelectSetup *sel = ctx->models.select;
+    SelectDev sdev;
+    if (sel && (rc = select_prepare(ctx, d, d->h2d, *sel, (const uint32_t *)d->gen_freq.p, chunk_blocks,
+                                    (int)std::min<size_t>(nc, pipe_streams()), &sdev))) return rc;
     EventSet evs;                       // [0, nc): chunk done; [nc, 2nc): chunk input on the device
     CU_TRY(ctx, evs.create(2 * nc));
     // pageable caller memory goes through the pinned rings (CopyPool); then the enqueue loop below runs on a feeder
@@ -1532,6 +1695,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     int32_t *d_status = (int32_t *)d->st_status.p;
     uint64_t *h_ooff = (uint64_t *)d->pin_off.p;
     int32_t *h_status = (int32_t *)d->pin_status.p;
+    uint32_t *h_bmod = (uint32_t *)d->pin_bmod.p;
     ChunkProgress prog;
     // While the feeder runs it is the only thread that touches ctx (error text, launch counter, timing spans).
     auto enqueue_all = [&]() -> int {
@@ -1546,7 +1710,10 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
                                       : cudaMemcpyAsync(d_in + b0, in + base + b0, b1 - b0, cudaMemcpyHostToDevice, d->h2d);
             if (e == cudaSuccess) e = cudaEventRecord(evs.ev[nc + k], d->h2d);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(s, evs.ev[nc + k], 0);
-            if (e == cudaSuccess)
+            if (e == cudaSuccess && sel)
+                rc2 = select_enqueue(ctx, s, *sel, sdev, (int)(k % pipe_streams()), d_in, d_off + c.first, c.count,
+                                     chunk_max[k], (uint32_t *)d_bmod + c.first, nullptr);
+            if (e == cudaSuccess && rc2 == REDUX_OK)
                 rc2 = encode_launch(ctx, d->device, s, pl, magic, d_in, d_off + c.first, d_bmod ? d_bmod + c.first : nullptr, c.count,
                                     d_out + res->chunk_base[k], chunk_cap[k], d_ooff + c.first + k,
                                     d_status + c.first, (uint8_t *)d->slots.p + c.first * pl.slot_stride,
@@ -1555,6 +1722,8 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
                 e = cudaMemcpyAsync(h_ooff + c.first + k, d_ooff + c.first + k, (c.count + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s);
             if (e == cudaSuccess && rc2 == REDUX_OK)
                 e = cudaMemcpyAsync(h_status + c.first, d_status + c.first, c.count * sizeof(int32_t), cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && rc2 == REDUX_OK && sel)
+                e = cudaMemcpyAsync(h_bmod + c.first, d_bmod + c.first, c.count * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
             if (e == cudaSuccess && rc2 == REDUX_OK) e = cudaEventRecord(evs.ev[k], s);
             if (rc2 != REDUX_OK) return rc2;
             if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, REDUX_CUDA_ERROR, "encode pipeline enqueue", e); }
@@ -1598,6 +1767,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
         const uint64_t *lo = h_ooff + c.first + k;
         for (uint64_t i = 0; i <= c.count; ++i) res->local_off[c.first + i] = pos + lo[i];
         std::memcpy(status + c.first, h_status + c.first, c.count * sizeof(int32_t));
+        if (sel) std::memcpy(ctx->models.chosen + sh.first + c.first, h_bmod + c.first, c.count * sizeof(uint32_t));
         res->chunk_total[k] = lo[c.count];
         if (streaming && (derr = place(k, pos)) != cudaSuccess) { dwhat = "encode pipeline D2H"; break; }
         pos += lo[c.count];
@@ -2129,4 +2299,109 @@ extern "C" int redux_train_models(redux_ctx_t *ctx, const redux_params_t *params
     CU_TRY(ctx, cudaMemcpyAsync(out_freqs, d->st_out.p, out_bytes, cudaMemcpyDeviceToHost, s));
     CU_TRY(ctx, cudaStreamSynchronize(s));
     return REDUX_OK;
+}
+
+// ================================================================== selecting start models (DESIGN.md 3.10)
+// redux_select_models: each block's start row is the candidate with the smallest ideal code length of the block
+// (redux_select.cuh).  The parameters and rows are checked before a context is needed, so a bad call is named the same
+// with or without a device.
+
+namespace {
+
+// Every block's symbol count must stay below 2^31 (the histogram pass's limit).
+int select_check_lengths(redux_ctx *ctx, const SelectSetup &t, const uint64_t *in_offsets, uint64_t n_blocks,
+                         uint64_t *max_len)
+{
+    *max_len = 0;
+    for (uint64_t i = 0; i < n_blocks; ++i) {
+        if (in_offsets[i + 1] < in_offsets[i]) return fail(ctx, REDUX_INVALID_INPUT, "in_offsets decrease");
+        *max_len = std::max(*max_len, in_offsets[i + 1] - in_offsets[i]);
+    }
+    if (*max_len * 8 / t.s >= kSelectMaxSymbols)
+        return fail(ctx, REDUX_UNSUPPORTED, "blocks of 2^31 symbols or more are not supported");
+    return REDUX_OK;
+}
+
+}  // namespace
+
+extern "C" int redux_select_models_device(redux_ctx_t *ctx, int device, void *stream_, const redux_params_t *params,
+                                          const uint32_t *model_freqs, uint32_t n_models, const uint8_t *d_in,
+                                          const uint64_t *d_in_offsets, uint64_t n_blocks, uint64_t max_block_len,
+                                          uint32_t *d_block_model, double *d_cost_bits)
+{
+    SelectSetup t;
+    int rc = select_setup(ctx, params, model_freqs, n_models, &t);
+    if (rc) return rc;
+    if (!ctx) return train_no_context();
+    DeviceState *d = find_dev(ctx, device);
+    if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
+    if (max_block_len * 8 / t.s >= kSelectMaxSymbols)
+        return fail(ctx, REDUX_UNSUPPORTED, "blocks of 2^31 symbols or more are not supported");
+    if (n_blocks == 0) return REDUX_OK;
+    if (!d_in_offsets || !d_block_model || (!d_in && max_block_len)) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    DeviceGuard g(device);
+    cudaStream_t s = (cudaStream_t)stream_;
+    CU_TRY(ctx, ws_acquire(d, s));
+    SelectDev dev;
+    if ((rc = select_prepare(ctx, d, s, t, nullptr, n_blocks, 1, &dev))) return rc;
+    if ((rc = select_enqueue(ctx, s, t, dev, 0, d_in, d_in_offsets, n_blocks, max_block_len, d_block_model, d_cost_bits)))
+        return rc;
+    CU_TRY(ctx, ws_release(d, s));
+    return REDUX_OK;
+}
+
+extern "C" int redux_select_models(redux_ctx_t *ctx, const redux_params_t *params, const uint32_t *model_freqs,
+                                   uint32_t n_models, const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                   uint32_t *block_model, double *cost_bits)
+{
+    SelectSetup t;
+    int rc = select_setup(ctx, params, model_freqs, n_models, &t);
+    if (rc) return rc;
+    if (!ctx) return train_no_context();
+    if (n_blocks == 0) return REDUX_OK;
+    if (!in_offsets || !block_model) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    uint64_t max_len = 0;
+    if ((rc = select_check_lengths(ctx, t, in_offsets, n_blocks, &max_len))) return rc;
+    const uint64_t first = in_offsets[0], total = in_offsets[n_blocks] - first;
+    if (!in && total) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    // the context's first device, like redux_train_models
+    DeviceState *d = &ctx->devs[0];
+    DeviceGuard g(d->device);
+    cudaStream_t s = d->stream;
+    std::vector<uint64_t> off(in_offsets, in_offsets + n_blocks + 1);
+    for (uint64_t &o : off) o -= first;
+    const size_t cost_bytes = cost_bits ? (size_t)n_blocks * n_models * sizeof(double) : 0;
+    CU_TRY(ctx, d->st_in.reserve(total + 16));               // + 16: the last aligned 16-byte load
+    CU_TRY(ctx, d->st_off.reserve(off.size() * sizeof(uint64_t)));
+    CU_TRY(ctx, d->st_bmod.reserve(n_blocks * sizeof(uint32_t)));
+    CU_TRY(ctx, d->st_out.reserve(cost_bytes));
+    if (total) CU_TRY(ctx, cudaMemcpyAsync(d->st_in.p, in + first, total, cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    SelectDev dev;
+    if ((rc = select_prepare(ctx, d, s, t, nullptr, n_blocks, 1, &dev))) return rc;
+    if ((rc = select_enqueue(ctx, s, t, dev, 0, (const uint8_t *)d->st_in.p, (const uint64_t *)d->st_off.p, n_blocks,
+                             max_len, (uint32_t *)d->st_bmod.p, cost_bits ? (double *)d->st_out.p : nullptr))) return rc;
+    CU_TRY(ctx, cudaMemcpyAsync(block_model, d->st_bmod.p, n_blocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    if (cost_bits) CU_TRY(ctx, cudaMemcpyAsync(cost_bits, d->st_out.p, cost_bytes, cudaMemcpyDeviceToHost, s));
+    CU_TRY(ctx, cudaStreamSynchronize(s));
+    return REDUX_OK;
+}
+
+extern "C" int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                         const uint32_t *model_freqs, uint32_t n_models, const uint8_t *in,
+                                         const uint64_t *in_offsets, uint64_t n_blocks, uint8_t *out,
+                                         uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+                                         uint32_t *block_model)
+{
+    SelectSetup t;
+    int rc = select_setup(ctx, params, model_freqs, n_models, &t);
+    if (rc) return rc;
+    if (!ctx) return train_no_context();
+    if (n_blocks && (!in_offsets || !block_model)) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    uint64_t max_len = 0;
+    if ((rc = select_check_lengths(ctx, t, in_offsets, n_blocks, &max_len))) return rc;
+    ModelScope ms(ctx, model_freqs, n_models, nullptr);
+    ctx->models.select = &t;
+    ctx->models.chosen = block_model;
+    return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
 }
