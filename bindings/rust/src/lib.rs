@@ -113,6 +113,28 @@ extern "C" {
                                      n_models: u32, input: *const u8, in_offsets: *const u64, n_blocks: u64,
                                      out: *mut u8, out_capacity: u64, out_offsets: *mut u64, status: *mut i32,
                                      block_model: *mut u32) -> c_int;
+    // zlib's CRC-32 of every block, computed on the device (d_lens: null, or the length of block i at d_in_offsets[i])
+    pub fn redux_crc32_blocks(ctx: *mut redux_ctx_t, input: *const u8, in_offsets: *const u64, n_blocks: u64,
+                              crc: *mut u32) -> c_int;
+    pub fn redux_crc32_blocks_device(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, d_in: *const u8,
+                                     d_in_offsets: *const u64, d_lens: *const u64, n_blocks: u64, max_block_len: u64,
+                                     d_crc: *mut u32) -> c_int;
+    // the batch calls plus crc[n_blocks]: the CRC of each input block (encode) or of each decoded slot (decode)
+    pub fn redux_encode_batch_models_crc(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t,
+                                         model_freqs: *const u32, n_models: u32, block_model: *const u32,
+                                         input: *const u8, in_offsets: *const u64, n_blocks: u64, out: *mut u8,
+                                         out_capacity: u64, out_offsets: *mut u64, status: *mut i32,
+                                         crc: *mut u32) -> c_int;
+    pub fn redux_encode_batch_select_crc(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t,
+                                         model_freqs: *const u32, n_models: u32, input: *const u8,
+                                         in_offsets: *const u64, n_blocks: u64, out: *mut u8, out_capacity: u64,
+                                         out_offsets: *mut u64, status: *mut i32, block_model: *mut u32,
+                                         crc: *mut u32) -> c_int;
+    pub fn redux_decode_batch_models_crc(ctx: *mut redux_ctx_t, model_kind: c_int, p: *const redux_params_t,
+                                         model_freqs: *const u32, n_models: u32, block_model: *const u32,
+                                         comp: *const u8, comp_offsets: *const u64, n_blocks: u64, raw: *mut u8,
+                                         raw_offsets: *const u64, raw_lens: *mut u64, consumed: *mut u64,
+                                         status: *mut i32, crc: *mut u32) -> c_int;
     pub fn redux_ctx_synchronize(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void) -> c_int;
 }
 

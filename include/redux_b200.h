@@ -258,6 +258,48 @@ int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const redux_para
                               uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
                               uint32_t *block_model);
 
+/* ---- CRC-32 of every block on the device (DESIGN.md 3.11).  crc[i] is CRC-32/ISO-HDLC of block i (reflected
+ * polynomial 0xEDB88320, initial value and final XOR 0xFFFFFFFF): the value of zlib's crc32() and crc32fast::hash, so
+ * a consumer can check it without this library.  It is defined on bytes whatever symbol_bits is; an empty block gives
+ * 0.  Block i is in[in_offsets[i] .. in_offsets[i+1]).  NULL buffers and offsets that decrease are
+ * REDUX_INVALID_INPUT; these checks come before a device is needed.  Without a device every form returns
+ * REDUX_CUDA_ERROR.  n_blocks == 0 does nothing.  The host form runs on the context's first device and returns when
+ * crc is written. */
+int redux_crc32_blocks(redux_ctx_t *ctx, const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                       uint32_t *crc);
+/* The same on device-resident buffers (d_in under the alignment contract below, d_in_offsets[n_blocks+1] or, with
+ * d_lens, d_in_offsets[n_blocks]; d_crc[n_blocks]), enqueued on `stream` like the other _device calls.
+ * d_lens == NULL: block i is d_in[d_in_offsets[i] .. d_in_offsets[i+1]); otherwise it is the d_lens[i] bytes at
+ * d_in + d_in_offsets[i], which is what a device-resident decode leaves in its slots and d_raw_lens.
+ * max_block_len: an upper bound of every block's length. */
+int redux_crc32_blocks_device(redux_ctx_t *ctx, int device, void *stream, const uint8_t *d_in,
+                              const uint64_t *d_in_offsets, const uint64_t *d_lens, uint64_t n_blocks,
+                              uint64_t max_block_len, uint32_t *d_crc);
+/* The batch calls with a CRC-32 per block (host memory, n_blocks entries), computed on the device in the same
+ * pipeline: the encode forms over each chunk's input once it is on the device, the decode form over the bytes the
+ * decoder wrote into each slot.  Encode: crc[i] is the CRC of input block i whatever its status (a block with a bad
+ * model index gets an empty stream and still the CRC of its input).  Decode: crc[i] is the CRC of the raw_lens[i]
+ * bytes written into slot i whatever the status (for a truncated stream, of the prefix decoded).  Everything else --
+ * streams, offsets, status, block_model, decoded bytes, lengths, consumed, return code -- is what the call without
+ * _crc returns.  The arguments of that call are checked as it checks them; in addition NULL offsets or crc, and
+ * offsets that decrease, are REDUX_INVALID_INPUT before a device is needed, and without a device every form returns
+ * REDUX_CUDA_ERROR. */
+int redux_encode_batch_models_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                  const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                  const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                  uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+                                  uint32_t *crc);
+int redux_encode_batch_select_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                  const uint32_t *model_freqs, uint32_t n_models,
+                                  const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                  uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+                                  uint32_t *block_model, uint32_t *crc);
+int redux_decode_batch_models_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                  const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                  const uint8_t *comp, const uint64_t *comp_offsets, uint64_t n_blocks,
+                                  uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
+                                  uint64_t *consumed, int32_t *status, uint32_t *crc);
+
 /* ---- batch, device-resident buffers (kernel-only timing; all pointers are device memory on
  * `device`, which must be one of the context's devices; work is enqueued on `stream` (a
  * cudaStream_t; NULL = the CUDA default stream) and is asynchronous to the host).

@@ -63,6 +63,7 @@ class OutCapacity(ReduxError):
 
 
 _ERRORS = {e.code: e for e in (Eof, InvalidInput, IoError, CudaError, Unsupported, OutCapacity)}
+_BLOCK_CODES = (OK, EOF, INVALID_INPUT, OUT_CAPACITY)      # what a batch call returns as one block's status
 
 
 class _ParamsC(C.Structure):
@@ -161,6 +162,11 @@ def lib():
     L.redux_select_models.argtypes = [vp, pp, vp, u32, vp, vp, u64, vp, vp]
     L.redux_select_models_device.argtypes = [vp, i32, vp, pp, vp, u32, vp, vp, u64, u64, vp, vp]
     L.redux_encode_batch_select.argtypes = [vp, i32, pp, vp, u32, vp, vp, u64, vp, u64, vp, vp, vp]
+    L.redux_crc32_blocks.argtypes = [vp, vp, vp, u64, vp]
+    L.redux_crc32_blocks_device.argtypes = [vp, i32, vp, vp, vp, vp, u64, u64, vp]
+    L.redux_encode_batch_models_crc.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, u64, vp, vp, vp]
+    L.redux_encode_batch_select_crc.argtypes = [vp, i32, pp, vp, u32, vp, vp, u64, vp, u64, vp, vp, vp, vp]
+    L.redux_decode_batch_models_crc.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, vp, vp, vp, vp, vp]
     _lib = L
     return L
 
@@ -339,6 +345,13 @@ def _model_table(models):
         if m.freq is not None:
             table[i] = m.freq
     return kind, p._c(), table
+
+
+def _encode_capacity(offsets, pc):
+    lens = offsets[1:] - offsets[:-1]
+    nsym = lens * np.uint64(8) // np.uint64(pc.symbol_bits) + np.uint64(1)
+    cap = int((nsym * np.uint64(pc.code_bits) + np.uint64(7)).sum() // 8) + 8 * (offsets.size - 1)
+    return np.empty(max(cap, 1), dtype=np.uint8)
 
 
 def _block_model(block_model):
@@ -654,6 +667,94 @@ class Context:
         if check:
             _raise(rc, self)
         return out[:int(out_off[n])], out_off, status[:n], block_model[:n]
+
+    # ---- CRC-32 of every block on the device (redux_crc32_blocks, DESIGN.md 3.11)
+    def crc32_blocks(self, data, offsets):
+        """zlib.crc32 of every block data[offsets[i]:offsets[i+1]], computed on the device.  Returns uint32[n]."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        crc = np.zeros(max(n, 1), dtype=np.uint32)
+        _raise(lib().redux_crc32_blocks(self._h, _ptr(data) if data.size else None, _ptr(offsets), n, _ptr(crc)),
+               self)
+        return crc[:n]
+
+    def crc32_blocks_device(self, d_in, d_in_offsets, n_blocks, max_block_len, d_crc, d_lens=None, device=0,
+                            stream=None):
+        """crc32_blocks on device-resident buffers: d_crc (uint32, n_blocks) receives the CRCs.  Block i is
+        d_in[d_in_offsets[i]:d_in_offsets[i+1]], or with d_lens the d_lens[i] bytes at d_in_offsets[i] (a decode's
+        slots and lengths).  Asynchronous on `stream`."""
+        _raise(lib().redux_crc32_blocks_device(self._h, device, stream, _ptr(d_in), _ptr(d_in_offsets), _ptr(d_lens),
+                                               n_blocks, max_block_len, _ptr(d_crc)), self)
+
+    def encode_batch_models_crc(self, data, offsets, models, block_model, out=None, check=True):
+        """encode_batch_models plus the CRC-32 of every input block, computed on the device in the same pass.
+        Returns (out uint8 array view, out_offsets, status, crc uint32[n]).
+        check=False returns the per-block codes (EOF, InvalidInput, OutCapacity) in status instead of raising the first
+        of them.  Unlike the call without _crc, any other failure (CudaError, Unsupported, any code that is not a
+        block's status) still raises with check=False, because status and crc would hold no results then."""
+        kind, pc, table = _model_table(models)
+        bm = _block_model(block_model)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        out = _encode_capacity(offsets, pc) if out is None else out
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        crc = np.zeros(max(n, 1), dtype=np.uint32)
+        rc = lib().redux_encode_batch_models_crc(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(bm),
+                                                 _ptr(data), _ptr(offsets), n, _ptr(out), out.size, _ptr(out_off),
+                                                 _ptr(status), _ptr(crc))
+        if check or rc not in _BLOCK_CODES:
+            _raise(rc, self)
+        return out[:int(out_off[n])], out_off, status[:n], crc[:n]
+
+    def encode_batch_select_crc(self, data, offsets, models, out=None, check=True):
+        """encode_batch_select plus the CRC-32 of every input block.  Returns (out uint8 array view, out_offsets,
+        status, block_model, crc uint32[n]).
+        check=False returns the per-block codes (EOF, InvalidInput, OutCapacity) in status instead of raising the first
+        of them.  Unlike the call without _crc, any other failure (CudaError, Unsupported, any code that is not a
+        block's status) still raises with check=False, because status and crc would hold no results then."""
+        kind, pc, table = _model_table(models)
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        out = _encode_capacity(offsets, pc) if out is None else out
+        out_off = np.zeros(n + 1, dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        block_model = np.zeros(max(n, 1), dtype=np.uint32)
+        crc = np.zeros(max(n, 1), dtype=np.uint32)
+        rc = lib().redux_encode_batch_select_crc(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(data),
+                                                 _ptr(offsets), n, _ptr(out), out.size, _ptr(out_off), _ptr(status),
+                                                 _ptr(block_model), _ptr(crc))
+        if check or rc not in _BLOCK_CODES:
+            _raise(rc, self)
+        return out[:int(out_off[n])], out_off, status[:n], block_model[:n], crc[:n]
+
+    def decode_batch_models_crc(self, comp, comp_offsets, raw_offsets, models, block_model, raw=None, check=True):
+        """decode_batch_models plus the CRC-32 of the raw_lens[i] bytes decoded into every slot.  Returns (raw uint8
+        array, raw_lens, consumed, status, crc uint32[n]).
+        check=False returns the per-block codes (EOF, InvalidInput, OutCapacity) in status instead of raising the first
+        of them.  Unlike the call without _crc, any other failure (CudaError, Unsupported, any code that is not a
+        block's status) still raises with check=False, because status and crc would hold no results then."""
+        kind, pc, table = _model_table(models)
+        bm = _block_model(block_model)
+        comp = np.ascontiguousarray(comp, dtype=np.uint8)
+        comp_offsets = np.ascontiguousarray(comp_offsets, dtype=np.uint64)
+        raw_offsets = np.ascontiguousarray(raw_offsets, dtype=np.uint64)
+        n = comp_offsets.size - 1
+        if raw is None:
+            raw = np.zeros(max(int(raw_offsets[-1]), 1), dtype=np.uint8)
+        raw_lens = np.zeros(max(n, 1), dtype=np.uint64)
+        consumed = np.zeros(max(n, 1), dtype=np.uint64)
+        status = np.zeros(max(n, 1), dtype=np.int32)
+        crc = np.zeros(max(n, 1), dtype=np.uint32)
+        rc = lib().redux_decode_batch_models_crc(self._h, kind, C.byref(pc), _ptr(table), table.shape[0], _ptr(bm),
+                                                 _ptr(comp), _ptr(comp_offsets), n, _ptr(raw), _ptr(raw_offsets),
+                                                 _ptr(raw_lens), _ptr(consumed), _ptr(status), _ptr(crc))
+        if check or rc not in _BLOCK_CODES:
+            _raise(rc, self)
+        return raw, raw_lens[:n], consumed[:n], status[:n], crc[:n]
 
     # ---- batch, device-resident (tensors or raw device addresses); asynchronous on `stream`
     def encode_batch_device(self, d_in, d_in_offsets, n_blocks, max_block_len, d_out, out_capacity,

@@ -20,7 +20,19 @@ the row each block starts from in its segment's index.
 A row is a model's frequency vector, fresh (all ones) or trained: every entry >= 1, total <= freq_max.  Block i's
 stream is compress() of the block with a model in that state.  pack / pack_stream still write version 1.
 pack_models / pack_stream_models take the index from the caller, pack_auto / pack_stream_auto let the device choose it
-(redux_encode_batch_select)."""
+(redux_encode_batch_select).
+
+Version 3 is version 2 plus the CRC-32 of every block's raw bytes (zlib's crc32, computed on the device while the
+block is coded), so a reader can tell a damaged file from a good one:
+
+    header  := "RDXB" u8 version(3) ... exactly as version 2, model table included
+    segment := u32 n_blocks  u32 last_block_raw_len  u32 model_index[n_blocks]  u32 comp_size[n_blocks]
+               u32 crc32[n_blocks]  stream[n_blocks]
+Every writer takes checksum=False; with checksum=True it writes version 3 (pack / pack_stream with a one-row table
+holding the fresh model).  unpack_stream decodes a version 3 segment only when another segment header or the end
+marker follows it, and writes it only after every block of it decoded with status OK, to its expected length,
+consuming exactly its stored size, to bytes whose CRC is the stored one; otherwise it raises ContainerError naming the
+segment (and the block and the check)."""
 import io
 import struct
 
@@ -54,15 +66,15 @@ def read_header(f):
 
 
 def read_header_any(f):
-    """Reads a version 1 or 2 header.  Returns (version, models, block_len): version 1 gives one fresh model.  A
-    version 2 table is checked here: ContainerError for no rows, a table over the library's cap or a row that is not a
-    model's state; Eof when the file ends inside it."""
+    """Reads a version 1, 2 or 3 header.  Returns (version, models, block_len): version 1 gives one fresh model.  A
+    version 2 or 3 table is checked here: ContainerError for no rows, a table over the library's cap or a row that is
+    not a model's state; Eof when the file ends inside it."""
     raw = f.read(HEADER.size)
     if len(raw) != HEADER.size:
         raise ContainerError("container header truncated")      # as read_header
     magic, ver, kind, s, fb, c, block_len = HEADER.unpack(raw)
-    if magic != MAGIC or ver not in (1, 2) or kind not in (rb.MODEL_LINEAR, rb.MODEL_TREE) or block_len == 0:
-        raise ContainerError("not an RDXB v1 or v2 container")
+    if magic != MAGIC or ver not in (1, 2, 3) or kind not in (rb.MODEL_LINEAR, rb.MODEL_TREE) or block_len == 0:
+        raise ContainerError("not an RDXB v1, v2 or v3 container")
     cls = rb.AdaptiveTreeModel if kind == rb.MODEL_TREE else rb.AdaptiveLinearModel
     params = rb.Parameters(s, fb, c)
     if ver == 1:
@@ -88,12 +100,13 @@ def read_header_any(f):
         m = cls(params)
         m.freq = row.copy()
         models.append(m)
-    return 2, models, block_len
+    return ver, models, block_len
 
 
-def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=None):
-    """Reads fin to the end, codes it in batches of `batch_blocks` blocks, writes the container to fout.
-    Returns (raw_bytes, container_bytes)."""
+def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=None, checksum=False):
+    """Reads fin to the end, codes it in batches of `batch_blocks` blocks, writes the container to fout: version 1,
+    or with checksum=True version 3 with a one-row table holding the fresh model.  Returns (raw_bytes,
+    container_bytes)."""
     # The header records the model KIND and Parameters only, and unpack_stream() rebuilds a fresh model from it: a
     # model trained before the call would produce streams nothing in the file says how to decode.  Likewise the
     # segment index stores whole bytes per block: with symbol_bits != 8 the reference drops a trailing partial
@@ -102,6 +115,11 @@ def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=N
         raise ContainerError("the container stores fresh models only (a trained model is not recorded in the header)")
     if model.params.symbol_bits != 8:
         raise ContainerError("the container stores byte-symbol streams only (symbol_bits must be 8)")
+    if checksum:
+        def encode(data, off, first):
+            comp, coff, _, crc = (context or rb._ctx()).encode_batch_models_crc(data, off, [model], None)
+            return comp, coff, np.zeros(off.size - 1, dtype=np.uint32), crc
+        return _pack_stream_v2(fin, fout, [model], block_len, batch_blocks, encode, True)
     ctx = context or rb._ctx()
     write_header(fout, model, block_len)
     raw_total, out_total = 0, HEADER.size
@@ -123,16 +141,17 @@ def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=N
     return raw_total, out_total + 8
 
 
-def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode):
-    """Writes a version 2 container of fin's bytes: the header and model table of `models`, then one segment per batch
-    of `batch_blocks` blocks.  encode(data, offsets, first) codes a batch whose first block is block `first` of the
-    input and returns (streams, stream offsets, model index).  Returns (raw_bytes, container_bytes)."""
+def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum):
+    """Writes a version 2 (checksum: version 3) container of fin's bytes: the header and model table of `models`, then
+    one segment per batch of `batch_blocks` blocks.  encode(data, offsets, first) codes a batch whose first block is
+    block `first` of the input and returns (streams, stream offsets, model index, CRCs; None without checksum).
+    Returns (raw_bytes, container_bytes)."""
     kind, pc, table = rb._model_table(models)
     if pc.symbol_bits != 8:
         raise ContainerError("the container stores byte-symbol streams only (symbol_bits must be 8)")
     if table.shape[0] * (table.shape[1] + 1) * 4 > MAX_MODEL_TABLE_BYTES:
         raise ContainerError("model table larger than the library takes in one call")
-    fout.write(HEADER.pack(MAGIC, 2, kind, pc.symbol_bits, pc.freq_bits, pc.code_bits, block_len))
+    fout.write(HEADER.pack(MAGIC, 3 if checksum else 2, kind, pc.symbol_bits, pc.freq_bits, pc.code_bits, block_len))
     fout.write(struct.pack("<I", table.shape[0]))
     fout.write(table.astype("<u4").tobytes())
     raw_total, out_total, first = 0, HEADER.size + 4 + table.nbytes, 0
@@ -143,24 +162,27 @@ def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode):
         data = np.frombuffer(chunk, dtype=np.uint8)
         n = (data.size + block_len - 1) // block_len
         off = np.minimum(np.arange(n + 1, dtype=np.uint64) * np.uint64(block_len), np.uint64(data.size))
-        comp, coff, idx = encode(data, off, first)
+        comp, coff, idx, crc = encode(data, off, first)
         sizes = (coff[1:] - coff[:-1]).astype("<u4")
         fout.write(struct.pack("<II", n, data.size - (n - 1) * block_len))
         fout.write(idx.astype("<u4").tobytes())
         fout.write(sizes.tobytes())
+        if checksum:
+            fout.write(crc.astype("<u4").tobytes())
         fout.write(comp.tobytes())
         raw_total += data.size
-        out_total += 8 + 4 * n + sizes.nbytes + comp.size
+        out_total += 8 + 4 * n + sizes.nbytes + (4 * n if checksum else 0) + comp.size
         first += n
     fout.write(struct.pack("<II", 0, 0))
     return raw_total, out_total + 8
 
 
-def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_blocks=16384, context=None):
-    """pack_stream with a start model per block, as version 2: block i (counted over the whole input) is coded from
-    models[block_model[i]], each model fresh or trained (one kind and one Parameters, byte symbols).  Raises
-    ContainerError for an index out of range, and for a block_model shorter than the blocks of a batch before that batch
-    is coded.  Returns (raw_bytes, container_bytes)."""
+def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_blocks=16384, context=None,
+                       checksum=False):
+    """pack_stream with a start model per block, as version 2 (checksum=True: version 3): block i (counted over the
+    whole input) is coded from models[block_model[i]], each model fresh or trained (one kind and one Parameters, byte
+    symbols).  Raises ContainerError for an index out of range, and for a block_model shorter than the blocks of a
+    batch before that batch is coded.  Returns (raw_bytes, container_bytes)."""
     models = list(models)
     rb._model_table(models)
     bm = np.ascontiguousarray(block_model, dtype=np.int64).ravel()
@@ -173,44 +195,69 @@ def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_bl
         if first + n > bm.size:
             raise ContainerError("block_model has %d entries for at least %d blocks" % (bm.size, first + n))
         idx = bm[first:first + n]
+        if checksum:
+            comp, coff, _, crc = (context or rb._ctx()).encode_batch_models_crc(data, off, models, idx)
+            return comp, coff, idx, crc
         comp, coff, _ = (context or rb._ctx()).encode_batch_models(data, off, models, idx)
-        return comp, coff, idx
+        return comp, coff, idx, None
 
-    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode)
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum)
 
 
-def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, context=None):
+def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, context=None, checksum=False):
     """pack_stream_models with each block's start model chosen on the device (Context.encode_batch_select): the model
-    with the smallest estimated compressed size of the block.  Writes version 2.  Returns (raw_bytes, container_bytes)."""
+    with the smallest estimated compressed size of the block.  Writes version 2 (checksum=True: version 3).  Returns
+    (raw_bytes, container_bytes)."""
     models = list(models)
 
     def encode(data, off, first):
+        if checksum:
+            comp, coff, _, idx, crc = (context or rb._ctx()).encode_batch_select_crc(data, off, models)
+            return comp, coff, idx, crc
         comp, coff, _, idx = (context or rb._ctx()).encode_batch_select(data, off, models)
-        return comp, coff, idx
+        return comp, coff, idx, None
 
-    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode)
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum)
+
+
+def check_segment(segment, status, raw_lens, lens, used, sizes, crc, stored_crc):
+    """The version 3 reader's checks on one decoded segment, block by block: status OK, the expected length, bytes
+    consumed equal to the stored size, the stored CRC.  Raises ContainerError naming the segment, the block and the
+    first check it fails."""
+    checks = (("status %s", status != rb.OK, status), ("decoded length %s", raw_lens != lens, raw_lens),
+              ("consumed %s bytes of its stream", used != sizes, used), ("CRC-32 %08x", crc != stored_crc, crc))
+    for i in range(len(status)):
+        for what, bad, got in checks:
+            if bad[i]:
+                raise ContainerError("segment %d, block %d: %s, not what the container records"
+                                     % (segment, i, what % (int(got[i]),)))
 
 
 def unpack_stream(fin, fout, context=None):
-    """Inverse of pack_stream and pack_stream_models (version 1 and 2). Returns (container_bytes, raw_bytes). Raises
-    Eof on a truncated file.  Each segment is checked before it is decoded."""
+    """Inverse of pack_stream, pack_stream_models and pack_stream_auto (versions 1, 2 and 3). Returns
+    (container_bytes, raw_bytes). Raises Eof on a truncated file, with one exception: a version 3 file that ends right
+    after a segment (neither the next segment's header nor the end marker follows) raises ContainerError, before that
+    segment is decoded.  Each segment is checked before it is decoded, and a version 3 segment again before its bytes
+    are written (check_segment)."""
     ctx = context
     ver, models, block_len = read_header_any(fin)
-    consumed, raw_total = HEADER.size, 0
-    if ver == 2:
+    consumed, raw_total, segment = HEADER.size, 0, 0
+    if ver >= 2:
         consumed += 4 + 4 * len(models) * models[0].params.symbol_count
+    head = None
     while True:
-        head = fin.read(8)
+        head = head if head is not None else fin.read(8)
         if len(head) != 8:
             raise rb.Eof("container ended inside a segment header")
         n, last = struct.unpack("<II", head)
+        head = None
         consumed += 8
         if n == 0:
             return consumed, raw_total
         if last == 0 or last > block_len:
             raise ContainerError("bad segment")
         idx = None
-        if ver == 2:
+        if ver >= 2:
             raw_idx = fin.read(4 * n)
             if len(raw_idx) != 4 * n:
                 raise rb.Eof("container ended inside a segment's model index")
@@ -222,6 +269,13 @@ def unpack_stream(fin, fout, context=None):
         if len(raw_sizes) != 4 * n:
             raise rb.Eof("container ended inside a segment index")
         sizes = np.frombuffer(raw_sizes, dtype="<u4").astype(np.uint64)
+        stored_crc = None
+        if ver == 3:
+            raw_crc = fin.read(4 * n)
+            if len(raw_crc) != 4 * n:
+                raise rb.Eof("container ended inside a segment's CRCs")
+            stored_crc = np.frombuffer(raw_crc, dtype="<u4").astype(np.uint32)
+            consumed += 4 * n
         coff = np.zeros(n + 1, dtype=np.uint64)
         np.cumsum(sizes, out=coff[1:])
         blob = fin.read(int(coff[-1]))
@@ -232,40 +286,51 @@ def unpack_stream(fin, fout, context=None):
         roff = np.zeros(n + 1, dtype=np.uint64)
         np.cumsum(lens, out=roff[1:])
         comp = np.frombuffer(blob, dtype=np.uint8)
+        if ver == 3:
+            # a checksummed file is whole: the segment is followed by another one or the end marker, checked before
+            # any of it is decoded or written
+            head = fin.read(8)
+            if len(head) != 8:
+                raise ContainerError("segment %d is followed by neither a segment nor the end marker" % segment)
         ctx = ctx or rb._ctx()
         if ver == 1:
             raw, raw_lens, used, status = ctx.decode_batch(comp, coff, roff, models[0])
-        else:
+        elif ver == 2:
             raw, raw_lens, used, status = ctx.decode_batch_models(comp, coff, roff, models, idx)
+        else:
+            raw, raw_lens, used, status, crc = ctx.decode_batch_models_crc(comp, coff, roff, models, idx, check=False)
+            check_segment(segment, status, raw_lens, lens, used, sizes, crc, stored_crc)
         if not (raw_lens == lens).all() or not (used == sizes).all():
             raise ContainerError("a block decoded to an unexpected length")
         fout.write(raw[: int(roff[-1])].tobytes())
         consumed += 4 * n + len(blob)
         raw_total += int(roff[-1])
+        segment += 1
 
 
-def pack(data, model, block_len=65536, context=None):
+def pack(data, model, block_len=65536, context=None, checksum=False):
     out = io.BytesIO()
-    pack_stream(io.BytesIO(bytes(data)), out, model, block_len, context=context)
+    pack_stream(io.BytesIO(bytes(data)), out, model, block_len, context=context, checksum=checksum)
     return out.getvalue()
 
 
-def pack_models(data, models, block_model, block_len=65536, context=None):
-    """pack with a start model per block (version 2); see pack_stream_models.  The whole block_model is checked
-    against the data's block count before anything is coded."""
+def pack_models(data, models, block_model, block_len=65536, context=None, checksum=False):
+    """pack with a start model per block (version 2, checksum=True: version 3); see pack_stream_models.  The whole
+    block_model is checked against the data's block count before anything is coded."""
     data = bytes(data)
     n = (len(data) + block_len - 1) // block_len
     if len(block_model) < n:
         raise ContainerError("block_model has %d entries for %d blocks" % (len(block_model), n))
     out = io.BytesIO()
-    pack_stream_models(io.BytesIO(data), out, models, block_model, block_len, context=context)
+    pack_stream_models(io.BytesIO(data), out, models, block_model, block_len, context=context, checksum=checksum)
     return out.getvalue()
 
 
-def pack_auto(data, models, block_len=65536, context=None):
-    """pack with each block's start model chosen on the device (version 2); see pack_stream_auto."""
+def pack_auto(data, models, block_len=65536, context=None, checksum=False):
+    """pack with each block's start model chosen on the device (version 2, checksum=True: version 3); see
+    pack_stream_auto."""
     out = io.BytesIO()
-    pack_stream_auto(io.BytesIO(bytes(data)), out, models, block_len, context=context)
+    pack_stream_auto(io.BytesIO(bytes(data)), out, models, block_len, context=context, checksum=checksum)
     return out.getvalue()
 
 

@@ -28,6 +28,7 @@
 #include "redux_warp_codec.cuh"
 #include "redux_split_encoder.cuh"
 #include "redux_select.cuh"
+#include "redux_crc.cuh"
 
 using namespace rdx;
 
@@ -245,6 +246,8 @@ struct DeviceState {
     // TrainJob::sample), histogram scratch of every stream
     DevBuf sel_rows, sel_meta, sel_sample, sel_scratch;
     HostBuf pin_bmod;                          // redux_encode_batch_select: the chosen rows on their way out
+    DevBuf st_crc; HostBuf pin_crc;            // the *_crc calls: each chunk's CRCs on their way out
+    int sms = 0;                               // multiprocessors: CTAs of the persistent CRC kernel
     uint8_t *text_lut = nullptr;
     DevBuf corpus; uint64_t corpus_len = 0;    // text-class corpus of the synthetic generator (redux_ctx_set_text_corpus)
     std::vector<MagicEntry> magics;
@@ -269,9 +272,11 @@ namespace { struct SelectSetup; }
 // freqs: n rows of symbol_count frequencies (host memory); block_model: the row of each block, NULL = row 0 for every
 // block (host memory in the host-buffer calls, device memory in the device-resident ones).
 // select (redux_encode_batch_select): the device chooses each block's row, and chosen (host memory) receives the choice.
+// crc (the *_crc calls): host memory that receives each block's CRC-32, of its input (encode) or of its output (decode).
 struct ModelArgs {
     bool on = false; const uint32_t *freqs = nullptr; uint32_t n = 0; const uint32_t *block_model = nullptr;
     const SelectSetup *select = nullptr; uint32_t *chosen = nullptr;
+    uint32_t *crc = nullptr;
 };
 
 struct redux_ctx {
@@ -336,6 +341,8 @@ cudaError_t configure_kernels()
     if ((e = allow_smem(train_count_kernel, kTrainSmemWords * sizeof(uint32_t))) != cudaSuccess) return e;
     // selection: the running histogram of alphabets up to 14 bits (64 KiB at 14 bits)
     if ((e = allow_smem(select_cost_kernel, sizeof(uint32_t) << kSelectMaxSmemSymbolBits)) != cudaSuccess) return e;
+    // CRC-32: the lane-replicated slice-by-4 tables (128 KiB)
+    if ((e = allow_smem(crc32_blocks_kernel, kCrcSmemBytes)) != cudaSuccess) return e;
     return allow_smem(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits));
 }
 
@@ -903,6 +910,7 @@ extern "C" int redux_ctx_create(const int *devices, int n_devices, redux_ctx_t *
         cudaDeviceProp prop;
         if (!g.ok || cudaGetDeviceProperties(&prop, dev) != cudaSuccess) { redux_ctx_destroy(ctx); return REDUX_CUDA_ERROR; }
         if (prop.major < 10) { redux_ctx_destroy(ctx); return REDUX_CUDA_ERROR; }   // sm_100a binary only
+        d.sms = prop.multiProcessorCount;
         bool streams_ok = cudaEventCreateWithFlags(&d.ws_busy, cudaEventDisableTiming) == cudaSuccess &&
                           cudaStreamCreateWithFlags(&d.copy, cudaStreamNonBlocking) == cudaSuccess &&
                           cudaStreamCreateWithFlags(&d.h2d, cudaStreamNonBlocking) == cudaSuccess;
@@ -1465,6 +1473,29 @@ int upload_block_models(redux_ctx *ctx, DeviceState *d, Shard sh, const uint32_t
     return REDUX_OK;
 }
 
+// ---- CRC-32 of every block (redux_crc32_blocks, DESIGN.md 3.11)
+// Enqueues on stream s: zeroes d_crc[n_blocks], then crc32_blocks_kernel over (block, piece) items.  Block i is
+// d_in[d_off[i] .. d_off[i+1]) or, with d_lens, the d_lens[i] bytes at d_in + d_off[i]; max_len bounds every block.
+int crc_enqueue(redux_ctx *ctx, const DeviceState *d, cudaStream_t s, const uint8_t *d_in, const uint64_t *d_off,
+                const uint64_t *d_lens, uint64_t n_blocks, uint64_t max_len, uint32_t *d_crc)
+{
+    if (!n_blocks) return REDUX_OK;
+    CU_TRY(ctx, cudaMemsetAsync(d_crc, 0, n_blocks * sizeof(uint32_t), s));
+    if (!max_len) return REDUX_OK;
+    CrcJob j;
+    j.in = d_in; j.in_off = d_off; j.lens = d_lens; j.crc = d_crc;
+    j.n_blocks = n_blocks;
+    j.piece = kCrcPiece;
+    // a block's padded message spans at most max_len + 30 bytes (15 before its first byte, 15 after its last)
+    j.n_items = n_blocks * ((max_len + 30 + kCrcPiece - 1) / kCrcPiece);
+    const uint64_t ctas = std::min<uint64_t>((j.n_items + kCrcThreads / 32 - 1) / (kCrcThreads / 32),
+                                             (uint64_t)std::max(d->sms, 1) * CrcLib::kMinBlocks);
+    crc32_blocks_kernel<<<(uint32_t)ctas, kCrcThreads, kCrcSmemBytes, s>>>(j);
+    ctx->launches++;
+    CU_TRY(ctx, cudaGetLastError());
+    return REDUX_OK;
+}
+
 // Waits for everything this device still has in flight (used on error paths before buffers are reused).
 void drain(DeviceState *d)
 {
@@ -1670,6 +1701,11 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     CU_TRY(ctx, d->flag.reserve(nc * sizeof(int32_t)));
     CU_TRY(ctx, d->pin_off.reserve((sh.count + nc) * sizeof(uint64_t)));
     CU_TRY(ctx, d->pin_status.reserve(sh.count * sizeof(int32_t)));
+    uint32_t *crc = ctx->models.crc;
+    if (crc) {
+        CU_TRY(ctx, d->st_crc.reserve(sh.count * sizeof(uint32_t)));
+        CU_TRY(ctx, d->pin_crc.reserve(sh.count * sizeof(uint32_t)));
+    }
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, d->h2d, pl, &magic))) return rc;
     if ((rc = prepare_models(ctx, d, d->h2d, p, sh.count, &pl))) return rc;
@@ -1696,6 +1732,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     uint64_t *h_ooff = (uint64_t *)d->pin_off.p;
     int32_t *h_status = (int32_t *)d->pin_status.p;
     uint32_t *h_bmod = (uint32_t *)d->pin_bmod.p;
+    uint32_t *d_crc = (uint32_t *)d->st_crc.p, *h_crc = (uint32_t *)d->pin_crc.p;
     ChunkProgress prog;
     // While the feeder runs it is the only thread that touches ctx (error text, launch counter, timing spans).
     auto enqueue_all = [&]() -> int {
@@ -1710,7 +1747,9 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
                                       : cudaMemcpyAsync(d_in + b0, in + base + b0, b1 - b0, cudaMemcpyHostToDevice, d->h2d);
             if (e == cudaSuccess) e = cudaEventRecord(evs.ev[nc + k], d->h2d);
             if (e == cudaSuccess) e = cudaStreamWaitEvent(s, evs.ev[nc + k], 0);
-            if (e == cudaSuccess && sel)
+            if (e == cudaSuccess && crc)
+                rc2 = crc_enqueue(ctx, d, s, d_in, d_off + c.first, nullptr, c.count, chunk_max[k], d_crc + c.first);
+            if (e == cudaSuccess && rc2 == REDUX_OK && sel)
                 rc2 = select_enqueue(ctx, s, *sel, sdev, (int)(k % pipe_streams()), d_in, d_off + c.first, c.count,
                                      chunk_max[k], (uint32_t *)d_bmod + c.first, nullptr);
             if (e == cudaSuccess && rc2 == REDUX_OK)
@@ -1724,6 +1763,8 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
                 e = cudaMemcpyAsync(h_status + c.first, d_status + c.first, c.count * sizeof(int32_t), cudaMemcpyDeviceToHost, s);
             if (e == cudaSuccess && rc2 == REDUX_OK && sel)
                 e = cudaMemcpyAsync(h_bmod + c.first, d_bmod + c.first, c.count * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && rc2 == REDUX_OK && crc)
+                e = cudaMemcpyAsync(h_crc + c.first, d_crc + c.first, c.count * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
             if (e == cudaSuccess && rc2 == REDUX_OK) e = cudaEventRecord(evs.ev[k], s);
             if (rc2 != REDUX_OK) return rc2;
             if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, REDUX_CUDA_ERROR, "encode pipeline enqueue", e); }
@@ -1768,6 +1809,7 @@ int encode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
         for (uint64_t i = 0; i <= c.count; ++i) res->local_off[c.first + i] = pos + lo[i];
         std::memcpy(status + c.first, h_status + c.first, c.count * sizeof(int32_t));
         if (sel) std::memcpy(ctx->models.chosen + sh.first + c.first, h_bmod + c.first, c.count * sizeof(uint32_t));
+        if (crc) std::memcpy(crc + sh.first + c.first, h_crc + c.first, c.count * sizeof(uint32_t));
         res->chunk_total[k] = lo[c.count];
         if (streaming && (derr = place(k, pos)) != cudaSuccess) { dwhat = "encode pipeline D2H"; break; }
         pos += lo[c.count];
@@ -1885,6 +1927,11 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     CU_TRY(ctx, d->pin_aux0.reserve(sh.count * sizeof(uint64_t)));
     CU_TRY(ctx, d->pin_aux1.reserve(sh.count * sizeof(uint64_t)));
     CU_TRY(ctx, d->pin_status.reserve(sh.count * sizeof(int32_t)));
+    uint32_t *crc = ctx->models.crc;
+    if (crc) {
+        CU_TRY(ctx, d->st_crc.reserve(sh.count * sizeof(uint32_t)));
+        CU_TRY(ctx, d->pin_crc.reserve(sh.count * sizeof(uint32_t)));
+    }
     const void *magic = nullptr;
     if ((rc = get_magic(ctx, d, d->pipe[0], pl, &magic))) return rc;
     if ((rc = prepare_models(ctx, d, d->pipe[0], p, sh.count, &pl))) return rc;
@@ -1904,6 +1951,7 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     int32_t *d_status = (int32_t *)d->st_status.p;
     uint64_t *h_len = (uint64_t *)d->pin_aux0.p, *h_cons = (uint64_t *)d->pin_aux1.p;
     int32_t *h_status = (int32_t *)d->pin_status.p;
+    uint32_t *d_crc = (uint32_t *)d->st_crc.p, *h_crc = (uint32_t *)d->pin_crc.p;
     ChunkProgress prog;
     auto enqueue_all = [&]() -> int {
         int up_slot = 0;
@@ -1921,6 +1969,9 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
             if (e == cudaSuccess)
                 rc2 = decode_launch(ctx, d->device, s, pl, magic, d_comp, d_coff + c.first, d_bmod ? d_bmod + c.first : nullptr, c.count, d_raw,
                                     d_roff + c.first, d_len + c.first, d_cons + c.first, d_status + c.first);
+            // the CRC of the raw_lens[i] bytes the decoder wrote into slot i
+            if (e == cudaSuccess && rc2 == REDUX_OK && crc)
+                rc2 = crc_enqueue(ctx, d, s, d_raw, d_roff + c.first, d_len + c.first, c.count, max_len, d_crc + c.first);
             // the whole slot range of the chunk goes back; bytes beyond raw_lens[i] inside a slot are unspecified
             // (into pageable memory: by the drainer below, through the ring)
             if (e == cudaSuccess && rc2 == REDUX_OK && stage_out) e = cudaEventRecord(evs.ev[nc + k], s);
@@ -1932,6 +1983,8 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
                 e = cudaMemcpyAsync(h_cons + c.first, d_cons + c.first, c.count * sizeof(uint64_t), cudaMemcpyDeviceToHost, s);
             if (e == cudaSuccess && rc2 == REDUX_OK)
                 e = cudaMemcpyAsync(h_status + c.first, d_status + c.first, c.count * sizeof(int32_t), cudaMemcpyDeviceToHost, s);
+            if (e == cudaSuccess && rc2 == REDUX_OK && crc)
+                e = cudaMemcpyAsync(h_crc + c.first, d_crc + c.first, c.count * sizeof(uint32_t), cudaMemcpyDeviceToHost, s);
             if (rc2 != REDUX_OK) return rc2;
             if (e != cudaSuccess) { (void)cudaGetLastError(); return fail(ctx, REDUX_CUDA_ERROR, "decode pipeline enqueue", e); }
             prog.advance();
@@ -1970,6 +2023,7 @@ int decode_shard(redux_ctx *ctx, DeviceState *d, const redux_params_t *p, const 
     std::memcpy(raw_lens + sh.first, h_len, sh.count * sizeof(uint64_t));
     std::memcpy(consumed + sh.first, h_cons, sh.count * sizeof(uint64_t));
     std::memcpy(status + sh.first, h_status, sh.count * sizeof(int32_t));
+    if (crc) std::memcpy(crc + sh.first, h_crc, sh.count * sizeof(uint32_t));
     return REDUX_OK;
 }
 
@@ -2404,4 +2458,132 @@ extern "C" int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const
     ctx->models.select = &t;
     ctx->models.chosen = block_model;
     return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
+}
+
+// ================================================================== CRC-32 of every block (DESIGN.md 3.11)
+// redux_crc32_blocks: zlib's CRC-32 of each block (redux_crc.cuh).  The _crc forms of the batch calls run the same
+// kernel inside encode_shard / decode_shard, over each chunk's input once it is on the device (encode) or over the
+// bytes the decoder wrote into each slot (decode), and bring the CRCs back beside the status.  Arguments are checked
+// before a context is needed, so a bad call is named the same with or without a device.
+
+namespace {
+
+// NULL offsets or outputs, offsets that decrease.
+int crc_check_offsets(redux_ctx *ctx, const uint64_t *off, uint64_t n_blocks, const char *name)
+{
+    if (!off) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    for (uint64_t i = 0; i < n_blocks; ++i)
+        if (off[i + 1] < off[i]) {
+            char msg[96];
+            snprintf(msg, sizeof msg, "%s decrease at block %llu", name, (unsigned long long)i);
+            return fail(ctx, REDUX_INVALID_INPUT, msg);
+        }
+    return REDUX_OK;
+}
+
+}  // namespace
+
+extern "C" int redux_crc32_blocks_device(redux_ctx_t *ctx, int device, void *stream_, const uint8_t *d_in,
+                                         const uint64_t *d_in_offsets, const uint64_t *d_lens, uint64_t n_blocks,
+                                         uint64_t max_block_len, uint32_t *d_crc)
+{
+    if (n_blocks && (!d_in_offsets || !d_crc || (!d_in && max_block_len)))
+        return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if (!ctx) return train_no_context();
+    DeviceState *d = find_dev(ctx, device);
+    if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
+    if (n_blocks == 0) return REDUX_OK;
+    DeviceGuard g(device);
+    cudaStream_t s = (cudaStream_t)stream_;
+    CU_TRY(ctx, ws_acquire(d, s));
+    int rc = crc_enqueue(ctx, d, s, d_in, d_in_offsets, d_lens, n_blocks, max_block_len, d_crc);
+    if (rc) return rc;
+    CU_TRY(ctx, ws_release(d, s));
+    return REDUX_OK;
+}
+
+extern "C" int redux_crc32_blocks(redux_ctx_t *ctx, const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                  uint32_t *crc)
+{
+    if (n_blocks == 0) return ctx ? REDUX_OK : train_no_context();
+    if (!crc) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    int rc = crc_check_offsets(ctx, in_offsets, n_blocks, "in_offsets");
+    if (rc) return rc;
+    const uint64_t first = in_offsets[0], total = in_offsets[n_blocks] - first;
+    if (!in && total) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if (!ctx) return train_no_context();
+    uint64_t max_len = 0;
+    for (uint64_t i = 0; i < n_blocks; ++i) max_len = std::max(max_len, in_offsets[i + 1] - in_offsets[i]);
+    // the context's first device, like redux_train_models
+    DeviceState *d = &ctx->devs[0];
+    DeviceGuard g(d->device);
+    cudaStream_t s = d->stream;
+    std::vector<uint64_t> off(in_offsets, in_offsets + n_blocks + 1);
+    for (uint64_t &o : off) o -= first;
+    CU_TRY(ctx, d->st_in.reserve(total + 16));               // + 16: the last aligned 16-byte load
+    CU_TRY(ctx, d->st_off.reserve(off.size() * sizeof(uint64_t)));
+    CU_TRY(ctx, d->st_crc.reserve(n_blocks * sizeof(uint32_t)));
+    CU_TRY(ctx, ws_acquire(d, s));
+    if (total) CU_TRY(ctx, cudaMemcpyAsync(d->st_in.p, in + first, total, cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    if ((rc = crc_enqueue(ctx, d, s, (const uint8_t *)d->st_in.p, (const uint64_t *)d->st_off.p, nullptr, n_blocks,
+                          max_len, (uint32_t *)d->st_crc.p))) return rc;
+    CU_TRY(ctx, cudaMemcpyAsync(crc, d->st_crc.p, n_blocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    CU_TRY(ctx, ws_release(d, s));
+    CU_TRY(ctx, cudaStreamSynchronize(s));
+    return REDUX_OK;
+}
+
+extern "C" int redux_encode_batch_models_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                             const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                             const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                                             uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets,
+                                             int32_t *status, uint32_t *crc)
+{
+    int rc;
+    if (n_blocks && !crc) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if ((rc = crc_check_offsets(ctx, in_offsets, n_blocks, "in_offsets"))) return rc;
+    if (!ctx) return train_no_context();
+    ModelScope ms(ctx, model_freqs, n_models, block_model);
+    ctx->models.crc = crc;
+    return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
+}
+
+extern "C" int redux_encode_batch_select_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                             const uint32_t *model_freqs, uint32_t n_models, const uint8_t *in,
+                                             const uint64_t *in_offsets, uint64_t n_blocks, uint8_t *out,
+                                             uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
+                                             uint32_t *block_model, uint32_t *crc)
+{
+    int rc;
+    if (n_blocks && !crc) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if ((rc = crc_check_offsets(ctx, in_offsets, n_blocks, "in_offsets"))) return rc;
+    SelectSetup t;
+    if ((rc = select_setup(ctx, params, model_freqs, n_models, &t))) return rc;
+    if (!ctx) return train_no_context();
+    if (n_blocks && !block_model) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    uint64_t max_len = 0;
+    if ((rc = select_check_lengths(ctx, t, in_offsets, n_blocks, &max_len))) return rc;
+    ModelScope ms(ctx, model_freqs, n_models, nullptr);
+    ctx->models.select = &t;
+    ctx->models.chosen = block_model;
+    ctx->models.crc = crc;
+    return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
+}
+
+extern "C" int redux_decode_batch_models_crc(redux_ctx_t *ctx, int model_kind, const redux_params_t *params,
+                                             const uint32_t *model_freqs, uint32_t n_models, const uint32_t *block_model,
+                                             const uint8_t *comp, const uint64_t *comp_offsets, uint64_t n_blocks,
+                                             uint8_t *raw, const uint64_t *raw_offsets, uint64_t *raw_lens,
+                                             uint64_t *consumed, int32_t *status, uint32_t *crc)
+{
+    int rc;
+    if (n_blocks && (!crc || !raw_lens || !consumed || !status)) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if ((rc = crc_check_offsets(ctx, comp_offsets, n_blocks, "comp_offsets"))) return rc;
+    if ((rc = crc_check_offsets(ctx, raw_offsets, n_blocks, "raw_offsets"))) return rc;
+    if (!ctx) return train_no_context();
+    ModelScope ms(ctx, model_freqs, n_models, block_model);
+    ctx->models.crc = crc;
+    return redux_decode_batch(ctx, model_kind, params, comp, comp_offsets, n_blocks, raw, raw_offsets, raw_lens,
+                              consumed, status);
 }
