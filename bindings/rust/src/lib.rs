@@ -113,6 +113,16 @@ extern "C" {
                                      n_models: u32, input: *const u8, in_offsets: *const u64, n_blocks: u64,
                                      out: *mut u8, out_capacity: u64, out_offsets: *mut u64, status: *mut i32,
                                      block_model: *mut u32) -> c_int;
+    // a table of K + 1 start models learned from the blocks (row 0 fresh), each block's row and every round's total
+    // (init, block_model, iteration_cost_bits: null allowed; init is host memory in both forms)
+    pub fn redux_build_models(ctx: *mut redux_ctx_t, p: *const redux_params_t, n_clusters: u32, iterations: u32,
+                              init: *const u32, input: *const u8, in_offsets: *const u64, n_blocks: u64,
+                              out_freqs: *mut u32, block_model: *mut u32, iteration_cost_bits: *mut f64) -> c_int;
+    pub fn redux_build_models_device(ctx: *mut redux_ctx_t, device: c_int, stream: *mut c_void, p: *const redux_params_t,
+                                     n_clusters: u32, iterations: u32, init: *const u32, d_in: *const u8,
+                                     d_in_offsets: *const u64, n_blocks: u64, max_block_len: u64,
+                                     d_out_freqs: *mut u32, d_block_model: *mut u32,
+                                     d_iteration_cost_bits: *mut f64) -> c_int;
     // zlib's CRC-32 of every block, computed on the device (d_lens: null, or the length of block i at d_in_offsets[i])
     pub fn redux_crc32_blocks(ctx: *mut redux_ctx_t, input: *const u8, in_offsets: *const u64, n_blocks: u64,
                               crc: *mut u32) -> c_int;

@@ -258,6 +258,40 @@ int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const redux_para
                               uint8_t *out, uint64_t out_capacity, uint64_t *out_offsets, int32_t *status,
                               uint32_t *block_model);
 
+/* ---- learning a table of start models from the blocks themselves (DESIGN.md 3.12).  Clusters the n_blocks blocks
+ * (in[in_offsets[i] .. in_offsets[i+1])) into n_clusters (K >= 1) groups by their ideal code length, Lloyd style, for
+ * `iterations` (>= 1) rounds.  Membership values are table indices: 0 = coded fresh, k in 1..K = cluster k.  init:
+ * NULL (block b starts in cluster 1 + floor(b K / n_blocks)) or n_blocks values <= K (host memory in both forms).
+ * One round from membership M: G_k = the sum of the symbol histograms of cluster k's blocks; candidate rows
+ * row(G_k, T_l) for every level of the ladder T_l = freq_max >> 2l (while T_l >= 2 symbol_count); row k of the
+ * round's table is the candidate with the least summed cost over cluster k's blocks (lowest l on a tie; level 0 for
+ * an empty cluster), row 0 is fresh (all ones); A = what redux_select_models chooses for that table, and the round's
+ * total is the sum of the chosen costs; the next round starts from M = A.  row(G, T): G = ones if it sums to 0;
+ * r_x = 1 + floor((T - symbol_count) G_x / sum G) for data symbols, the remainder to the bin with the largest G_x
+ * (lowest x on a tie), r_EOF = 1: total exactly T.
+ * out_freqs receives the (K + 1) x symbol_count table of the round with the least total (the earliest on a tie),
+ * block_model (NULL ok) that round's A, and iteration_cost_bits (NULL ok) every round's total in bits.  block_model
+ * equals redux_select_models on the returned table.  Both model kinds give the same result.  Deterministic: the host
+ * and device forms and repeated calls give identical results.
+ * Before a device is needed: K == 0, iterations == 0, an init value above K (named by redux_ctx_last_error) and
+ * n_blocks == 0 are REDUX_INVALID_INPUT; symbol_bits > 16, a table of K + 1 rows over REDUX_MAX_MODEL_TABLE_BYTES, a
+ * block of 2^31 symbols or more, and scratch (histograms, ladder costs, cluster sums, candidates) over
+ * REDUX_MAX_BUILD_SCRATCH_BYTES are REDUX_UNSUPPORTED.  Without a device both forms return REDUX_CUDA_ERROR.  The host
+ * form runs on the context's first device and returns when its outputs are written. */
+#define REDUX_MAX_BUILD_SCRATCH_BYTES ((uint64_t)4 << 30)
+int redux_build_models(redux_ctx_t *ctx, const redux_params_t *params, uint32_t n_clusters, uint32_t iterations,
+                       const uint32_t *init, const uint8_t *in, const uint64_t *in_offsets, uint64_t n_blocks,
+                       uint32_t *out_freqs, uint32_t *block_model, double *iteration_cost_bits);
+/* The same on device-resident buffers (d_in under the alignment contract below, d_in_offsets[n_blocks+1],
+ * d_out_freqs[(K + 1) x symbol_count], d_block_model NULL or [n_blocks], d_iteration_cost_bits NULL or [iterations];
+ * init stays a HOST pointer, copied during the call), enqueued on `stream` like the other _device calls, with no
+ * round trip to the host between rounds.  max_block_len: an upper bound of every block's length. */
+int redux_build_models_device(redux_ctx_t *ctx, int device, void *stream, const redux_params_t *params,
+                              uint32_t n_clusters, uint32_t iterations, const uint32_t *init,
+                              const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_blocks,
+                              uint64_t max_block_len, uint32_t *d_out_freqs, uint32_t *d_block_model,
+                              double *d_iteration_cost_bits);
+
 /* ---- CRC-32 of every block on the device (DESIGN.md 3.11).  crc[i] is CRC-32/ISO-HDLC of block i (reflected
  * polynomial 0xEDB88320, initial value and final XOR 0xFFFFFFFF): the value of zlib's crc32() and crc32fast::hash, so
  * a consumer can check it without this library.  It is defined on bytes whatever symbol_bits is; an empty block gives

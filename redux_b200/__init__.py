@@ -162,6 +162,8 @@ def lib():
     L.redux_select_models.argtypes = [vp, pp, vp, u32, vp, vp, u64, vp, vp]
     L.redux_select_models_device.argtypes = [vp, i32, vp, pp, vp, u32, vp, vp, u64, u64, vp, vp]
     L.redux_encode_batch_select.argtypes = [vp, i32, pp, vp, u32, vp, vp, u64, vp, u64, vp, vp, vp]
+    L.redux_build_models.argtypes = [vp, pp, u32, u32, vp, vp, vp, u64, vp, vp, vp]
+    L.redux_build_models_device.argtypes = [vp, i32, vp, pp, u32, u32, vp, vp, vp, u64, u64, vp, vp, vp]
     L.redux_crc32_blocks.argtypes = [vp, vp, vp, u64, vp]
     L.redux_crc32_blocks_device.argtypes = [vp, i32, vp, vp, vp, vp, u64, u64, vp]
     L.redux_encode_batch_models_crc.argtypes = [vp, i32, pp, vp, u32, vp, vp, vp, u64, vp, u64, vp, vp, vp]
@@ -383,6 +385,23 @@ def _trained_models(cls, params, rows):
         m.freq = r.copy()
         out.append(m)
     return out
+
+
+def _build_args(model, init, n):
+    """(Parameters, uint32 init or None) of build_models; a trained model and an init of the wrong length are
+    refused."""
+    if not isinstance(model, Model):
+        raise InvalidInput("build_models: model must be an AdaptiveLinearModel or AdaptiveTreeModel")
+    if model.freq is not None and (np.asarray(model.freq) != 1).any():
+        raise InvalidInput("build_models: model gives the kind and Parameters only, and must be fresh")
+    if init is None:
+        return model.params, None
+    init = np.ascontiguousarray(init, dtype=np.int64).ravel()
+    if init.size != n:
+        raise InvalidInput("build_models: %d init values for %d blocks" % (init.size, n))
+    if init.size and init.min() < 0:
+        raise InvalidInput("build_models: a negative init value")
+    return model.params, np.ascontiguousarray(np.minimum(init, (1 << 32) - 1), dtype=np.uint32)
 
 
 def _ptr(x):
@@ -667,6 +686,40 @@ class Context:
         if check:
             _raise(rc, self)
         return out[:int(out_off[n])], out_off, status[:n], block_model[:n]
+
+    # ---- learning start models from the blocks themselves (redux_build_models, DESIGN.md 3.12)
+    def build_models(self, data, offsets, model, k, iterations=8, init=None):
+        """Clusters the blocks data[offsets[i]:offsets[i+1]] into k groups by their ideal code length and returns
+        (models, block_model, iteration_cost_bits): k + 1 models of model's kind and Parameters (models[0] fresh, the
+        others learned from the blocks), each block's index into them (what select_models picks for them) and every
+        round's total cost in bits.  model gives the kind and Parameters only: a trained one raises InvalidInput.
+        init: None (contiguous ranges) or each block's starting cluster, 0 (fresh) to k."""
+        data = np.ascontiguousarray(data, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offsets.size - 1
+        params, init = _build_args(model, init, n)
+        table = np.zeros((k + 1, params.symbol_count), dtype=np.uint32)
+        block_model = np.zeros(max(n, 1), dtype=np.uint32)
+        totals = np.zeros(max(iterations, 1), dtype=np.float64)
+        pc = params._c()
+        _raise(lib().redux_build_models(self._h, C.byref(pc), k, iterations, _ptr(init),
+                                        _ptr(data) if data.size else None, _ptr(offsets), n, _ptr(table),
+                                        _ptr(block_model), _ptr(totals)), self)
+        models = [type(model)(params)] + _trained_models(type(model), params, table[1:])
+        return models, block_model[:n], totals[:iterations]
+
+    def build_models_device(self, d_in, d_in_offsets, n_blocks, max_block_len, model, k, d_out_freqs,
+                            d_block_model=None, d_iteration_cost_bits=None, iterations=8, init=None, device=0,
+                            stream=None):
+        """build_models on device-resident buffers: d_out_freqs (uint32, (k + 1) x symbol_count) receives the table,
+        d_block_model (uint32, n_blocks) and d_iteration_cost_bits (float64, iterations), if given, the choice and the
+        totals.  Asynchronous on `stream`; init is host memory."""
+        params, init = _build_args(model, init, n_blocks)
+        pc = params._c()
+        _raise(lib().redux_build_models_device(self._h, device, stream, C.byref(pc), k, iterations, _ptr(init),
+                                               _ptr(d_in), _ptr(d_in_offsets), n_blocks, max_block_len,
+                                               _ptr(d_out_freqs), _ptr(d_block_model),
+                                               _ptr(d_iteration_cost_bits)), self)
 
     # ---- CRC-32 of every block on the device (redux_crc32_blocks, DESIGN.md 3.11)
     def crc32_blocks(self, data, offsets):

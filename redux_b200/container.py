@@ -20,7 +20,8 @@ the row each block starts from in its segment's index.
 A row is a model's frequency vector, fresh (all ones) or trained: every entry >= 1, total <= freq_max.  Block i's
 stream is compress() of the block with a model in that state.  pack / pack_stream still write version 1.
 pack_models / pack_stream_models take the index from the caller, pack_auto / pack_stream_auto let the device choose it
-(redux_encode_batch_select).
+(redux_encode_batch_select), and pack_learned / pack_stream_learned also learn the table from the first batch of
+blocks (redux_build_models) before the device chooses.
 
 Version 3 is version 2 plus the CRC-32 of every block's raw bytes (zlib's crc32, computed on the device while the
 block is coded), so a reader can tell a damaged file from a good one:
@@ -141,11 +142,12 @@ def pack_stream(fin, fout, model, block_len=65536, batch_blocks=16384, context=N
     return raw_total, out_total + 8
 
 
-def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum):
+def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum, chunk=None):
     """Writes a version 2 (checksum: version 3) container of fin's bytes: the header and model table of `models`, then
     one segment per batch of `batch_blocks` blocks.  encode(data, offsets, first) codes a batch whose first block is
     block `first` of the input and returns (streams, stream offsets, model index, CRCs; None without checksum).
-    Returns (raw_bytes, container_bytes)."""
+    chunk: the first batch's bytes when the caller has read them from fin already.  Returns (raw_bytes,
+    container_bytes)."""
     kind, pc, table = rb._model_table(models)
     if pc.symbol_bits != 8:
         raise ContainerError("the container stores byte-symbol streams only (symbol_bits must be 8)")
@@ -156,10 +158,11 @@ def _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum
     fout.write(table.astype("<u4").tobytes())
     raw_total, out_total, first = 0, HEADER.size + 4 + table.nbytes, 0
     while True:
-        chunk = fin.read(block_len * batch_blocks)
+        chunk = chunk if chunk is not None else fin.read(block_len * batch_blocks)
         if not chunk:
             break
         data = np.frombuffer(chunk, dtype=np.uint8)
+        chunk = None
         n = (data.size + block_len - 1) // block_len
         off = np.minimum(np.arange(n + 1, dtype=np.uint64) * np.uint64(block_len), np.uint64(data.size))
         comp, coff, idx, crc = encode(data, off, first)
@@ -204,11 +207,8 @@ def pack_stream_models(fin, fout, models, block_model, block_len=65536, batch_bl
     return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum)
 
 
-def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, context=None, checksum=False):
-    """pack_stream_models with each block's start model chosen on the device (Context.encode_batch_select): the model
-    with the smallest estimated compressed size of the block.  Writes version 2 (checksum=True: version 3).  Returns
-    (raw_bytes, container_bytes)."""
-    models = list(models)
+def _select_encoder(models, context, checksum):
+    """_pack_stream_v2's encode with each block's model chosen on the device (Context.encode_batch_select)."""
 
     def encode(data, off, first):
         if checksum:
@@ -217,7 +217,39 @@ def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, con
         comp, coff, _, idx = (context or rb._ctx()).encode_batch_select(data, off, models)
         return comp, coff, idx, None
 
-    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, encode, checksum)
+    return encode
+
+
+def pack_stream_auto(fin, fout, models, block_len=65536, batch_blocks=16384, context=None, checksum=False):
+    """pack_stream_models with each block's start model chosen on the device (Context.encode_batch_select): the model
+    with the smallest estimated compressed size of the block.  Writes version 2 (checksum=True: version 3).  Returns
+    (raw_bytes, container_bytes)."""
+    models = list(models)
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, _select_encoder(models, context, checksum),
+                           checksum)
+
+
+def pack_stream_learned(fin, fout, model, k=16, iterations=8, block_len=65536, batch_blocks=16384, context=None,
+                        checksum=False):
+    """pack_stream_auto with a model table learned from the data itself: the first batch of `batch_blocks` blocks is
+    clustered into k groups (Context.build_models, `iterations` rounds), and every batch is then coded with each
+    block's start model chosen on the device from the k + 1 models (fresh first).  model gives the kind and Parameters
+    only (fresh, byte symbols).  Writes version 2 (checksum=True: version 3); unpack_stream reads it.  Returns
+    (raw_bytes, container_bytes)."""
+    if model.freq is not None and (np.asarray(model.freq) != 1).any():
+        raise ContainerError("pack_learned learns its models: pass a fresh model for the kind and Parameters")
+    if model.params.symbol_bits != 8:
+        raise ContainerError("the container stores byte-symbol streams only (symbol_bits must be 8)")
+    chunk = fin.read(block_len * batch_blocks)
+    models = [model]
+    if chunk:
+        data = np.frombuffer(chunk, dtype=np.uint8)
+        n = (data.size + block_len - 1) // block_len
+        off = np.minimum(np.arange(n + 1, dtype=np.uint64) * np.uint64(block_len), np.uint64(data.size))
+        models, _, _ = (context or rb._ctx()).build_models(data, off, model, k, iterations)
+
+    return _pack_stream_v2(fin, fout, models, block_len, batch_blocks, _select_encoder(models, context, checksum),
+                           checksum, chunk)
 
 
 def check_segment(segment, status, raw_lens, lens, used, sizes, crc, stored_crc):
@@ -331,6 +363,15 @@ def pack_auto(data, models, block_len=65536, context=None, checksum=False):
     pack_stream_auto."""
     out = io.BytesIO()
     pack_stream_auto(io.BytesIO(bytes(data)), out, models, block_len, context=context, checksum=checksum)
+    return out.getvalue()
+
+
+def pack_learned(data, model, k=16, iterations=8, block_len=65536, context=None, checksum=False):
+    """pack with a model table learned from the data (version 2, checksum=True: version 3); see
+    pack_stream_learned."""
+    out = io.BytesIO()
+    pack_stream_learned(io.BytesIO(bytes(data)), out, model, k, iterations, block_len, context=context,
+                        checksum=checksum)
     return out.getvalue()
 
 

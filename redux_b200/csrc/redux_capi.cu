@@ -28,6 +28,7 @@
 #include "redux_warp_codec.cuh"
 #include "redux_split_encoder.cuh"
 #include "redux_select.cuh"
+#include "redux_build.cuh"
 #include "redux_crc.cuh"
 
 using namespace rdx;
@@ -245,6 +246,7 @@ struct DeviceState {
     // redux_select_models: candidate rows, SelectSetup::meta, {0, no limit} per block of a slice (the histogram pass's
     // TrainJob::sample), histogram scratch of every stream
     DevBuf sel_rows, sel_meta, sel_sample, sel_scratch;
+    DevBuf bld_scratch;                        // redux_build_models: histograms, ladder costs, cluster sums, ... (BuildLayout)
     HostBuf pin_bmod;                          // redux_encode_batch_select: the chosen rows on their way out
     DevBuf st_crc; HostBuf pin_crc;            // the *_crc calls: each chunk's CRCs on their way out
     int sms = 0;                               // multiprocessors: CTAs of the persistent CRC kernel
@@ -341,6 +343,7 @@ cudaError_t configure_kernels()
     if ((e = allow_smem(train_count_kernel, kTrainSmemWords * sizeof(uint32_t))) != cudaSuccess) return e;
     // selection: the running histogram of alphabets up to 14 bits (64 KiB at 14 bits)
     if ((e = allow_smem(select_cost_kernel, sizeof(uint32_t) << kSelectMaxSmemSymbolBits)) != cudaSuccess) return e;
+    if ((e = allow_smem(build_ladder_kernel, sizeof(uint32_t) << kSelectMaxSmemSymbolBits)) != cudaSuccess) return e;
     // CRC-32: the lane-replicated slice-by-4 tables (128 KiB)
     if ((e = allow_smem(crc32_blocks_kernel, kCrcSmemBytes)) != cudaSuccess) return e;
     return allow_smem(decode_generic_kernel, generic_smem_bytes(kGenericSmemSymbolBits));
@@ -946,7 +949,7 @@ extern "C" void redux_ctx_destroy(redux_ctx_t *ctx)
         for (DevBuf *b : {&d.slots, &d.sizes, &d.flag, &d.st_in, &d.st_off, &d.st_bmod, &d.st_out, &d.st_ooff,
                           &d.st_status, &d.st_aux0, &d.st_aux1, &d.st_roff, &d.corpus, &d.gen_magic, &d.gen_tabs, &d.gen_init,
                           &d.gen_freq, &d.gen_start, &d.split_hist, &d.split_pairs, &d.train_rows, &d.train_sample,
-                          &d.sel_rows, &d.sel_meta, &d.sel_sample, &d.sel_scratch}) b->release();
+                          &d.sel_rows, &d.sel_meta, &d.sel_sample, &d.sel_scratch, &d.bld_scratch}) b->release();
         for (auto &m : d.magics) cudaFree(m.ptr);
         if (d.text_lut) cudaFree(d.text_lut);
         for (StageRing *r : {d.ring_up, d.ring_down}) if (r) { r->release(); delete r; }
@@ -1404,34 +1407,48 @@ int select_prepare(redux_ctx *ctx, DeviceState *d, cudaStream_t stream, const Se
     return REDUX_OK;
 }
 
+// Enqueues the histogram pass of cnt blocks on stream s: their full histograms into hist (cnt x nsym, zeroed here).
+// sample: {0, no limit} for each of the cnt blocks.
+int hist_enqueue(redux_ctx *ctx, cudaStream_t s, uint32_t sym_bits, uint32_t nsym, const uint2 *sample,
+                 const uint8_t *d_in, const uint64_t *d_in_off, uint64_t cnt, uint64_t max_n, uint32_t *hist)
+{
+    CU_TRY(ctx, cudaMemsetAsync(hist, 0, (size_t)cnt * nsym * sizeof(uint32_t), s));
+    TrainJob j;
+    j.in = d_in; j.in_off = d_in_off;
+    j.table = nullptr; j.sample = sample;
+    j.out = hist; j.n_samples = cnt;
+    j.s = sym_bits; j.nsym = nsym;
+    j.chunk = kTrainChunk;
+    j.chunks = (uint32_t)std::max<uint64_t>((max_n + kTrainChunk - 1) / kTrainChunk, 1);
+    j.n_ctas = max_n ? cnt * j.chunks : 0;
+    j.copies = train_copies(sym_bits);
+    if (j.n_ctas) {
+        const size_t smem = ((size_t)j.copies << sym_bits) * sizeof(uint32_t);
+        train_count_kernel<<<(uint32_t)std::min<uint64_t>(j.n_ctas, 0x7FFFFFFFull), kTrainThreads, smem, s>>>(j);
+        ctx->launches++;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    return REDUX_OK;
+}
+
 // Enqueues the selection of n_blocks blocks on stream s with scratch area `slot`: per slice, the histogram pass
-// (train_count_kernel into zeroed rows) and select_cost_kernel.  d_cost: NULL or n_blocks x n_models doubles.
+// (hist_enqueue) and select_cost_kernel.  When d_hist (n_blocks x nsym) already holds the histograms the pass is
+// skipped and the scratch area holds only the running histograms (slice x 2^s words, symbol_bits > 14).  d_cost: NULL
+// or n_blocks x n_models doubles; d_best_cost: NULL or n_blocks doubles, the chosen model's cost.
 int select_enqueue(redux_ctx *ctx, cudaStream_t s, const SelectSetup &t, const SelectDev &dev, int slot,
                    const uint8_t *d_in, const uint64_t *d_in_off, uint64_t n_blocks, uint64_t max_block_len,
-                   uint32_t *d_block_model, double *d_cost)
+                   uint32_t *d_block_model, double *d_cost, const uint32_t *d_hist = nullptr,
+                   double *d_best_cost = nullptr)
 {
     uint8_t *scratch = dev.scratch + (size_t)slot * dev.slice * t.block_bytes();
-    uint32_t *hist = (uint32_t *)scratch, *run = hist + dev.slice * t.nsym;
+    uint32_t *hist = (uint32_t *)scratch, *run = d_hist ? hist : hist + dev.slice * t.nsym;
     const uint64_t max_n = max_block_len * 8 / t.s;
     const uint32_t *meta = dev.meta;
     for (uint64_t first = 0; first < n_blocks; first += dev.slice) {
         const uint64_t cnt = std::min<uint64_t>(dev.slice, n_blocks - first);
-        CU_TRY(ctx, cudaMemsetAsync(hist, 0, (size_t)cnt * t.nsym * sizeof(uint32_t), s));
-        TrainJob j;
-        j.in = d_in; j.in_off = d_in_off + first;
-        j.table = nullptr; j.sample = dev.sample;
-        j.out = hist; j.n_samples = cnt;
-        j.s = t.s; j.nsym = t.nsym;
-        j.chunk = kTrainChunk;
-        j.chunks = (uint32_t)std::max<uint64_t>((max_n + kTrainChunk - 1) / kTrainChunk, 1);
-        j.n_ctas = max_n ? cnt * j.chunks : 0;
-        j.copies = train_copies(t.s);
-        if (j.n_ctas) {
-            const size_t smem = ((size_t)j.copies << t.s) * sizeof(uint32_t);
-            train_count_kernel<<<(uint32_t)std::min<uint64_t>(j.n_ctas, 0x7FFFFFFFull), kTrainThreads, smem, s>>>(j);
-            ctx->launches++;
-            CU_TRY(ctx, cudaGetLastError());
-        }
+        int rc;
+        if (!d_hist && (rc = hist_enqueue(ctx, s, t.s, t.nsym, dev.sample, d_in, d_in_off + first, cnt, max_n, hist)))
+            return rc;
         SelectJob sj;
         sj.in = d_in; sj.in_off = d_in_off + first;
         sj.rows = dev.rows;
@@ -1439,9 +1456,10 @@ int select_enqueue(redux_ctx *ctx, cudaStream_t s, const SelectSetup &t, const S
         sj.order = meta + 2 * t.n_models;
         sj.group = sj.order + t.n_models;
         sj.split = sj.group + t.n_groups + 1;
-        sj.hist = hist; sj.run = run;
+        sj.hist = d_hist ? d_hist + first * t.nsym : hist; sj.run = run;
         sj.block_model = d_block_model + first;
         sj.cost = d_cost ? d_cost + first * t.n_models : nullptr;
+        sj.best_cost = d_best_cost ? d_best_cost + first : nullptr;
         sj.n_blocks = cnt;
         sj.n_models = t.n_models; sj.n_groups = t.n_groups; sj.s = t.s; sj.nsym = t.nsym;
         const size_t smem = t.s <= kSelectMaxSmemSymbolBits ? sizeof(uint32_t) << t.s : 0;
@@ -2458,6 +2476,234 @@ extern "C" int redux_encode_batch_select(redux_ctx_t *ctx, int model_kind, const
     ctx->models.select = &t;
     ctx->models.chosen = block_model;
     return redux_encode_batch(ctx, model_kind, params, in, in_offsets, n_blocks, out, out_capacity, out_offsets, status);
+}
+
+// ================================================================== learning start models (DESIGN.md 3.12)
+// redux_build_models: Lloyd-style clustering of the blocks by their ideal code length (redux_build.cuh).  The host
+// checks the arguments and lays out the scratch, then enqueues every round on one stream with no round trip: the
+// histogram pass once, then per round the cluster sums, the candidate rows, the ladder costs, the ladder choice with
+// the round's table and meta, select_cost_kernel on the cached histograms, and the total.
+
+namespace {
+
+struct BuildSetup {
+    uint32_t s = 8, nsym = 257, fmax = 0, K = 0, iterations = 0, L = 0;
+    uint32_t T[kBuildMaxLevels] = {};
+    std::vector<uint32_t> init;              // n_blocks memberships
+};
+
+// Byte offsets into DeviceState::bld_scratch.  `bounded` is what REDUX_MAX_BUILD_SCRATCH_BYTES limits.  Above 14 bits
+// the ladder and selection kernels keep a running histogram per block in global memory, `slice` blocks per launch
+// (kSelectScratchBytes of them); below, one launch takes every block.
+struct BuildLayout {
+    size_t hist, lcost, G, cand, cstart, bounded;
+    size_t member[2], best, table, meta, level, split, totals, sample, run, total;
+    uint64_t slice;
+    BuildLayout(const BuildSetup &t, uint64_t n) {
+        size_t at = 0;
+        auto take = [&at](size_t bytes) { const size_t o = at; at += (bytes + 255) & ~(size_t)255; return o; };
+        hist = take((size_t)n * t.nsym * 4);
+        lcost = take((size_t)n * t.L * 8);
+        G = take(((size_t)t.K << t.s) * 8);
+        cand = take((size_t)t.K * t.L * t.nsym * 4);
+        cstart = take((size_t)t.K * t.L * 8);
+        bounded = at;
+        member[0] = take((size_t)n * 4); member[1] = take((size_t)n * 4);
+        best = take((size_t)n * 8);
+        table = take((size_t)(t.K + 1) * t.nsym * 4);
+        meta = take((size_t)(3 * (t.K + 1) + 2 * (t.L + 1) + 1) * 4);
+        level = take((size_t)t.K * 4);
+        split = take((size_t)t.L * 4);
+        totals = take((size_t)t.iterations * 8);
+        sample = take((size_t)n * sizeof(uint2));
+        slice = t.s > kSelectMaxSmemSymbolBits ? std::max<uint64_t>(1, std::min<uint64_t>(n, kSelectScratchBytes >> (t.s + 2)))
+                                               : n;
+        run = take(t.s > kSelectMaxSmemSymbolBits ? (size_t)slice << (t.s + 2) : 0);
+        total = at;
+    }
+};
+
+// The checks every form makes before a device is needed.
+int build_setup(redux_ctx *ctx, const redux_params_t *p, uint32_t K, uint32_t iterations, const uint32_t *init,
+                uint64_t n_blocks, BuildSetup *t)
+{
+    if (!p) return fail(ctx, REDUX_INVALID_INPUT, "params is NULL");
+    if (!params_valid(p->symbol_bits, p->freq_bits, p->code_bits))
+        return fail(ctx, REDUX_INVALID_INPUT, "Parameters::new rejects these parameters");
+    if (p->symbol_bits > kGenericMaxSymbolBits)
+        return fail(ctx, REDUX_UNSUPPORTED, "device path implements symbol_bits <= 16");
+    if (K == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_clusters is 0");
+    if (iterations == 0) return fail(ctx, REDUX_INVALID_INPUT, "iterations is 0");
+    t->s = p->symbol_bits; t->nsym = (1u << t->s) + 1;
+    t->fmax = (uint32_t)(((uint64_t)1 << p->freq_bits) - 1);
+    t->K = K; t->iterations = iterations;
+    if ((uint64_t)(K + 1ull) * (t->nsym + 1) * sizeof(uint32_t) > REDUX_MAX_MODEL_TABLE_BYTES)
+        return fail(ctx, REDUX_UNSUPPORTED, "n_clusters + 1 rows of (symbol_count + 1) entries exceed REDUX_MAX_MODEL_TABLE_BYTES");
+    if (n_blocks == 0) return fail(ctx, REDUX_INVALID_INPUT, "n_blocks is 0: no blocks to learn from");
+    t->L = build_ladder(t->s, p->freq_bits, t->T);
+    t->init.resize(n_blocks);
+    for (uint64_t b = 0; b < n_blocks; ++b) {
+        if (init && init[b] > K) {
+            char msg[96];
+            snprintf(msg, sizeof msg, "init of block %llu is %u > n_clusters", (unsigned long long)b, init[b]);
+            return fail(ctx, REDUX_INVALID_INPUT, msg);
+        }
+        t->init[b] = init ? init[b] : 1u + (uint32_t)((unsigned __int128)b * K / n_blocks);
+    }
+    if (BuildLayout(*t, n_blocks).bounded > REDUX_MAX_BUILD_SCRATCH_BYTES)
+        return fail(ctx, REDUX_UNSUPPORTED, "histograms, ladder costs, cluster sums and candidates exceed REDUX_MAX_BUILD_SCRATCH_BYTES");
+    return REDUX_OK;
+}
+
+// Enqueues the whole build on stream s of device d, after the caller's ws_acquire (one device call in flight,
+// DESIGN.md 4).  d_out: (K+1) x nsym; d_bmod: NULL or n_blocks; d_totals: NULL or iterations doubles.
+int build_enqueue(redux_ctx *ctx, DeviceState *d, cudaStream_t s, const BuildSetup &t, const uint8_t *d_in,
+                  const uint64_t *d_in_off, uint64_t n, uint64_t max_block_len, uint32_t *d_out, uint32_t *d_bmod,
+                  double *d_totals)
+{
+    const BuildLayout lay(t, n);
+    CU_TRY(ctx, d->bld_scratch.reserve(lay.total));
+    uint8_t *base = (uint8_t *)d->bld_scratch.p;
+    uint32_t *hist = (uint32_t *)(base + lay.hist), *table = (uint32_t *)(base + lay.table);
+    uint32_t *meta = (uint32_t *)(base + lay.meta), *split = (uint32_t *)(base + lay.split);
+    uint32_t *member[2] = {(uint32_t *)(base + lay.member[0]), (uint32_t *)(base + lay.member[1])};
+    double *best = (double *)(base + lay.best), *totals = (double *)(base + lay.totals);
+    std::vector<uint32_t> ones(t.nsym, 1u), splits(t.L);
+    for (uint32_t l = 0; l < t.L; ++l) splits[l] = t.fmax - t.T[l];
+    // the histogram pass counts every symbol of a block: start row 0 (unused), no limit below the block's own
+    const std::vector<uint2> sample(n, make_uint2(0u, (uint32_t)(kSelectMaxSymbols - 1)));
+    CU_TRY(ctx, cudaMemcpyAsync(member[0], t.init.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(table, ones.data(), t.nsym * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(split, splits.data(), t.L * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(base + lay.sample, sample.data(), n * sizeof(uint2), cudaMemcpyHostToDevice, s));
+    int rc;
+    if ((rc = hist_enqueue(ctx, s, t.s, t.nsym, (const uint2 *)(base + lay.sample), d_in, d_in_off, n,
+                           max_block_len * 8 / t.s, hist))) return rc;
+
+    // the selection over the round's table (select_enqueue on the cached histograms): the table and meta the ladder
+    // choice writes, and the running histograms above 14 bits, which the ladder kernel shares
+    SelectSetup st;
+    st.s = t.s; st.nsym = t.nsym; st.n_models = t.K + 1; st.n_groups = t.L + 1;
+    SelectDev dev;
+    dev.rows = table; dev.meta = meta; dev.scratch = base + lay.run; dev.slice = lay.slice;
+
+    BuildJob j;
+    j.hist = hist;
+    j.G = (unsigned long long *)(base + lay.G);
+    j.cand = (uint32_t *)(base + lay.cand); j.cand_start = (uint2 *)(base + lay.cstart);
+    j.lcost = (const double *)(base + lay.lcost);
+    j.table = table; j.meta = meta; j.level = (uint32_t *)(base + lay.level);
+    j.n_blocks = n; j.K = t.K; j.L = t.L; j.s = t.s; j.nsym = t.nsym; j.fmax = t.fmax;
+    std::copy(t.T, t.T + kBuildMaxLevels, j.T);
+    BuildLadderJob lj;
+    lj.sel.in = d_in; lj.sel.rows = j.cand; lj.sel.start = j.cand_start; lj.sel.split = split;
+    lj.sel.order = nullptr; lj.sel.group = nullptr; lj.sel.block_model = nullptr; lj.sel.cost = nullptr;
+    lj.sel.run = (uint32_t *)(base + lay.run);
+    lj.sel.n_models = t.K * t.L; lj.sel.n_groups = t.L; lj.sel.s = t.s; lj.sel.nsym = t.nsym;
+    lj.L = t.L;
+    BuildTotalJob tj;
+    tj.best_cost = best; tj.totals = totals; tj.table = table;
+    tj.out_table = d_out; tj.out_choice = d_bmod;
+    tj.n_blocks = n; tj.table_words = (uint64_t)(t.K + 1) * t.nsym;
+    const size_t ladder_smem = t.s <= kSelectMaxSmemSymbolBits ? sizeof(uint32_t) << t.s : 0;
+    for (uint32_t it = 0; it < t.iterations; ++it) {
+        uint32_t *M = member[it & 1], *A = member[(it + 1) & 1];
+        j.member = M;
+        CU_TRY(ctx, cudaMemsetAsync(j.G, 0, ((size_t)t.K << t.s) * 8, s));
+        build_cluster_kernel<<<(uint32_t)((n + kBuildClusterRun - 1) / kBuildClusterRun), kBuildThreads, 0, s>>>(j);
+        build_row_kernel<<<t.K * t.L, kBuildThreads, 0, s>>>(j);
+        ctx->launches += 2;
+        CU_TRY(ctx, cudaGetLastError());
+        for (uint64_t first = 0; first < n; first += dev.slice) {
+            const uint64_t cnt = std::min<uint64_t>(dev.slice, n - first);
+            lj.sel.in_off = d_in_off + first; lj.sel.hist = hist + first * t.nsym; lj.sel.n_blocks = cnt;
+            lj.member = M + first; lj.lcost = (double *)j.lcost + first * t.L;
+            build_ladder_kernel<<<(uint32_t)std::min<uint64_t>(cnt, 0x7FFFFFFFull), kSelectThreads, ladder_smem, s>>>(lj);
+            ctx->launches++;
+            CU_TRY(ctx, cudaGetLastError());
+        }
+        build_choice_kernel<<<t.K, kBuildThreads, 0, s>>>(j);
+        build_meta_kernel<<<1, 32, 0, s>>>(j);
+        ctx->launches += 2;
+        CU_TRY(ctx, cudaGetLastError());
+        if ((rc = select_enqueue(ctx, s, st, dev, 0, d_in, d_in_off, n, max_block_len, A, nullptr, hist, best)))
+            return rc;
+        tj.choice = A; tj.it = it;
+        build_total_kernel<<<1, kBuildTotalThreads, 0, s>>>(tj);
+        ctx->launches++;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    if (d_totals)
+        CU_TRY(ctx, cudaMemcpyAsync(d_totals, totals, t.iterations * sizeof(double), cudaMemcpyDeviceToDevice, s));
+    CU_TRY(ctx, ws_release(d, s));
+    return REDUX_OK;
+}
+
+}  // namespace
+
+extern "C" int redux_build_models_device(redux_ctx_t *ctx, int device, void *stream_, const redux_params_t *params,
+                                         uint32_t n_clusters, uint32_t iterations, const uint32_t *init,
+                                         const uint8_t *d_in, const uint64_t *d_in_offsets, uint64_t n_blocks,
+                                         uint64_t max_block_len, uint32_t *d_out_freqs, uint32_t *d_block_model,
+                                         double *d_iteration_cost_bits)
+{
+    BuildSetup t;
+    int rc = build_setup(ctx, params, n_clusters, iterations, init, n_blocks, &t);
+    if (rc) return rc;
+    if (max_block_len * 8 / t.s >= kSelectMaxSymbols)
+        return fail(ctx, REDUX_UNSUPPORTED, "blocks of 2^31 symbols or more are not supported");
+    if (!ctx) return train_no_context();
+    DeviceState *d = find_dev(ctx, device);
+    if (!d) return fail(ctx, REDUX_INVALID_INPUT, "device is not part of this context");
+    if (!d_in_offsets || !d_out_freqs || (!d_in && max_block_len)) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    DeviceGuard g(device);
+    cudaStream_t s = (cudaStream_t)stream_;
+    CU_TRY(ctx, ws_acquire(d, s));
+    return build_enqueue(ctx, d, s, t, d_in, d_in_offsets, n_blocks, max_block_len, d_out_freqs, d_block_model,
+                         d_iteration_cost_bits);
+}
+
+extern "C" int redux_build_models(redux_ctx_t *ctx, const redux_params_t *params, uint32_t n_clusters,
+                                  uint32_t iterations, const uint32_t *init, const uint8_t *in,
+                                  const uint64_t *in_offsets, uint64_t n_blocks, uint32_t *out_freqs,
+                                  uint32_t *block_model, double *iteration_cost_bits)
+{
+    BuildSetup t;
+    int rc = build_setup(ctx, params, n_clusters, iterations, init, n_blocks, &t);
+    if (rc) return rc;
+    if (!in_offsets || !out_freqs) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    SelectSetup st;
+    st.s = t.s;
+    uint64_t max_len = 0;
+    if ((rc = select_check_lengths(ctx, st, in_offsets, n_blocks, &max_len))) return rc;
+    const uint64_t first = in_offsets[0], total = in_offsets[n_blocks] - first;
+    if (!in && total) return fail(ctx, REDUX_INVALID_INPUT, "NULL buffer");
+    if (!ctx) return train_no_context();
+    // the context's first device, like redux_train_models
+    DeviceState *d = &ctx->devs[0];
+    DeviceGuard g(d->device);
+    cudaStream_t s = d->stream;
+    std::vector<uint64_t> off(in_offsets, in_offsets + n_blocks + 1);
+    for (uint64_t &o : off) o -= first;
+    const size_t table_bytes = (size_t)(n_clusters + 1) * t.nsym * sizeof(uint32_t);
+    CU_TRY(ctx, d->st_in.reserve(total + 16));               // + 16: the last aligned 16-byte load
+    CU_TRY(ctx, d->st_off.reserve(off.size() * sizeof(uint64_t)));
+    CU_TRY(ctx, d->st_bmod.reserve(n_blocks * sizeof(uint32_t)));
+    CU_TRY(ctx, d->st_out.reserve(table_bytes));
+    CU_TRY(ctx, d->st_aux0.reserve(iterations * sizeof(double)));
+    CU_TRY(ctx, ws_acquire(d, s));
+    if (total) CU_TRY(ctx, cudaMemcpyAsync(d->st_in.p, in + first, total, cudaMemcpyHostToDevice, s));
+    CU_TRY(ctx, cudaMemcpyAsync(d->st_off.p, off.data(), off.size() * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+    if ((rc = build_enqueue(ctx, d, s, t, (const uint8_t *)d->st_in.p, (const uint64_t *)d->st_off.p, n_blocks, max_len,
+                            (uint32_t *)d->st_out.p, (uint32_t *)d->st_bmod.p, (double *)d->st_aux0.p))) return rc;
+    CU_TRY(ctx, cudaMemcpyAsync(out_freqs, d->st_out.p, table_bytes, cudaMemcpyDeviceToHost, s));
+    if (block_model)
+        CU_TRY(ctx, cudaMemcpyAsync(block_model, d->st_bmod.p, n_blocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    if (iteration_cost_bits)
+        CU_TRY(ctx, cudaMemcpyAsync(iteration_cost_bits, d->st_aux0.p, iterations * sizeof(double),
+                                    cudaMemcpyDeviceToHost, s));
+    CU_TRY(ctx, cudaStreamSynchronize(s));
+    return REDUX_OK;
 }
 
 // ================================================================== CRC-32 of every block (DESIGN.md 3.11)

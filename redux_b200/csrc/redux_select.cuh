@@ -44,6 +44,7 @@ struct SelectJob {
     uint32_t *run;               // n_blocks x 2^s running histograms (symbol_bits > 14), else unused
     uint32_t *block_model;       // n_blocks: the choice
     double *cost;                // n_blocks x n_models costs in bits, or NULL
+    double *best_cost = nullptr; // n_blocks: the chosen model's cost in bits, or NULL (redux_build_models)
     uint64_t n_blocks;
     uint32_t n_models, n_groups, s, nsym;
 };
@@ -123,18 +124,24 @@ __device__ __forceinline__ double select_partial(const SelectJob &j, const Selec
 }
 
 // Lane 0: the cost in bits of model k from its warp's 32 partial sums (in lane order) and the per-model terms
-//     lnG(T+m) - lnG(T) + ln(T' / r_EOF);
-// written to the cost row when asked, and kept if it beats the warp's best so far (lowest index among equal costs).
-__device__ __forceinline__ void select_finish(const SelectJob &j, const SelectBlock &b, uint64_t blk, uint32_t k,
-                                              uint32_t m, const double *part, SelectBest *best)
+//     lnG(T+m) - lnG(T) + ln(T' / r_EOF).
+__device__ __forceinline__ double select_bits(const SelectJob &j, uint32_t k, uint32_t m, const double *part)
 {
-    (void)b;
     double acc = 0.0;
     for (uint32_t l = 0; l < 32; ++l) acc += part[l];
     const double t = (double)j.start[k].x, tp = t + (double)m;
     if (m) acc += lgamma(tp) - lgamma(t);
     acc += log(tp / (double)j.start[k].y);
-    const double c = acc * kSelectInvLn2;
+    return acc * kSelectInvLn2;
+}
+
+// Lane 0: select_bits of model k, written to the cost row when asked, and kept if it beats the warp's best so far
+// (lowest index among equal costs).
+__device__ __forceinline__ void select_finish(const SelectJob &j, const SelectBlock &b, uint64_t blk, uint32_t k,
+                                              uint32_t m, const double *part, SelectBest *best)
+{
+    (void)b;
+    const double c = select_bits(j, k, m, part);
     if (j.cost) j.cost[blk * j.n_models + k] = c;
     if (c < best->c || (c == best->c && k < best->k)) { best->c = c; best->k = k; }
 }
@@ -146,6 +153,7 @@ __device__ __forceinline__ void select_choose(const SelectJob &j, uint64_t blk, 
     for (uint32_t i = 1; i < kSelectWarps; ++i)
         if (best[i].c < w.c || (best[i].c == w.c && best[i].k < w.k)) w = best[i];
     j.block_model[blk] = w.k;
+    if (j.best_cost) j.best_cost[blk] = w.c;
 }
 
 // The adaptive symbols of group g in a block of n symbols.
